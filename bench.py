@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (one process per GPU under torchrun for N>1)
     python bench.py --impl reference --gpus N --steps K ...  # the reference's own modules on the box's host cores
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's outputs as DIR/*.npy
 
 Workload (BASELINE.json metric "tokens/sec/GPU (LLaMA-3-8B SMT 0.71%)", configs[2]/[3]): a random-init LLaMA-3-8B
 (`LlamaForCausalLM`, bf16) whose q/k/v projections own 869 selected 256x256 blocks (0.71 % of the 122 528 blocks the
@@ -25,6 +26,7 @@ eagerly on the B200 for full steps of the same workload; `dp_check` (N>1) verifi
 from __future__ import annotations
 
 import argparse
+import contextlib
 import json
 import os
 import statistics
@@ -69,7 +71,15 @@ def parse_args():
     ap.add_argument("--capture-steps", type=int, default=4, help="gradient-capture passes of the warm-up phase")
     ap.add_argument("--torch-profile", type=str, default="", help="(diagnostic) write a torch.profiler kernel table of two "
                                                                   "steps to this file: GPU busy time vs step time")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", type=str, default="", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed to DIR/<name>.npy (see "
+                         "dump_outputs) so that two builds can be compared output for output; the warm-up then "
+                         "runs its attention backward on the deterministic math kernel, so its reported times are "
+                         "those of that kernel and it may select other blocks than a run without this flag")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 # ---------------------------------------------------------------------------------------------------------------
@@ -242,6 +252,30 @@ def build_model(args, device):
         torch.set_default_dtype(torch.float32)
     model.config.use_cache = False
     return model
+
+
+DUMP_SAMPLE = 1 << 22       # positions kept per weight array: 2 x 16 MB of float32
+
+
+def dump_outputs(out_dir, loss, model, opt):
+    """What the last timed step hands its caller: `loss.npy` (float64, [1]; this rank's loss on its own micro-batch,
+    not the mean over data-parallel ranks) and the trainable compact weights it
+    updated, as the model holds them (`selected_weight.npy`, bf16 values in float32) and as the optimizer's fp32
+    masters (`master_weight.npy`).  Both are the concatenation of every trainable parameter in `named_parameters()`
+    order, reduced to the same fixed, seeded sample of at most DUMP_SAMPLE sorted positions."""
+    import numpy as np
+    import torch
+    params = [p for _n, p in model.named_parameters() if p.requires_grad]
+    weights = torch.cat([p.detach().reshape(-1).float() for p in params])
+    masters = torch.cat([opt.state[p]["master"].reshape(-1) for p in params])
+    if weights.numel() > DUMP_SAMPLE:
+        pos = torch.randint(0, weights.numel(), (DUMP_SAMPLE,), generator=torch.Generator().manual_seed(0)).unique()
+        pos = pos.to(weights.device)
+        weights, masters = weights[pos], masters[pos]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "loss.npy"), np.array([loss.item()], dtype=np.float64))
+    np.save(os.path.join(out_dir, "selected_weight.npy"), weights.cpu().numpy())
+    np.save(os.path.join(out_dir, "master_weight.npy"), masters.cpu().numpy())
 
 
 def _median_ms(fn, iters=5, warmup=2, flush=None):
@@ -494,13 +528,24 @@ def run_ours(args):
             dp.allreduce_block_sums(acc_m)
         return acc_a, acc_m, times
 
+    # With --dump-outputs the warm-up's backward passes, which decide the blocks the timed steps train, run on the math
+    # attention kernel: the fused attention backward kernels accumulate in a run-dependent order, and the block scores
+    # of a random-init model are near-ties, so otherwise two runs select different blocks.  The timed steps are unchanged.
+    if args.dump_outputs:
+        from torch.nn.attention import SDPBackend, sdpa_kernel
+        warmup_attention = lambda: sdpa_kernel(SDPBackend.MATH)     # noqa: E731
+    else:
+        warmup_attention = contextlib.nullcontext
+
     # ---- extra (1 GPU): the reference's OWN warm-up policy - real full-fine-tuning steps while capturing ------------------
     full_ft = None
     if not args.no_extra and world == 1 and args.layers == 32:
-        full_ft = full_ft_warmup_record(model, dev_ids, steps=2)
+        with warmup_attention():
+            full_ft = full_ft_warmup_record(model, dev_ids, steps=2)
         set_capture_requires_grad(n_mlp > 0)
     launches_capture0 = ops.LAUNCHES["total"]
-    acc, acc_mlp, capture_ms = capture_phase(n_mlp > 0, max(1, args.capture_steps))
+    with warmup_attention():
+        acc, acc_mlp, capture_ms = capture_phase(n_mlp > 0, max(1, args.capture_steps))
     capture_launches = ops.LAUNCHES["total"] - launches_capture0
     # the same pass without any capture hooks: what the hooks + score kernels add per step
     plain_ms = None
@@ -714,6 +759,8 @@ def run_ours(args):
     e1.record()
     barrier()
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, loss, model, opt)
     ms_total = e0.elapsed_time(e1)
     launches = ops.LAUNCHES["total"] - launches0
     host_flush_ms = (ops.HOST_TIME["flush_s"] - host0["flush_s"]) * 1e3 / max(args.steps, 1)
@@ -984,6 +1031,9 @@ def run_ours(args):
                                        "passes, grad-ready hooks -> on-device block-sum accumulators, gradients released at "
                                        "once; the reference's full-FT policy is measured in warmup_full_ft_policy"),
                        "warmup_full_ft_policy": full_ft,
+                       # warm-up times below (and the full-FT record's) describe this attention backward
+                       "warmup_attention_backward": ("math (deterministic, --dump-outputs)" if args.dump_outputs
+                                                     else "default SDPA kernel"),
                        "warmup_path_ms": {"capture_pass_first_cold": capture_ms[0],
                                           "capture_pass_steady": statistics.median(capture_ms[1:]) if len(capture_ms) > 1 else None,
                                           "same_pass_without_capture_hooks": plain_ms,

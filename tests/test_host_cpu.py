@@ -4,6 +4,7 @@ parameter groups) mirrors the reference, and the product path fails LOUDLY witho
 import ctypes
 import os
 import re
+import warnings
 
 import numpy as np
 import pytest
@@ -13,6 +14,8 @@ from conftest import ROOT
 from oracle import golden_inputs as GI
 from oracle import smt_oracle as O
 from oracle.ref_shim import load_reference, reference_available
+
+NOT_STAGED = "the original project's smt modules are not staged (oracle/build_ref.py): comparison with them not run"
 
 
 def test_library_exports_every_header_symbol(built_library):
@@ -115,6 +118,8 @@ def test_freeze_matches_reference(mixture, layernorm):
         S, _ = load_reference()
         ref = S.freeze_unselected_matrix_layer(_tiny_llama(), sel_mlp, sel_attn, mixture=mixture, layernorm=layernorm)
         assert flags == {n: p.requires_grad for n, p in ref.named_parameters()}
+    else:
+        warnings.warn(NOT_STAGED)
     assert flags["model.layers.1.mlp.up_proj.weight"] and not flags["model.layers.0.mlp.up_proj.weight"]
     assert not flags["lm_head.weight"] and not flags["model.norm.weight"]
     assert flags["model.layers.1.self_attn.o_proj.weight"]        # smt.py:732 dispatches o_proj too
@@ -140,6 +145,8 @@ def test_param_groups_match_reference():
         for a, b in zip(ref, groups):
             assert [id(p) for p in a["params"]] == [id(p) for p in b["params"]]
             assert {k: v for k, v in a.items() if k != "params"} == {k: v for k, v in b.items() if k != "params"}
+    else:
+        warnings.warn(NOT_STAGED)
 
 
 def test_public_api_names_and_signatures():
@@ -170,6 +177,8 @@ def test_public_api_names_and_signatures():
             list(inspect.signature(S.LinearLayer_MatrixSparsity.__init__).parameters)
         assert list(inspect.signature(M.LinearLayer_ChannelSparsity.__init__).parameters) == \
             list(inspect.signature(S.LinearLayer_ChannelSparsity.__init__).parameters)
+    else:
+        warnings.warn(NOT_STAGED)
 
 
 def test_freeze_unselected_channel_layer_matches_reference():

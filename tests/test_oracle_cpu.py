@@ -79,7 +79,7 @@ def test_config1_budget_and_dims_match_golden():
     assert gold["total_blocks"] == 596
 
 
-@pytest.mark.skipif(not reference_available(), reason="/root/reference not present (GPU box)")
+@pytest.mark.skipif(not reference_available(), reason="the original project's smt modules are not staged (oracle/build_ref.py)")
 def test_oracle_against_live_reference():
     S, H = load_reference()
     torch.manual_seed(5)
