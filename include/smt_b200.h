@@ -242,6 +242,41 @@ SMT_API int smt_fused_linear_dgrad(const void* const* dy_host, const int64_t* ld
                                    const void* const* W_host, const int64_t* ldw_host, const int* N_host,
                                    void* dx, int64_t lddx, int dtype, void* stream);
 
+/* ---- elementwise work of a LLaMA decoder layer (bf16, fp32 arithmetic, deterministic) -------------------------------
+ * All tensors are contiguous bf16 (rstd: fp32) with 16-byte aligned storage.  The forward kernels reproduce the
+ * roundings of the HF modules they replace (transformers' LlamaRMSNorm, apply_rotary_pos_emb, LlamaMLP's
+ * `act_fn(gate) * up`), one bf16 rounding per PyTorch op. */
+
+/* RMSNorm over rows of H elements (H % 8 == 0, H <= 32768), T rows:
+ *   res == NULL:  x = a
+ *   res != NULL:  x = bf16(res + a), written to h_out       (the residual add in front of the norm)
+ *   rstd[t] = rsqrt(mean(x^2) + eps)   (fp32, kept for backward)
+ *   y = bf16(w * bf16(x * rstd))       (HF's two roundings; only the order of the row sum differs) */
+SMT_API int smt_rmsnorm_forward(const void* a, const void* res, const void* w, int64_t T, int H, float eps,
+                                void* h_out, void* y, float* rstd, void* stream);
+/* Input gradient of the norm above for a frozen weight (no dw):
+ *   g = dy * w,  xhat = x * rstd,  dx = bf16(rstd * (g - xhat * mean(g * xhat)) [+ dres])
+ * `dres` (optional) is the gradient that reaches x along the residual stream; adding it here replaces autograd's
+ * separate bf16 add at the fork.  `x` is the norm's input (h_out of a residual forward). */
+SMT_API int smt_rmsnorm_backward(const void* x, const void* w, const float* rstd, const void* dy,
+                                 const void* dres, int64_t T, int H, void* dx, void* stream);
+/* Rotary position embedding of q [B, S, Hq, 128] and k [B, S, Hk, 128] in one launch (the memory layout of the
+ * q/k projections' outputs).  cos / sin: [*, S, 128], batch stride `cs_bstride` elements (0 = shared by the batch).
+ *   forward   out = bf16(bf16(x * cos) + bf16(rotate_half(x) * sin)),  rotate_half(x) = (-x[64:], x[:64])
+ *   backward  the transpose with autograd's roundings:
+ *             dx = bf16(bf16(g * cos) + t),  t[:64] = bf16(g[64:] * sin[64:]),  t[64:] = -bf16(g[:64] * sin[:64])
+ * Outputs are separate tensors of the inputs' shape. */
+SMT_API int smt_rope_forward(const void* q, const void* k, const void* cos_, const void* sin_, int B, int S, int Hq,
+                             int Hk, int64_t cs_bstride, void* q_out, void* k_out, void* stream);
+SMT_API int smt_rope_backward(const void* dq_out, const void* dk_out, const void* cos_, const void* sin_, int B, int S,
+                              int Hq, int Hk, int64_t cs_bstride, void* dq, void* dk, void* stream);
+/* SwiGLU over n elements (n % 8 == 0):
+ *   forward   h  = bf16(bf16(silu(g)) * u)
+ *   backward  du = bf16(dh * bf16(silu(g))),  dg = bf16(silu'(g) * bf16(dh * u))   (torch's silu_backward formula) */
+SMT_API int smt_swiglu_forward(const void* g, const void* u, int64_t n, void* h, void* stream);
+SMT_API int smt_swiglu_backward(const void* g, const void* u, const void* dh, int64_t n, void* dg, void* du,
+                                void* stream);
+
 /* ---- compact optimizer ---------------------------------------------------------------- */
 
 /* out_sqnorm[0] = sum grad[i]^2 (fp32, deterministic two-stage tree). workspace: 4 KiB floats. */

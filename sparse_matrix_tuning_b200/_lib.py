@@ -83,6 +83,12 @@ _SIGNATURES = {
     "smt_fused_linear_supported": (C.c_int, [C.c_int, _P, C.c_int, C.c_int, C.c_int]),
     "smt_fused_linear_forward": (C.c_int, [_P, C.c_int64, C.c_int64, C.c_int, C.c_int, _P, _P, _P, _P, _P, C.c_int, _P]),
     "smt_fused_linear_dgrad": (C.c_int, [_P, _P, C.c_int64, C.c_int, C.c_int, _P, _P, _P, _P, C.c_int64, C.c_int, _P]),
+    "smt_rmsnorm_forward": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int, C.c_float, _P, _P, _P, _P]),
+    "smt_rmsnorm_backward": (C.c_int, [_P, _P, _P, _P, _P, C.c_int64, C.c_int, _P, _P]),
+    "smt_rope_forward": (C.c_int, [_P, _P, _P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int64, _P, _P, _P]),
+    "smt_rope_backward": (C.c_int, [_P, _P, _P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int64, _P, _P, _P]),
+    "smt_swiglu_forward": (C.c_int, [_P, _P, C.c_int64, _P, _P]),
+    "smt_swiglu_backward": (C.c_int, [_P, _P, _P, C.c_int64, _P, _P, _P]),
     "smt_grad_sqnorm_workspace_bytes": (C.c_size_t, []),
     "smt_grad_sqnorm": (C.c_int, [_P, C.c_int, C.c_int64, _P, _P, C.c_size_t, _P]),
     "smt_compact_adam": (C.c_int, [_P, _P, _P, _P, C.c_int, C.c_int64,

@@ -16,7 +16,7 @@ CSRC = os.path.join(HERE, "csrc")
 OUT_DIR = os.path.join(HERE, "_C")
 LIB_PATH = os.path.join(OUT_DIR, "libsmt_b200.so")
 SOURCES = ["capi.cu", "score_kernels.cu", "topk_kernel.cu", "block_copy_kernels.cu", "channel_kernels.cu", "adam_kernels.cu",
-           "block_grad_gemm.cu", "block_grad_runs.cu", "dense_gemm.cu"]
+           "block_grad_gemm.cu", "block_grad_runs.cu", "dense_gemm.cu", "decoder_kernels.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden"]
 

@@ -22,7 +22,7 @@ extern "C" SMT_API const char* smt_last_error(void) { return smt::g_err; }
 
 extern "C" SMT_API int smt_last_launch_count(void) { return smt::g_launches; }
 
-extern "C" SMT_API int smt_version(void) { return 200; /* 0.2.0: smt_gemm_item v2 (flags, sq_slot), sq partials, fused dense GEMMs */ }
+extern "C" SMT_API int smt_version(void) { return 210; /* 0.2.1: + decoder-layer elementwise kernels (RMSNorm, RoPE, SwiGLU) */ }
 
 extern "C" SMT_API int smt_device_info(int* sm_count_host, int* cc_major_host, int* cc_minor_host) {
   int dev = 0;

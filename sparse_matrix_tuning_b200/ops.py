@@ -534,6 +534,102 @@ def fused_linear_dgrad(dys: Sequence[torch.Tensor], weights: Sequence[torch.Tens
     return dx
 
 
+# ---- elementwise work of a LLaMA decoder layer (RMSNorm, RoPE, SwiGLU) ----------------------------------------------
+
+def _bf16_operands(*ts) -> None:
+    require_cuda(*ts)
+    for t in ts:
+        if t is not None:
+            _req(t.dtype == torch.bfloat16 and t.is_contiguous() and t.data_ptr() % 16 == 0,
+                 "contiguous, 16-byte aligned bfloat16 tensors")
+
+
+def rmsnorm_forward(a: torch.Tensor, weight: torch.Tensor, eps: float, res: Optional[torch.Tensor] = None):
+    """RMSNorm over the last dimension of `a` (or of h = bf16(res + a)).  Returns (y, rstd [rows] fp32, h or None)."""
+    _bf16_operands(a, weight, res)
+    H = a.shape[-1]
+    _req(weight.shape == (H,) and (res is None or res.shape == a.shape), "weight [H] and res of a's shape")
+    T = a.numel() // H if H else 0
+    y = torch.empty_like(a)
+    h = torch.empty_like(a) if res is not None else None
+    rstd = torch.empty(T, dtype=torch.float32, device=a.device)
+    check(load().smt_rmsnorm_forward(ptr(a), ptr(res), ptr(weight), T, H, float(eps), ptr(h), ptr(y), ptr(rstd), _st(a)),
+          "smt_rmsnorm_forward")
+    if T > 0:
+        _count()
+    return y, rstd, h
+
+
+def rmsnorm_backward(x: torch.Tensor, weight: torch.Tensor, rstd: torch.Tensor, dy: torch.Tensor,
+                     dres: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """Input gradient of `rmsnorm_forward` for a frozen weight, plus `dres` (the residual stream's gradient) if given."""
+    _bf16_operands(x, weight, dy, dres)
+    H = x.shape[-1]
+    T = x.numel() // H if H else 0
+    _req(dy.shape == x.shape and (dres is None or dres.shape == x.shape) and weight.shape == (H,),
+         "dy and dres of x's shape, weight [H]")
+    _req(rstd.dtype == torch.float32 and rstd.is_contiguous() and rstd.numel() == T, "fp32 rstd with one entry per row")
+    dx = torch.empty_like(x)
+    check(load().smt_rmsnorm_backward(ptr(x), ptr(weight), ptr(rstd), ptr(dy), ptr(dres), T, H, ptr(dx), _st(x)),
+          "smt_rmsnorm_backward")
+    if T > 0:
+        _count()
+    return dx
+
+
+def _rope(fn_name: str, q: torch.Tensor, k: torch.Tensor, cos: torch.Tensor, sin: torch.Tensor):
+    _bf16_operands(q, k)
+    require_cuda(cos, sin)
+    _req(q.dim() == 4 and k.dim() == 4 and q.shape[:2] == k.shape[:2] and q.shape[3] == 128 and k.shape[3] == 128,
+         "q [B, S, Hq, 128] and k [B, S, Hk, 128]")
+    B, S, Hq, _ = q.shape
+    Hk = k.shape[2]
+    _req(cos.shape == sin.shape and cos.dim() == 3 and cos.shape[1:] == (S, 128) and cos.shape[0] in (1, B)
+         and cos.dtype == torch.bfloat16 and sin.dtype == torch.bfloat16, "bf16 cos / sin of shape [1 or B, S, 128]")
+    _req(cos.stride() == sin.stride() and cos.stride()[1:] == (128, 1) and cos.data_ptr() % 16 == 0
+         and sin.data_ptr() % 16 == 0 and cos.stride(0) % 8 == 0, "cos / sin with rows of 128 contiguous elements")
+    bstride = 0 if cos.shape[0] == 1 else cos.stride(0)
+    qo, ko = torch.empty_like(q), torch.empty_like(k)
+    check(getattr(load(), fn_name)(ptr(q), ptr(k), ptr(cos), ptr(sin), B, S, Hq, Hk, bstride, ptr(qo), ptr(ko), _st(q)),
+          fn_name)
+    if q.numel() + k.numel() > 0:
+        _count()
+    return qo, ko
+
+
+def rope_forward(q: torch.Tensor, k: torch.Tensor, cos: torch.Tensor, sin: torch.Tensor):
+    """HF `apply_rotary_pos_emb` on q [B, S, Hq, 128] and k [B, S, Hk, 128] (contiguous) in ONE launch."""
+    return _rope("smt_rope_forward", q, k, cos, sin)
+
+
+def rope_backward(dq_out: torch.Tensor, dk_out: torch.Tensor, cos: torch.Tensor, sin: torch.Tensor):
+    """Gradients of q and k through `rope_forward`, in ONE launch."""
+    return _rope("smt_rope_backward", dq_out, dk_out, cos, sin)
+
+
+def swiglu_forward(g: torch.Tensor, u: torch.Tensor) -> torch.Tensor:
+    """bf16(bf16(silu(g)) * u), elementwise."""
+    _bf16_operands(g, u)
+    _req(g.shape == u.shape and g.numel() % 8 == 0, "g and u of one shape, numel % 8 == 0")
+    h = torch.empty_like(g)
+    check(load().smt_swiglu_forward(ptr(g), ptr(u), g.numel(), ptr(h), _st(g)), "smt_swiglu_forward")
+    if g.numel():
+        _count()
+    return h
+
+
+def swiglu_backward(g: torch.Tensor, u: torch.Tensor, dh: torch.Tensor):
+    """(dg, du) of `swiglu_forward` in ONE pass over g, u and dh."""
+    _bf16_operands(g, u, dh)
+    _req(g.shape == u.shape == dh.shape and g.numel() % 8 == 0, "g, u and dh of one shape, numel % 8 == 0")
+    dg, du = torch.empty_like(g), torch.empty_like(u)
+    check(load().smt_swiglu_backward(ptr(g), ptr(u), ptr(dh), g.numel(), ptr(dg), ptr(du), _st(g)),
+          "smt_swiglu_backward")
+    if g.numel():
+        _count()
+    return dg, du
+
+
 # ---- optimizer ---------------------------------------------------------------------------------------------
 
 def grad_sqnorm(grad: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:

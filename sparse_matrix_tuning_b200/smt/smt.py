@@ -33,13 +33,14 @@ from __future__ import annotations
 import contextlib
 import re
 import threading
+import warnings
 import weakref
 from typing import Dict, Tuple
 
 import torch
 from torch import nn
 
-from .. import ops
+from .. import decoder_fusion, ops
 from .._lib import SMTLibraryError
 
 Block_dimension = 256
@@ -325,8 +326,10 @@ class LinearLayer_MatrixSparsity(nn.Module):
 # layer into a group: the first call (q_proj) runs ONE hand-written tcgen05 GEMM over [Wq; Wk; Wv] and hands k_proj /
 # v_proj their slices when they are called with the same tensor; backward runs ONE GEMM over K = 4096 + 1024 + 1024
 # for the input gradient and feeds the block-gradient path of each sparse member.  Module names, parameters and
-# state dicts are untouched (the override is an instance attribute); members may be LinearLayer_MatrixSparsity or frozen,
-# bias-free nn.Linear.  Anything the kernel does not support falls back to the members' own forward.
+# state dicts are untouched (the override is a method bound to the instance); members may be LinearLayer_MatrixSparsity
+# or frozen, bias-free nn.Linear.  Anything the kernel does not support falls back to the members' own forward.
+# The same call also moves the layer's elementwise ops (norms, residual add, RoPE, SwiGLU) onto native kernels
+# (decoder_fusion.py).
 
 class fusedLinearZ(torch.autograd.Function):
     """forward(ctx, input, group, *selected_weights of the sparse members) -> one output per member."""
@@ -410,10 +413,18 @@ def _fusable_member(m) -> bool:
     return isinstance(m, nn.Linear) and m.bias is None and not m.weight.requires_grad
 
 
+def _shared_group_forward(self, x):
+    return self._smt_shared_group.call(self._smt_group_role, self, x)
+
+
 def fuse_qkv_projections(model) -> int:
-    """Ties q_proj / k_proj / v_proj of every attention module into one fused dense GEMM per direction (see above).
-    Returns the number of layers fused.  Call after `convert_linear_layer_to_matrix_sparsity`; undone by
-    `unfuse_qkv_projections` (and automatically by `convert_matrix_sparsity_to_linear_layer`)."""
+    """Fuses the dense-side work of every decoder layer it can: q_proj / k_proj / v_proj of each attention module become
+    one fused dense GEMM per direction (see above), and in a LLaMA decoder layer whose projections were fused the
+    elementwise ops around them - the two RMSNorms with the residual add, RoPE and SwiGLU - run on the native kernels of
+    `decoder_fusion` (the model's final norm too).  Returns the number of layers whose projections were fused.  Call
+    after `convert_linear_layer_to_matrix_sparsity`; undone by `unfuse_qkv_projections` (and automatically by
+    `convert_matrix_sparsity_to_linear_layer`).  The overrides are methods bound to each module, so a `copy.deepcopy`
+    of the model computes with the copy's weights."""
     fused = 0
     for parent in model.modules():
         trio = [getattr(parent, n, None) for n in ("q_proj", "k_proj", "v_proj")]
@@ -428,18 +439,34 @@ def fuse_qkv_projections(model) -> int:
         group = _SharedInputGroup(trio)
         for role, mod in enumerate(trio):
             mod._smt_shared_group = group
-            mod.forward = (lambda x, _g=group, _r=role, _m=mod: _g.call(_r, _m, x))
+            mod._smt_group_role = role
+            decoder_fusion.install_forward(mod, _shared_group_forward)
         fused += 1
+    layers = [m for m in model.modules() if getattr(getattr(getattr(m, "self_attn", None), "q_proj", None),
+                                                   "_smt_shared_group", None) is not None]
+    n_elementwise = sum(decoder_fusion.install_layer(m) for m in layers)
+    if n_elementwise:
+        for m in model.modules():
+            if isinstance(getattr(m, "layers", None), nn.ModuleList) and any(l in layers for l in m.layers):
+                decoder_fusion.install_norm(getattr(m, "norm", None))
+    if n_elementwise < len(layers):
+        warnings.warn(f"fuse_qkv_projections: elementwise ops of {len(layers) - n_elementwise} of {len(layers)} decoder "
+                      "layers left to transformers (not a LLaMA decoder layer of the supported transformers version, "
+                      "head_dim 128, SiLU)")
     return fused
 
 
 def unfuse_qkv_projections(model) -> int:
+    """Restores every module `fuse_qkv_projections` touched to its class's own forward; returns the number of q/k/v
+    groups undone."""
     n = 0
     for mod in model.modules():
         if getattr(mod, "_smt_shared_group", None) is not None:
-            mod.__dict__.pop("forward", None)
+            decoder_fusion.remove_forward(mod)
             mod.__dict__.pop("_smt_shared_group", None)
+            mod.__dict__.pop("_smt_group_role", None)
             n += 1
+    decoder_fusion.remove_all(model)
     return n // 3
 
 
