@@ -277,6 +277,19 @@ SMT_API int smt_swiglu_forward(const void* g, const void* u, int64_t n, void* h,
 SMT_API int smt_swiglu_backward(const void* g, const void* u, const void* dh, int64_t n, void* dg, void* du,
                                 void* stream);
 
+/* ---- causal-LM loss --------------------------------------------------------------------- */
+
+/* Causal-LM cross-entropy over rows of bf16 logits (transformers' ForCausalLMLoss for one chunk of rows), with the
+ * gradient written over the logits:
+ *   lse_t   = m_t + log(sum_v exp(x[t,v] - m_t))                          (fp32)
+ *   loss[t] = lse_t - x[t, y_t]   (0 where y_t == ignore_index; NaN where y_t is outside [0, V))
+ *   x[t,v] <- bf16(scale * (exp(x[t,v] - lse_t) - [v == y_t]))            (the whole row 0 where y_t == ignore_index,
+ *                                                                          NaN where y_t is outside [0, V))
+ * scale: device fp32 scalar (1 / number of valid labels, or 1 / num_items_in_batch), read on the device (no host sync).
+ * V % 8 == 0, ldl % 8 == 0, 16-byte aligned logits; int64 labels.  Deterministic (no atomics). */
+SMT_API int smt_cross_entropy_rows(void* logits, int64_t ldl, int64_t T, int V, const int64_t* labels,
+                                   int64_t ignore_index, const float* scale, float* loss_rows, void* stream);
+
 /* ---- compact optimizer ---------------------------------------------------------------- */
 
 /* out_sqnorm[0] = sum grad[i]^2 (fp32, deterministic two-stage tree). workspace: 4 KiB floats. */

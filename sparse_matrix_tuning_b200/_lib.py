@@ -89,6 +89,7 @@ _SIGNATURES = {
     "smt_rope_backward": (C.c_int, [_P, _P, _P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int64, _P, _P, _P]),
     "smt_swiglu_forward": (C.c_int, [_P, _P, C.c_int64, _P, _P]),
     "smt_swiglu_backward": (C.c_int, [_P, _P, _P, C.c_int64, _P, _P, _P]),
+    "smt_cross_entropy_rows": (C.c_int, [_P, C.c_int64, C.c_int64, C.c_int, _P, C.c_int64, _P, _P, _P]),
     "smt_grad_sqnorm_workspace_bytes": (C.c_size_t, []),
     "smt_grad_sqnorm": (C.c_int, [_P, C.c_int, C.c_int64, _P, _P, C.c_size_t, _P]),
     "smt_compact_adam": (C.c_int, [_P, _P, _P, _P, C.c_int, C.c_int64,

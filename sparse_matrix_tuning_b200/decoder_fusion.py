@@ -17,6 +17,10 @@ Each override takes the native path only for CUDA bf16 tensors of a supported sh
 cache; anything else runs the class's own `forward`.  The overrides are bound with `types.MethodType`, so
 `copy.deepcopy` of a model rebinds them to the copy.  Installed and removed by `smt.fuse_qkv_projections` /
 `smt.unfuse_qkv_projections`.
+
+`install_causal_lm(model)` (`smt.fuse_causal_lm_loss`) overrides `LlamaForCausalLM.forward` so that a training call with
+labels runs the frozen lm_head and the causal-LM cross-entropy chunk by chunk (`LinearCrossEntropyFn`, the kernel of
+`csrc/loss_kernels.cu`) and never materialises the fp32 logits; such a call returns `logits=None`.
 """
 from __future__ import annotations
 
@@ -110,6 +114,58 @@ class SwiGLUFn(torch.autograd.Function):
         g, u = ctx.saved_tensors
         dg, du = ops.swiglu_backward(g, u, dh.contiguous())
         return dg, du
+
+
+# Rows of logits per chunk of `LinearCrossEntropyFn`, a multiple of 256 (the GEMM's M tile, so that results do not depend
+# on it).  Measured on one B200 (1 000 W), lm_head + loss forward + backward at T = 8 192, K = 4 096, V = 128 256
+# (profiles/r04_causal_lm_loss.md): chunks of 2 048 / 4 096 / 8 192 rows take 14.1-14.4 ms in two runs (medians; single
+# repetitions differ by up to 1 ms), with 0.66 / 1.19 / 2.24 GB of peak memory above the inputs; 1 024 rows take
+# 14.5-14.7 ms (the input-gradient GEMM then has 64 tiles for 74 CTA pairs).  2 048 is the smallest transient at no
+# measured cost.
+_CE_CHUNK_ROWS = 2048
+
+
+class LinearCrossEntropyFn(torch.autograd.Function):
+    """loss = sum_t CE(h_t W^T, y_t) / denom for h [T, K] (bf16) and a frozen W [V, K]; labels y [T] (int64, shifted).
+
+    The input gradient is computed in forward, chunk by chunk: logits = h_c W^T (bf16), the loss kernel overwrites
+    them with d loss / d logits, dh_c = dlogits W.  Only one chunk of bf16 logits exists at a time and no fp32 logits at
+    all; the saved state is dh [T, K].  Backward returns dh * grad_output (exact for grad_output == 1)."""
+
+    @staticmethod
+    def forward(ctx, h, weight, labels, denom, ignore_index):
+        T = h.shape[0]
+        scale = denom.float().reciprocal().reshape(1)      # the fp32 1/denom autograd of HF's loss propagates
+        loss_rows = torch.empty(T, dtype=torch.float32, device=h.device)
+        dh = torch.empty_like(h)
+        for s in range(0, T, _CE_CHUNK_ROWS):
+            e = min(T, s + _CE_CHUNK_ROWS)
+            logits = ops.fused_linear_forward(h[s:e], [weight])[0]
+            loss_rows[s:e] = ops.cross_entropy_rows(logits, labels[s:e], scale, ignore_index)
+            ops.fused_linear_dgrad([logits], [weight], out=dh[s:e])
+            del logits
+        ctx.save_for_backward(dh)
+        return loss_rows.sum() / denom
+
+    @staticmethod
+    def backward(ctx, grad_output):
+        dh, = ctx.saved_tensors
+        return dh * grad_output, None, None, None, None
+
+
+def causal_lm_loss(h, weight, labels, ignore_index=-100, shift_labels=None, num_items_in_batch=None, **_):
+    """transformers' `ForCausalLMLoss(h @ weight.T, labels, ...)` through `LinearCrossEntropyFn`: labels shifted (or
+    `shift_labels` as given), mean over the labels that are not `ignore_index`, or sum / `num_items_in_batch`."""
+    if shift_labels is None:
+        labels = nn.functional.pad(labels, (0, 1), value=ignore_index)
+        shift_labels = labels[..., 1:]
+    y = shift_labels.reshape(-1).to(device=h.device, dtype=torch.int64).contiguous()
+    h2 = h.reshape(-1, h.shape[-1]).contiguous()
+    if num_items_in_batch is None:
+        denom = (y != ignore_index).sum()                   # on the device: no host sync
+    else:
+        denom = torch.as_tensor(num_items_in_batch, device=h.device)
+    return LinearCrossEntropyFn.apply(h2, weight, y, denom, int(ignore_index))
 
 
 # ---- when the native path applies ------------------------------------------------------------------------------------
@@ -230,6 +286,41 @@ def _decoder_forward(self, hidden_states, attention_mask=None, position_ids=None
     return residual + hidden_states
 
 
+def _lm_head_ok(model, h) -> bool:
+    head = model.lm_head
+    if type(head) is not nn.Linear or head.bias is not None:
+        return False
+    w = head.weight
+    return _native(h, w) and h.requires_grad and not w.requires_grad and w.shape[0] == model.config.vocab_size \
+        and h.shape[-1] == w.shape[1] and w.shape[0] % 8 == 0 and ops.fused_linear_supported([w]) \
+        and ops.fused_linear_supported([w], dgrad=True)
+
+
+def _causal_lm_forward(self, input_ids=None, attention_mask=None, position_ids=None, past_key_values=None,
+                       inputs_embeds=None, labels=None, use_cache=None, logits_to_keep=0, **kwargs):
+    args = dict(input_ids=input_ids, attention_mask=attention_mask, position_ids=position_ids,
+                past_key_values=past_key_values, inputs_embeds=inputs_embeds, use_cache=use_cache)
+    if labels is None or not isinstance(logits_to_keep, int) or logits_to_keep != 0 or past_key_values is not None \
+            or not torch.is_grad_enabled() or getattr(_hf_only, "depth", 0):
+        return type(self).forward(self, **args, labels=labels, logits_to_keep=logits_to_keep, **kwargs)
+    # `return_dict` as transformers' `can_return_tuple` resolves it
+    return_dict = self.config.return_dict if hasattr(self, "config") else True
+    passed = kwargs.pop("return_dict", return_dict)
+    if passed is not None:
+        return_dict = passed
+    outputs = self.model(**args, **kwargs)
+    h = outputs.last_hidden_state
+    if outputs.past_key_values is None and self.loss_function is _causal_lm_loss_fn() and _lm_head_ok(self, h):
+        loss = causal_lm_loss(h, self.lm_head.weight, labels, **kwargs)
+        logits = None
+    else:
+        logits = self.lm_head(h)
+        loss = self.loss_function(logits=logits, labels=labels, vocab_size=self.config.vocab_size, **kwargs)
+    out = _llama().CausalLMOutputWithPast(loss=loss, logits=logits, past_key_values=outputs.past_key_values,
+                                          hidden_states=outputs.hidden_states, attentions=outputs.attentions)
+    return out if return_dict else out.to_tuple()
+
+
 # ---- version guard and installation ----------------------------------------------------------------------------------
 
 _EXPECTED_PARAMS = {
@@ -238,6 +329,8 @@ _EXPECTED_PARAMS = {
     "LlamaAttention": ["self", "hidden_states", "position_embeddings", "attention_mask", "past_key_values", "kwargs"],
     "LlamaDecoderLayer": ["self", "hidden_states", "attention_mask", "position_ids", "past_key_values", "use_cache",
                           "position_embeddings", "kwargs"],
+    "LlamaForCausalLM": ["self", "input_ids", "attention_mask", "position_ids", "past_key_values", "inputs_embeds",
+                         "labels", "use_cache", "logits_to_keep", "kwargs"],
 }
 _llama_mod = None
 
@@ -248,6 +341,11 @@ def _llama():
         from transformers.models.llama import modeling_llama
         _llama_mod = modeling_llama
     return _llama_mod
+
+
+def _causal_lm_loss_fn():
+    from transformers.loss.loss_utils import ForCausalLMLoss
+    return ForCausalLMLoss
 
 
 def _class_matches(module, name: str) -> bool:
@@ -289,6 +387,21 @@ def install_norm(norm) -> bool:
         return False
     install_forward(norm, _rmsnorm_forward)
     return True
+
+
+def install_causal_lm(model) -> bool:
+    """The fused lm_head + causal-LM loss override on a `LlamaForCausalLM`; False for any other class."""
+    if not _class_matches(model, "LlamaForCausalLM"):
+        return False
+    install_forward(model, _causal_lm_forward)
+    return True
+
+
+def remove_causal_lm(model) -> bool:
+    """Undo `install_causal_lm`; False when the model had no such override."""
+    if getattr(model.__dict__.get("forward"), "__func__", None) is not _causal_lm_forward:
+        return False
+    return remove_forward(model)
 
 
 def remove_all(model) -> int:

@@ -512,8 +512,10 @@ def fused_linear_forward(x2d: torch.Tensor, weights: Sequence[torch.Tensor]) -> 
     return ys
 
 
-def fused_linear_dgrad(dys: Sequence[torch.Tensor], weights: Sequence[torch.Tensor]) -> torch.Tensor:
-    """sum_j dy_j @ W_j in ONE tcgen05 launch (smt.py:406 for every module that reads x, plus autograd's adds)."""
+def fused_linear_dgrad(dys: Sequence[torch.Tensor], weights: Sequence[torch.Tensor],
+                       out: Optional[torch.Tensor] = None) -> torch.Tensor:
+    """sum_j dy_j @ W_j in ONE tcgen05 launch (smt.py:406 for every module that reads x, plus autograd's adds).
+    `out`: optional [T, K] destination with unit column stride (e.g. a row slice of a larger buffer)."""
     require_cuda(*dys, *weights)
     _req(len(dys) == len(weights) and len(dys) >= 1, "len(dys) == len(weights) >= 1")
     T, K = dys[0].shape[0], weights[0].shape[1]
@@ -521,14 +523,20 @@ def fused_linear_dgrad(dys: Sequence[torch.Tensor], weights: Sequence[torch.Tens
         _req(dy.dim() == 2 and dy.stride(1) == 1 and dy.shape == (T, w.shape[0]) and dy.dtype == w.dtype,
              "dy.dim() == 2 and dy.stride(1) == 1 and dy.shape == (T, N_j) and dy.dtype == w.dtype")
         _req(dy.data_ptr() % 16 == 0 and (dy.stride(0) * 2) % 16 == 0, "16-byte aligned dy")
-    dx = torch.empty(T, K, dtype=dys[0].dtype, device=dys[0].device)
+    if out is None:
+        dx = torch.empty(T, K, dtype=dys[0].dtype, device=dys[0].device)
+    else:
+        require_cuda(out)
+        _req(out.shape == (T, K) and out.dtype == dys[0].dtype and out.stride(1) == 1 and out.data_ptr() % 16 == 0
+             and (out.stride(0) * 2) % 16 == 0, "out [T, K] of dy's dtype, unit column stride, 16-byte aligned rows")
+        dx = out
     n = len(weights)
     wp, wl = _seg_arrays(weights)
     dp_, dl = _seg_arrays(dys)
     ns = (C.c_int * n)(*[int(w.shape[0]) for w in weights])
     with _timed("fused_linear_dgrad", dx.device, (T, K, sum(w.shape[0] for w in weights))):
-        check(load().smt_fused_linear_dgrad(dp_, dl, T, K, n, wp, wl, ns, ptr(dx), K, dtype_id(dx.dtype), _st(dx)),
-              "smt_fused_linear_dgrad")
+        check(load().smt_fused_linear_dgrad(dp_, dl, T, K, n, wp, wl, ns, ptr(dx), dx.stride(0) if T > 0 else K,
+                                            dtype_id(dx.dtype), _st(dx)), "smt_fused_linear_dgrad")
     if T > 0:
         _count()
     return dx
@@ -628,6 +636,29 @@ def swiglu_backward(g: torch.Tensor, u: torch.Tensor, dh: torch.Tensor):
     if g.numel():
         _count()
     return dg, du
+
+
+# ---- causal-LM loss --------------------------------------------------------------------------------------------------
+
+def cross_entropy_rows(logits: torch.Tensor, labels: torch.Tensor, scale: torch.Tensor,
+                       ignore_index: int = -100) -> torch.Tensor:
+    """Per-row cross-entropy of bf16 `logits` [T, V] against int64 `labels` [T]; returns the fp32 losses [T] (0 for
+    `ignore_index`, NaN for a label outside [0, V)) and OVERWRITES `logits` with the gradient of sum(loss) * scale.
+    `scale`: fp32 device scalar, read on the device."""
+    require_cuda(logits, labels, scale)
+    _req(logits.dim() == 2 and logits.dtype == torch.bfloat16 and logits.stride(1) == 1
+         and logits.stride(0) % 8 == 0 and logits.data_ptr() % 16 == 0 and logits.shape[1] % 8 == 0,
+         "bf16 logits [T, V] with V % 8 == 0, unit column stride, row pitch % 8 == 0 and 16-byte alignment")
+    T, V = logits.shape
+    _req(labels.dtype == torch.int64 and labels.is_contiguous() and labels.shape == (T,), "contiguous int64 labels [T]")
+    _req(scale.dtype == torch.float32 and scale.numel() == 1, "fp32 scale with one element")
+    loss = torch.empty(T, dtype=torch.float32, device=logits.device)
+    check(load().smt_cross_entropy_rows(ptr(logits), logits.stride(0) if T > 0 else V, T, V, ptr(labels),
+                                        int(ignore_index), ptr(scale), ptr(loss), _st(logits)),
+          "smt_cross_entropy_rows")
+    if T > 0:
+        _count()
+    return loss
 
 
 # ---- optimizer ---------------------------------------------------------------------------------------------

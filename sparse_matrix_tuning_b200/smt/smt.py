@@ -470,6 +470,23 @@ def unfuse_qkv_projections(model) -> int:
     return n // 3
 
 
+def fuse_causal_lm_loss(model) -> bool:
+    """Runs a `LlamaForCausalLM`'s lm_head and causal-LM cross-entropy as one chunked native op that never builds the
+    fp32 logits (`decoder_fusion.LinearCrossEntropyFn`).  It applies to training calls with `labels` (grad mode on,
+    `logits_to_keep=0`, no KV cache, CUDA bf16, a frozen bias-free lm_head with `out_features == vocab_size`); those
+    return the loss with `logits=None`.  `shift_labels`, `ignore_index` and `num_items_in_batch` are honoured as
+    transformers' `ForCausalLMLoss` honours them.  Every other call runs the class's own forward, so evaluation under
+    `no_grad` still gets logits.  Returns False (and changes nothing) for any other model class.  The override is a
+    method bound to the model, so a `copy.deepcopy` computes with the copy's weights; undone by
+    `unfuse_causal_lm_loss`."""
+    return decoder_fusion.install_causal_lm(model)
+
+
+def unfuse_causal_lm_loss(model) -> bool:
+    """Restores the class's own forward on a model `fuse_causal_lm_loss` touched; False when there was nothing to undo."""
+    return decoder_fusion.remove_causal_lm(model)
+
+
 # ---- model surgery ---------------------------------------------------------------------------------------
 
 def _selection_key_and_table(name: str, mixture: bool, selected_submatrix, selected_submatrix_attention):
