@@ -82,6 +82,22 @@ SMT_API int smt_block_sum_finalize(const float* block_sums, float* scores, int64
 SMT_API int smt_block_score_reduce(const float* acc, int rows, int cols, int64_t ld, int block,
                            int strategy, float* scores, void* stream);
 
+/* Factored block sums for a frozen-weight warm-up — replace fine_tune.py:716-768 (capture of every q/k/v(/MLP)
+ * weight gradient) and smt_helper.py:55-78 (its reduction to b x b blocks) for `mean_abs`, without forming dW.
+ * For y = x W^T:  sum_{o in r, k in c} dW[o, k] = sum_t Dy[t, r] * X[t, c],  with Dy, X the per-token block sums of
+ * dy and x below.  Both calls are deterministic (fixed reduction order, no atomics, nothing depends on the SM count)
+ * and no-ops for T = 0, even with NULL pointers.
+ *
+ * out[t, j] = sum_{k < b} src[t, j*b + k]  (fp32).  src: [T, F] row-major, `dtype` (F32 / BF16 / F16), row pitch `ld`
+ * elements, unit column stride, 16-byte aligned base and pitch; F % b == 0; out: contiguous [T, F/b] fp32. */
+SMT_API int smt_token_block_sums(const void* src, int dtype, int64_t T, int F, int64_t ld, int block, float* out,
+                                 void* stream);
+/* block_sums[r, c] += sum_t dy_sums[t, r] * x_sums[t, c]  — contiguous fp32 [rb, cb], [T, rb], [T, cb].
+ * T is split into fixed chunks of 128 tokens whose partial products go to `workspace`, then added in chunk order. */
+SMT_API size_t smt_block_outer_accumulate_workspace_bytes(int64_t T, int rb, int cb);
+SMT_API int smt_block_outer_accumulate(float* block_sums, const float* dy_sums, const float* x_sums, int64_t T,
+                                       int rb, int cb, void* workspace, size_t workspace_bytes, void* stream);
+
 /* acc[S, C] += sum_b |x[b, S, C]|  — the activation hook of fine_tune.py:649-678 reduced over the
  * batch dimension, which is all smt_helper.py:170 consumes. */
 SMT_API int smt_act_score_accumulate(float* acc, const void* x, int x_dtype, int batch, int seq, int channels,

@@ -55,6 +55,9 @@ _SIGNATURES = {
     "smt_block_sum_accumulate": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_int64, C.c_int, _P]),
     "smt_block_sum_finalize": (C.c_int, [_P, _P, C.c_int64, C.c_int, _P]),
     "smt_block_score_reduce": (C.c_int, [_P, C.c_int, C.c_int, C.c_int64, C.c_int, C.c_int, _P, _P]),
+    "smt_token_block_sums": (C.c_int, [_P, C.c_int, C.c_int64, C.c_int, C.c_int64, C.c_int, _P, _P]),
+    "smt_block_outer_accumulate_workspace_bytes": (C.c_size_t, [C.c_int64, C.c_int, C.c_int]),
+    "smt_block_outer_accumulate": (C.c_int, [_P, _P, _P, C.c_int64, C.c_int, C.c_int, _P, C.c_size_t, _P]),
     "smt_act_score_accumulate": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.c_int, _P]),
     "smt_channel_score_reduce": (C.c_int, [_P, C.c_int, C.c_int, C.c_int, _P, _P]),
     "smt_topk_workspace_bytes": (C.c_size_t, [C.c_int64]),

@@ -1,10 +1,13 @@
 // Warm-up scoring kernels (HBM-bound): elementwise fp32 accumulation of gradients, per-block
-// signed-sum accumulation, block-score reduction with the four reference strategies, and the
+// signed-sum accumulation, block-score reduction with the four reference strategies, the factored
+// block sums of a frozen-weight warm-up (token block sums + their outer product), and the
 // activation (channel) scoring pair.
 //
 // Reference call sites replaced (paths relative to the reference root):
 //   deepspeed/fine_tune.py:716-768   D2H copy + CPU `+=` of every q/k/v(/MLP) gradient
 //   deepspeed/smt/smt_helper.py:55-78, 233-251   reshape to [R/b, b, C/b, b] and reduce dims (1,3)
+//   (smt_token_block_sums + smt_block_outer_accumulate replace both of the above for `mean_abs`
+//    without the weight gradient ever being formed)
 //   deepspeed/fine_tune.py:649-678   activation hook (|x|, allreduce, D2H, `+=`)
 //   deepspeed/smt/smt_helper.py:168-183   channel scores
 #include "common.cuh"
@@ -234,6 +237,137 @@ __global__ void __launch_bounds__(kThreads) channel_score_reduce_kernel(
   }
 }
 
+// ---- factored block sums (frozen-weight warm-up) -------------------------------------------------
+// For y = x W^T the signed sum of block (r, c) of dW factors over tokens:
+//   sum_{o in r, k in c} dW[o, k] = sum_t Dy[t, r] * X[t, c],  Dy / X = per-token segment sums of dy / x.
+// token_block_sums_kernel makes Dy and X (one read of the activation), block_outer_* contracts them.
+
+#ifndef SMT_TBS_UNROLL
+#define SMT_TBS_UNROLL 4       // segment groups in flight per thread
+#endif
+
+// out[t, j] = sum_{k < B} src[t, j*B + k].  L lanes of a warp share one segment (L = min(vectors per segment, 32)),
+// each lane loads P = vectors / L 128-bit vectors of it; the lane sums run in a fixed order, then an xor butterfly over
+// the L lanes.  The arithmetic of a segment never depends on which warp handles it, so any grid gives the same bits.
+template <int B, int DT>
+__global__ void __launch_bounds__(kThreads) token_block_sums_kernel(
+    const void* __restrict__ src, int64_t ld, int64_t T, int seg_per_row, float* __restrict__ out) {
+  constexpr int ES = DT == SMT_F32 ? 4 : 2;
+  constexpr int VEC = 16 / ES;                          // elements per 128-bit vector
+  constexpr int NV = B / VEC;                           // vectors per segment: 8 .. 64
+  constexpr int L = NV < 32 ? NV : 32;                  // lanes per segment
+  constexpr int P = NV / L;                             // vectors per lane per segment
+  constexpr int SPW = 32 / L;                           // segments per warp and group
+  constexpr int U = SMT_TBS_UNROLL;
+  const int lane = threadIdx.x & 31, sub = lane / L, l = lane % L;
+  const int64_t n_seg = T * seg_per_row;
+  const int64_t n_groups = (n_seg + SPW - 1) / SPW;
+  const int64_t warps = (int64_t)gridDim.x * (kThreads / 32);
+  const char* base = reinterpret_cast<const char*>(src);
+  for (int64_t g0 = (int64_t)blockIdx.x * (kThreads / 32) + (threadIdx.x >> 5); g0 < n_groups; g0 += U * warps) {
+    uint4 v[U][P];
+#pragma unroll
+    for (int u = 0; u < U; ++u) {                       // all loads first: U x P x 16 B in flight per lane
+      const int64_t s = (g0 + u * warps) * SPW + sub;
+      const bool ok = s < n_seg;
+      int64_t t = 0, j = 0;
+      if (ok && n_seg <= 0xffffffffll) {                 // 32-bit division is far cheaper than 64-bit
+        t = (uint32_t)s / (uint32_t)seg_per_row;
+        j = (uint32_t)s - (uint32_t)t * (uint32_t)seg_per_row;
+      } else if (ok) {
+        t = s / seg_per_row;
+        j = s - t * seg_per_row;
+      }
+      const char* p = base + (t * ld + j * B) * ES + (int64_t)l * 16;
+#pragma unroll
+      for (int q = 0; q < P; ++q) v[u][q] = ok ? ld_stream_u4(p + q * L * 16) : make_uint4(0u, 0u, 0u, 0u);
+    }
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+      float acc = 0.f;
+#pragma unroll
+      for (int q = 0; q < P; ++q) {
+        if (DT == SMT_F32) {
+          acc += (__uint_as_float(v[u][q].x) + __uint_as_float(v[u][q].y)) +
+                 (__uint_as_float(v[u][q].z) + __uint_as_float(v[u][q].w));
+        } else {
+          float f[8];
+          unpack8<DT>(v[u][q], f);
+          acc += ((f[0] + f[1]) + (f[2] + f[3])) + ((f[4] + f[5]) + (f[6] + f[7]));
+        }
+      }
+#pragma unroll
+      for (int o = L / 2; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
+      const int64_t s = (g0 + u * warps) * SPW + sub;
+      if (l == 0 && s < n_seg) out[s] = acc;
+    }
+  }
+}
+
+// Tokens per partial of block_outer_accumulate: a fixed partition of T (independent of the device), so the sums are
+// bit-identical on every GPU and from run to run.  (Chunks of 512 tokens with four fma chains measured slower: 25-27 us
+// against 15-19 us at T = 8 192, fewer CTAs each waiting on two staging rounds.)
+constexpr int kOuterChunk = 128;
+constexpr int kOuterTile = 16;                          // 16 x 16 outputs per CTA, one per thread
+
+// part[k, r, c] = sum over the tokens of chunk k of dy[t, r] * x[t, c], tokens in increasing order.
+__global__ void __launch_bounds__(kThreads) block_outer_partial_kernel(
+    const float* __restrict__ dy, const float* __restrict__ x, int64_t T, int rb, int cb, float* __restrict__ part) {
+  __shared__ float sdy[kOuterChunk][kOuterTile];
+  __shared__ float sx[kOuterChunk][kOuterTile];
+  const int64_t t0 = (int64_t)blockIdx.x * kOuterChunk;
+  const int c0 = blockIdx.y * kOuterTile, r0 = blockIdx.z * kOuterTile;
+  for (int i = threadIdx.x; i < kOuterChunk * kOuterTile; i += kThreads) {
+    const int tt = i / kOuterTile, k = i % kOuterTile;
+    const int64_t t = t0 + tt;
+    sdy[tt][k] = (t < T && r0 + k < rb) ? dy[t * rb + r0 + k] : 0.f;
+    sx[tt][k] = (t < T && c0 + k < cb) ? x[t * cb + c0 + k] : 0.f;
+  }
+  __syncthreads();
+  const int ty = threadIdx.x / kOuterTile, tx = threadIdx.x % kOuterTile;
+  float acc = 0.f;
+#pragma unroll 8
+  for (int tt = 0; tt < kOuterChunk; ++tt) acc = fmaf(sdy[tt][ty], sx[tt][tx], acc);
+  const int r = r0 + ty, c = c0 + tx;
+  if (r < rb && c < cb) part[((int64_t)blockIdx.x * rb + r) * cb + c] = acc;
+}
+
+// block_sums[i] += sum_k part[k, i], k in increasing order (loads issued 8 at a time, the sum stays sequential).
+__global__ void __launch_bounds__(kThreads) block_outer_reduce_kernel(
+    const float* __restrict__ part, int64_t n_chunks, int64_t n, float* __restrict__ block_sums) {
+  const int64_t i = (int64_t)blockIdx.x * kThreads + threadIdx.x;
+  if (i >= n) return;
+  float s = 0.f;
+  int64_t k = 0;
+  for (; k + 8 <= n_chunks; k += 8) {
+    float v[8];
+#pragma unroll
+    for (int j = 0; j < 8; ++j) v[j] = part[(k + j) * n + i];
+#pragma unroll
+    for (int j = 0; j < 8; ++j) s += v[j];
+  }
+  for (; k < n_chunks; ++k) s += part[k * n + i];
+  block_sums[i] += s;
+}
+
+// One wave: at most as many CTAs as can be resident, so no CTA of a second partial wave runs its grid-stride loop
+// after the others have finished (the launches are 10-60 us long, so a tail wave is a large fraction of them).
+template <int B, int DT>
+void launch_token_block_sums(const void* src, int64_t ld, int64_t T, int seg_per_row, float* out, int64_t want,
+                             cudaStream_t st) {
+  static int per_sm = 0;
+  if (per_sm == 0) {
+    int o = 0;
+    if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&o, token_block_sums_kernel<B, DT>, kThreads, 0) != cudaSuccess ||
+        o <= 0)
+      o = 4;
+    per_sm = o;
+  }
+  const int64_t cap = (int64_t)sm_count() * per_sm;
+  const int grid = (int)(want < cap ? want : cap);
+  token_block_sums_kernel<B, DT><<<grid, kThreads, 0, st>>>(src, ld, T, seg_per_row, out);
+}
+
 inline int streaming_grid(int64_t work_items) {
   // enough CTAs for ~8 resident per SM, capped by the work
   int64_t want = (work_items + kThreads - 1) / kThreads;
@@ -337,6 +471,73 @@ extern "C" SMT_API int smt_block_sum_finalize(const float* block_sums, float* sc
   if (n <= 0) return SMT_OK;
   int grid = (int)((n + 255) / 256);
   block_sum_finalize_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(block_sums, scores, n, (float)(block * block));
+  SMT_CHECK_LAUNCH();
+  return SMT_OK;
+}
+
+extern "C" SMT_API int smt_token_block_sums(const void* src, int dtype, int64_t T, int F, int64_t ld, int block,
+                                            float* out, void* stream) {
+  SMT_CHECK_ARG(T >= 0 && F >= 0, "smt_token_block_sums: negative size (T = %lld, F = %d)", (long long)T, F);
+  SMT_CHECK_ARG(dtype >= SMT_F32 && dtype <= SMT_F16, "smt_token_block_sums: bad dtype %d", dtype);
+  SMT_CHECK_ARG(block_ok(block), "smt_token_block_sums: block size %d not in {64,128,256}", block);
+  SMT_CHECK_ARG(F % block == 0, "smt_token_block_sums: F = %d is not a multiple of block %d", F, block);
+  if (T == 0 || F == 0) return SMT_OK;
+  SMT_CHECK_ARG(src && out, "smt_token_block_sums: null pointer");
+  SMT_CHECK_ARG(ld >= F, "smt_token_block_sums: ld %lld < F %d", (long long)ld, F);
+  SMT_CHECK_ARG(aligned16(src) && (ld * dtype_bytes(dtype)) % 16 == 0,
+                "smt_token_block_sums: src must be 16-byte aligned (ptr and row pitch)");
+  SMT_CHECK_ARG((reinterpret_cast<uintptr_t>(out) & 3u) == 0, "smt_token_block_sums: out must be 4-byte aligned");
+  const int seg_per_row = F / block;
+  const int vec = dtype == SMT_F32 ? 4 : 8;
+  const int lanes = block / vec < 32 ? block / vec : 32;
+  const int64_t groups = (T * seg_per_row + 32 / lanes - 1) / (32 / lanes);   // one warp per group
+  const int64_t want = (groups + (kThreads / 32) * SMT_TBS_UNROLL - 1) / ((kThreads / 32) * SMT_TBS_UNROLL);
+  cudaStream_t st = (cudaStream_t)stream;
+#define SMT_LAUNCH_TBS(B)                                                                                            \
+  do {                                                                                                               \
+    if (dtype == SMT_F32) launch_token_block_sums<B, SMT_F32>(src, ld, T, seg_per_row, out, want, st);              \
+    else if (dtype == SMT_BF16) launch_token_block_sums<B, SMT_BF16>(src, ld, T, seg_per_row, out, want, st);       \
+    else launch_token_block_sums<B, SMT_F16>(src, ld, T, seg_per_row, out, want, st);                               \
+  } while (0)
+  if (block == 256) SMT_LAUNCH_TBS(256);
+  else if (block == 128) SMT_LAUNCH_TBS(128);
+  else SMT_LAUNCH_TBS(64);
+#undef SMT_LAUNCH_TBS
+  SMT_CHECK_LAUNCH();
+  return SMT_OK;
+}
+
+extern "C" SMT_API size_t smt_block_outer_accumulate_workspace_bytes(int64_t T, int rb, int cb) {
+  if (T <= 0 || rb <= 0 || cb <= 0) return 0;
+  return (size_t)((T + kOuterChunk - 1) / kOuterChunk) * (size_t)rb * (size_t)cb * sizeof(float);
+}
+
+extern "C" SMT_API int smt_block_outer_accumulate(float* block_sums, const float* dy_sums, const float* x_sums,
+                                                  int64_t T, int rb, int cb, void* workspace, size_t workspace_bytes,
+                                                  void* stream) {
+  SMT_CHECK_ARG(T >= 0 && rb >= 0 && cb >= 0, "smt_block_outer_accumulate: negative size (T = %lld, rb = %d, cb = %d)",
+                (long long)T, rb, cb);
+  if (T == 0 || rb == 0 || cb == 0) return SMT_OK;
+  SMT_CHECK_ARG(block_sums && dy_sums && x_sums && workspace, "smt_block_outer_accumulate: null pointer");
+  SMT_CHECK_ARG(((reinterpret_cast<uintptr_t>(block_sums) | reinterpret_cast<uintptr_t>(dy_sums) |
+                  reinterpret_cast<uintptr_t>(x_sums) | reinterpret_cast<uintptr_t>(workspace)) & 3u) == 0,
+                "smt_block_outer_accumulate: pointers must be 4-byte aligned");
+  const int64_t n_chunks = (T + kOuterChunk - 1) / kOuterChunk;
+  const size_t need = smt_block_outer_accumulate_workspace_bytes(T, rb, cb);
+  if (workspace_bytes < need) {
+    ::smt::set_error("smt_block_outer_accumulate: workspace %zu B < %zu B", workspace_bytes, need);
+    return SMT_ERR_WORKSPACE;
+  }
+  const int tiles_c = (cb + kOuterTile - 1) / kOuterTile, tiles_r = (rb + kOuterTile - 1) / kOuterTile;
+  SMT_CHECK_ARG(n_chunks <= 0x7fffffff && tiles_c <= 65535 && tiles_r <= 65535, "smt_block_outer_accumulate: too large");
+  cudaStream_t st = (cudaStream_t)stream;
+  float* part = static_cast<float*>(workspace);
+  block_outer_partial_kernel<<<dim3((unsigned)n_chunks, tiles_c, tiles_r), kThreads, 0, st>>>(dy_sums, x_sums, T, rb,
+                                                                                               cb, part);
+  SMT_CHECK_LAUNCH();
+  const int64_t n = (int64_t)rb * cb;
+  block_outer_reduce_kernel<<<(unsigned)((n + kThreads - 1) / kThreads), kThreads, 0, st>>>(part, n_chunks, n,
+                                                                                           block_sums);
   SMT_CHECK_LAUNCH();
   return SMT_OK;
 }

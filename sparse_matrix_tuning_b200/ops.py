@@ -153,6 +153,40 @@ def block_score_reduce(acc: torch.Tensor, block: int, strategy: str = "mean_abs"
     return out
 
 
+def token_block_sums(t2d: torch.Tensor, block: int) -> torch.Tensor:
+    """out[t, j] = sum_{k < b} t2d[t, j*b + k] as fp32 [T, F/b]: the per-token block sums of a module's input or output
+    gradient that `block_outer_accumulate` contracts into weight-gradient block sums (fine_tune.py:716-768 and
+    smt_helper.py:55-78 without the weight gradient)."""
+    require_cuda(t2d)
+    _req(t2d.dim() == 2 and t2d.stride(1) == 1, "t2d.dim() == 2 and t2d.stride(1) == 1")
+    T, F = t2d.shape
+    _req(block in (64, 128, 256) and F % block == 0, "block in (64, 128, 256) and F % block == 0")
+    out = torch.empty((T, F // block), dtype=torch.float32, device=t2d.device)
+    check(load().smt_token_block_sums(ptr(t2d), dtype_id(t2d.dtype), T, F, t2d.stride(0) if T > 0 else F, block,
+                                      ptr(out), _st(t2d)), "smt_token_block_sums")
+    if T > 0 and F > 0:
+        _count()
+    return out
+
+
+def block_outer_accumulate(block_sums: torch.Tensor, dy_sums: torch.Tensor, x_sums: torch.Tensor) -> None:
+    """block_sums[r, c] += sum_t dy_sums[t, r] * x_sums[t, c] (fp32, deterministic: a fixed partition of T)."""
+    require_cuda(block_sums, dy_sums, x_sums)
+    for t in (block_sums, dy_sums, x_sums):
+        _req(t.dim() == 2 and t.dtype == torch.float32 and t.is_contiguous(), "contiguous 2-D fp32 tensors")
+    T, rb = dy_sums.shape
+    cb = x_sums.shape[1]
+    _req(x_sums.shape[0] == T and tuple(block_sums.shape) == (rb, cb),
+         "dy_sums [T, rb], x_sums [T, cb] and block_sums [rb, cb]")
+    lib = load()
+    ws_bytes = lib.smt_block_outer_accumulate_workspace_bytes(T, rb, cb)
+    ws = _workspace(ws_bytes, block_sums.device, tag="block_outer")
+    check(lib.smt_block_outer_accumulate(ptr(block_sums), ptr(dy_sums), ptr(x_sums), T, rb, cb, ptr(ws), ws_bytes,
+                                         _st(block_sums)), "smt_block_outer_accumulate")
+    if T > 0 and rb * cb > 0:
+        _count(2)
+
+
 def act_score_accumulate(acc: torch.Tensor, x: torch.Tensor) -> None:
     """acc[S, C] += sum_b |x[b, S, C]|. fine_tune.py:649-678 (reduced over batch)."""
     require_cuda(acc, x)

@@ -14,6 +14,7 @@ statistic that q/k/v always use — fine_tune.py:306-313 never forwards `calcula
 from __future__ import annotations
 
 import re
+import weakref
 from typing import Callable, Dict, Iterable, Optional, Tuple
 
 import torch
@@ -138,6 +139,102 @@ class WarmupGradAccumulator:
             n = self.acc[k].numel()
             self.acc[k].copy_(flat[off:off + n].view_as(self.acc[k]))
             off += n
+
+
+class FactoredBlockSumAccumulator:
+    """Block sums of the targeted weight gradients of a FROZEN model, built from activations and output gradients.
+
+    For y = x W^T the signed sum of block (r, c) of dW factors over the tokens t:
+        sum_{o in r, k in c} dW[o, k] = sum_t Dy[t, r] * X[t, c],
+    Dy[t, r] = sum_{o in r} dy[t, o] and X[t, c] = sum_{k in c} x[t, k].  A forward hook on every targeted nn.Linear
+    reduces its input to X (`ops.token_block_sums`, one read of x; x itself is not kept), a tensor hook on its output
+    reduces dy to Dy in backward and adds Dy^T X to the module's [R/b, C/b] accumulator (`ops.block_outer_accumulate`).
+    No weight gradient is ever formed, so the model stays frozen and the warm-up pass can run the same fused path as
+    the training step (`fuse_qkv_projections`, `fuse_causal_lm_loss`).
+
+    Same surface as `WarmupGradAccumulator(mode="block_sum")` - `acc` / `shapes` keyed (module_name, layer),
+    `scores("mean_abs")`, `flat_state()` / `load_flat_state()` - so `dp.allreduce_block_sums` and
+    `smt_helper.select_submatrix_from_scores` take it unchanged.  Only `mean_abs` is linear in the gradient; `abs_mean`,
+    `L1` and `L2` need `WarmupGradAccumulator(mode="elementwise")`.
+
+    Usage - freezing is the caller's job:
+        for p in model.parameters(): p.requires_grad_(False)
+        model.enable_input_require_grads()          # the hidden states must require grad for dy to exist
+        fuse_qkv_projections(model); fuse_causal_lm_loss(model)            # optional
+        acc = FactoredBlockSumAccumulator(block=256).attach(model)  ... warm-up passes (forward + backward) ...
+        acc.detach(); keys, scores = acc.scores("mean_abs"); sel = select_submatrix_from_scores(keys, scores, n)
+        unfuse_qkv_projections(model)
+        freeze_unselected_matrix_layer(...); convert_linear_layer_to_matrix_sparsity(...); fuse_qkv_projections(model)
+    Forwards whose output does not require grad (`no_grad` evaluation, the first forward of reentrant checkpointing)
+    are ignored; the forward that non-reentrant checkpointing recomputes costs one more X pass and adds nothing.
+    """
+
+    def __init__(self, block: int = 256, mlp: bool = False, attention: bool = True):
+        self.block, self.mlp, self.attention = block, mlp, attention
+        self.acc: Dict[Key, torch.Tensor] = {}
+        self.shapes: Dict[Key, Tuple[int, int]] = {}
+        self._handles = []
+        self._x_cache = None         # (weakref to the last input, its version, its X): q/k/v share their input
+
+    def attach(self, model) -> "FactoredBlockSumAccumulator":
+        """Forward hooks on q/k/v (and gate/up/down with mlp=True) of `model`; o_proj is never captured
+        (fine_tune.py:747).  Accumulators are created here, in module order.  Returns self."""
+        b = self.block
+        found = []
+        for name, mod in model.named_modules():
+            if not isinstance(mod, torch.nn.Linear):
+                continue
+            key = classify_parameter(name + ".weight", self.mlp, self.attention)
+            if key is None:
+                continue
+            R, Cc = mod.weight.shape
+            if R % b or Cc % b:
+                raise SMTLibraryError(f"{name}: weight {R}x{Cc} is not a multiple of the block size {b}")
+            found.append((key, mod, R, Cc))
+        for key, mod, R, Cc in found:
+            if key not in self.acc:
+                self.shapes[key] = (R, Cc)
+                self.acc[key] = torch.zeros((R // b, Cc // b), dtype=torch.float32, device=mod.weight.device)
+            self._handles.append(mod.register_forward_hook(lambda _m, args, out, key=key: self._forward(key, args[0], out)))
+        return self
+
+    def detach(self) -> None:
+        for h in self._handles:
+            h.remove()
+        self._handles = []
+        self._x_cache = None
+
+    def _forward(self, key: Key, x: torch.Tensor, out: torch.Tensor) -> None:
+        if not (torch.is_grad_enabled() and out.requires_grad):
+            return
+        if not (x.is_cuda and out.is_cuda):
+            raise SMTLibraryError("FactoredBlockSumAccumulator works on CUDA activations (no CPU path)")
+        c = self._x_cache
+        if c is not None and c[0]() is x and c[1] == x._version:
+            X = c[2]
+        else:
+            X = ops.token_block_sums(_rows(x), self.block)
+            self._x_cache = (weakref.ref(x), x._version, X)
+        acc = self.acc[key]
+        out.register_hook(lambda dy: ops.block_outer_accumulate(acc, ops.token_block_sums(_rows(dy), self.block), X))
+
+    def scores(self, calculate_strategy: str = "mean_abs"):
+        """(keys, [R/b, C/b] score tensors) ready for smt_helper.select_submatrix_from_scores."""
+        if calculate_strategy != "mean_abs":
+            raise SMTLibraryError("factored block sums are linear in the gradient and only reproduce 'mean_abs'")
+        keys = list(self.acc.keys())
+        return keys, [ops.block_sum_finalize(self.acc[k], self.block) for k in keys]
+
+    flat_state = WarmupGradAccumulator.flat_state
+    load_flat_state = WarmupGradAccumulator.load_flat_state
+
+
+def _rows(t: torch.Tensor) -> torch.Tensor:
+    """[..., F] -> [T, F] with unit column stride and a 16-byte aligned base and row pitch."""
+    t2 = t.reshape(-1, t.shape[-1])
+    if t2.stride(1) != 1 or t2.data_ptr() % 16 or (t2.stride(0) * t2.element_size()) % 16:
+        t2 = t2.clone(memory_format=torch.contiguous_format)
+    return t2
 
 
 class WarmupActivationAccumulator:
