@@ -210,19 +210,17 @@ SMT_API int smt_block_grad_gemm_grouped(const void* maps, const smt_gemm_item* i
                                         int64_t T, int block, int in_dtype, void* out_base, int out_dtype,
                                         int accumulate, int64_t ld_out, float* sq_partials, void* workspace,
                                         size_t workspace_bytes, void* stream);
-/* Strip-sharing form of the single-problem call: a tile is a RUN - one block row and up to
- * smt_block_grad_gemm_run_width(block) (4 / 2 / 2 for b = 64 / 128 / 256) of its selected block columns - so the dy strip
- * is fetched once per run and the x strips form one wide UMMA operand (b = 256: one 128-row half of the block row per
- * run, `half`).  Same arithmetic as smt_block_grad_gemm (fp32 accumulation over all T, one rounding; deterministic).
+/* Strip-sharing form of the single-problem call for b = 64 / 128: a tile is a RUN - one block row and up to
+ * smt_block_grad_gemm_run_width(block) (4 / 2 for b = 64 / 128, 0 = no run tiles, as for b = 256) of its selected block
+ * columns - so the dy strip is fetched once per run and the x strips form one wide UMMA operand.  Same arithmetic as
+ * smt_block_grad_gemm (fp32 accumulation over all T, one rounding; deterministic).
  * The caller forms the runs (ops.block_grad_gemm does, from the Python index list) and passes them as a DEVICE array;
  * `out_blk[j]` is the position of block (row, cols[j]) in the index list, i.e. its result goes to G + out_blk[j]*b*b. */
 typedef struct smt_gemm_run {
   int32_t row;         /* block row (dy strip)                                        */
-  int32_t half;        /* b = 256: 0 / 1 = rows [0,128) / [128,256) of the block; else 0 */
   int32_t ncols;       /* 1 .. run width                                               */
   int32_t cols[4];     /* block columns (x strips)                                     */
   int32_t out_blk[4];  /* index of (row, cols[j]) in the caller's block list           */
-  int32_t pad_;
 } smt_gemm_run;
 SMT_API int smt_block_grad_gemm_run_width(int block);
 SMT_API size_t smt_block_grad_gemm_runs_workspace_bytes(int n_runs, int block, int64_t T);
@@ -231,9 +229,6 @@ SMT_API int smt_block_grad_gemm_runs(const void* x, int64_t ldx, int in_features
                                      int64_t T, int in_dtype, const smt_gemm_run* runs, int n_runs, int block,
                                      void* G, int out_dtype, int accumulate,
                                      void* workspace, size_t workspace_bytes, void* stream);
-/* debug: register a device buffer of 8*max_ctas uint64; each CTA of smt_block_grad_gemm stamps %globaltimer at its
- * phase boundaries (tools/trace_gemm.py). NULL switches tracing off. Not for production use. */
-SMT_API int smt_debug_set_gemm_trace(void* dev_buf, int max_ctas);
 /* introspection for tests/bench: split-K factor and CTA count the launch above would use. */
 SMT_API int smt_block_grad_gemm_plan(int n_blocks, int block, int64_t T, int in_dtype,
                              int* splits_host, int* ctas_host);

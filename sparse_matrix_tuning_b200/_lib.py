@@ -12,7 +12,7 @@ import threading
 import torch
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-LIB_PATH = os.environ.get("SMT_B200_LIB") or os.path.join(_HERE, "_C", "libsmt_b200.so")   # (override: kernel experiments)
+LIB_PATH = os.path.join(_HERE, "_C", "libsmt_b200.so")
 
 F32, BF16, F16 = 0, 1, 2
 MEAN_ABS, ABS_MEAN, L1, L2 = 0, 1, 2, 3
@@ -37,8 +37,7 @@ ITEM_OVERWRITE = 1   # SMT_ITEM_OVERWRITE
 
 class GemmRun(C.Structure):
     """Mirror of `smt_gemm_run`."""
-    _fields_ = [("row", C.c_int32), ("half", C.c_int32), ("ncols", C.c_int32), ("cols", C.c_int32 * 4),
-                ("out_blk", C.c_int32 * 4), ("pad_", C.c_int32)]
+    _fields_ = [("row", C.c_int32), ("ncols", C.c_int32), ("cols", C.c_int32 * 4), ("out_blk", C.c_int32 * 4)]
 
 
 class SMTLibraryError(RuntimeError):
@@ -74,7 +73,6 @@ _SIGNATURES = {
     "smt_block_grad_gemm_runs_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int64]),
     "smt_block_grad_gemm_runs": (C.c_int, [_P, C.c_int64, C.c_int, _P, C.c_int64, C.c_int, C.c_int64, C.c_int,
                                            _P, C.c_int, C.c_int, _P, C.c_int, C.c_int, _P, C.c_size_t, _P]),
-    "smt_debug_set_gemm_trace": (C.c_int, [_P, C.c_int]),
     "smt_encode_operand_map": (C.c_int, [_P, _P, C.c_int64, C.c_int64, C.c_int64, C.c_int, C.c_int]),
     "smt_block_grad_gemm_grouped_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int64]),
     "smt_block_grad_gemm_grouped_uses_2sm": (C.c_int, [C.c_int, C.c_int, C.c_int64]),

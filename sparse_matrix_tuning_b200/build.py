@@ -53,7 +53,7 @@ def build(force: bool = False, verbose: bool = False) -> str:
 
     def compile_one(src: str) -> str:
         obj = os.path.join(obj_dir, src.replace(".cu", ".o"))
-        cmd = [nvcc, *NVCC_FLAGS, *os.environ.get("SMT_NVCC_EXTRA", "").split(), "-c", os.path.join(CSRC, src), "-o", obj]
+        cmd = [nvcc, *NVCC_FLAGS, "-c", os.path.join(CSRC, src), "-o", obj]
         if verbose:
             cmd.insert(1, "-Xptxas=-v")
         r = subprocess.run(cmd, capture_output=True, text=True)

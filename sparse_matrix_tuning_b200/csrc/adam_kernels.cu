@@ -36,13 +36,8 @@ struct AdamArgs {
   float lr, beta1, beta2, eps, wd, bc1, bc2, grad_scale, max_norm;
 };
 
-#ifndef SMT_ADAM_MINB
-#define SMT_ADAM_MINB 5   // resident CTAs per SM the register allocation is tuned for: measured best of {3,4,5,6,8} (profiles/r01_kernels.md)
-#endif
-#ifndef SMT_ADAM_VEC
-#define SMT_ADAM_VEC 4    // elements per thread per iteration (4 or 8); 4 x 5 CTAs/SM beat 8 x 4 by 12 %
-#endif
-constexpr int kAdamVec = SMT_ADAM_VEC;
+constexpr int kAdamMinBlocks = 5;   // resident CTAs per SM the register allocation is tuned for: measured best of {3,4,5,6,8} (profiles/r01_kernels.md)
+constexpr int kAdamVec = 4;         // elements per thread per iteration (4 or 8); 4 x 5 CTAs/SM beat 8 x 4 by 12 %
 
 template <int GDT, int N>
 __device__ __forceinline__ void load_grad(const void* p, int64_t e, float (&g)[N]) {
@@ -100,7 +95,7 @@ __device__ __forceinline__ void store_vals(void* base, int64_t e, const float (&
 }
 
 template <int GDT, int CDT, int WDT>
-__global__ void __launch_bounds__(kAdamThreads, SMT_ADAM_MINB) compact_adam_kernel(
+__global__ void __launch_bounds__(kAdamThreads, kAdamMinBlocks) compact_adam_kernel(
     float* __restrict__ master, float* __restrict__ exp_avg, float* __restrict__ exp_avg_sq,
     const void* __restrict__ grad, int64_t n_vec, AdamArgs a, const float* __restrict__ sqnorm, int n_sq,
     void* __restrict__ compact_out, const smt_block_ref* __restrict__ table, int block_shift) {
@@ -303,7 +298,7 @@ extern "C" SMT_API int smt_compact_adam(float* master, float* exp_avg, float* ex
   AdamArgs a{lr, beta1, beta2, eps, weight_decay, bias_correction1, bias_correction2, grad_scale, max_norm};
   const int64_t n_vec8 = n_elems / kAdamVec;       // vectors of kAdamVec elements (n_elems is a multiple of 8)
   int64_t want = (n_vec8 + kAdamThreads - 1) / kAdamThreads;
-  const int64_t cap = (int64_t)sm_count() * SMT_ADAM_MINB * 2;
+  const int64_t cap = (int64_t)sm_count() * kAdamMinBlocks * 2;
   const int grid = (int)(want < cap ? want : cap);
   cudaStream_t st = (cudaStream_t)stream;
   if (grad_dtype == SMT_F32) return launch_adam_c<SMT_F32>(compact_dtype, w_dtype, grid, st, master, exp_avg, exp_avg_sq, grad, n_vec8, a, sqnorm, n_sqnorm, compact_out, table, shift);

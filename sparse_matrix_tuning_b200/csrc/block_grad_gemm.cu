@@ -41,31 +41,17 @@ namespace {
 // fixed cost (~100-150 clk per TMA box plus the barrier round trip) that a whole-block b = 256 tile hides behind
 // 1 024 clk of UMMA work; the small tiles do not, so they take 128-token stages (half as many boxes and barrier
 // round trips per token; +23-56 % on B200, profiles/r01_kernels.md section 1c).
-#ifndef SMT_GEMM_KTILE
-#define SMT_GEMM_KTILE 64                     // b = 256
-#endif
-#ifndef SMT_GEMM_KTILE_128
-#define SMT_GEMM_KTILE_128 128                // b = 128
-#endif
-#ifndef SMT_GEMM_KTILE_64
-#define SMT_GEMM_KTILE_64 256                 // b = 64
-#endif
-#ifndef SMT_GEMM_B64_ALIAS
-#define SMT_GEMM_B64_ALIAS 1                  // b = 64: no shared-memory slot for the unused upper half of the M=128 operand
-#endif
-#ifndef SMT_GEMM_MAX_STAGES
-#define SMT_GEMM_MAX_STAGES 8
-#endif
+constexpr int kKTile256 = 64;
+constexpr int kKTile128 = 128;
+constexpr int kKTile64 = 256;
+constexpr int kMaxStages = 8;
 constexpr int ktile_for(int block) {
-  return block == 256 ? SMT_GEMM_KTILE : block == 128 ? SMT_GEMM_KTILE_128 : SMT_GEMM_KTILE_64;
+  return block == 256 ? kKTile256 : block == 128 ? kKTile128 : kKTile64;
 }
 constexpr int kMaxKTile = 256;                // TMA box height limit
 static_assert(ktile_for(256) % 16 == 0 && ktile_for(128) % 16 == 0 && ktile_for(64) % 16 == 0, "K tile");
 static_assert(ktile_for(256) <= kMaxKTile && ktile_for(128) <= kMaxKTile && ktile_for(64) <= kMaxKTile, "K tile");
-#ifndef SMT_GEMM_EPI_WARPS
-#define SMT_GEMM_EPI_WARPS 8                  // multiple of 4 (one TMEM lane quarter per warp % 4)
-#endif
-constexpr int kEpiWarps = SMT_GEMM_EPI_WARPS;
+constexpr int kEpiWarps = 8;                  // multiple of 4 (one TMEM lane quarter per warp % 4)
 constexpr int kGemmThreads = 64 + 32 * kEpiWarps;   // warp 0 TMA, warp 1 MMA + TMEM alloc, warps 2-9 epilogue
 constexpr int kSmemBudget = 200 * 1024;       // pipeline stages (dynamic smem), leaves room for barriers
 constexpr int kMinTokensPerSplit = 256;
@@ -76,24 +62,18 @@ struct Cfg {
   static constexpr int MH = MH_;                              // M=128 accumulators per CTA
   static constexpr int KT = ktile_for(B);                     // tokens per pipeline stage
   static constexpr int CHUNK_BYTES = KT * 128;                // one {64 features x KT tokens} TMA box of 16-bit data
-  static constexpr int A_LOAD = B >= 128 ? 2 * MH : 1;        // dy chunks fetched per stage
-  // An M=128 MMA always spans two 64-row chunks.  For b = 64 only the first is loaded; with SMT_GEMM_B64_ALIAS the
-  // second half of the operand aliases the x chunk that follows it in the stage (initialised shared memory; it
+  // dy chunks fetched per stage.  An M=128 MMA always spans two 64-row chunks.  For b = 64 only the first is loaded;
+  // the second half of the operand aliases the x chunk that follows it in the stage (initialised shared memory; it
   // feeds accumulator rows 64..127, which are never read) instead of owning a slot.
-  static constexpr int A_SLOTS = (A_LOAD < 2 && !SMT_GEMM_B64_ALIAS) ? 2 : A_LOAD;
+  static constexpr int A_LOAD = B >= 128 ? 2 * MH : 1;
   static constexpr int B_LOAD = B / 64;                       // N = B
   static constexpr int TILES_PER_BLOCK = (B == 256 && MH == 1) ? 2 : 1;
   static constexpr int TILE_ROWS = B >= 128 ? 128 * MH : B;   // output rows one CTA produces
   static constexpr int TILE_ELEMS = TILE_ROWS * B;
-  static constexpr int STAGE_BYTES = (A_SLOTS + B_LOAD) * CHUNK_BYTES;
+  static constexpr int STAGE_BYTES = (A_LOAD + B_LOAD) * CHUNK_BYTES;
   static constexpr int STAGES_RAW = kSmemBudget / STAGE_BYTES;
-  static constexpr int STAGES = STAGES_RAW > SMT_GEMM_MAX_STAGES ? SMT_GEMM_MAX_STAGES : STAGES_RAW;
-#ifdef SMT_GEMM_EXPERIMENT_SKIP_CHUNKS   // perf-only experiment (wrong results): skip that many A chunks per stage
-  static constexpr int A_ISSUE = A_LOAD > SMT_GEMM_EXPERIMENT_SKIP_CHUNKS ? A_LOAD - SMT_GEMM_EXPERIMENT_SKIP_CHUNKS : 1;
-#else
-  static constexpr int A_ISSUE = A_LOAD;
-#endif
-  static constexpr int TX_BYTES = (A_ISSUE + B_LOAD) * CHUNK_BYTES;
+  static constexpr int STAGES = STAGES_RAW > kMaxStages ? kMaxStages : STAGES_RAW;
+  static constexpr int TX_BYTES = (A_LOAD + B_LOAD) * CHUNK_BYTES;
   static constexpr int TMEM_COLS = MH * B < 32 ? 32 : MH * B;  // 512 / 256 / 128 / 64 (powers of two)
   static constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + 1024;  // + alignment slack
   static_assert(STAGES * STAGE_BYTES >= kEpiWarps * 32 * kStageRow * 4, "epilogue staging must fit in the pipeline smem");
@@ -109,7 +89,6 @@ struct GemmParams {
   float* ws;                      // fp32 partial tiles when splits > 1
   float* sq;                      // grouped, no split-K: per-block sum-of-squares slots (items[i].sq_slot), or NULL
   int* counters;                  // fused reduction: 2 self-resetting ints per tile (NULL = separate reduce kernel)
-  unsigned long long* trace;      // debug (SMT_GEMM_TRACE=1): 8 globaltimer stamps per CTA, else NULL
   int64_t ld_out;                 // row pitch of an output tile in elements (== block for compact storage)
   int splits;
   int kt_total;                   // number of K tiles = ceil(T / ktile_for(block))
@@ -162,7 +141,6 @@ __global__ void __launch_bounds__(kGemmThreads, 1) block_grad_umma_kernel(
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int tile = blockIdx.x, split = blockIdx.y;
-  if (threadIdx.x == 0) SMT_TRACE(0);                       // CTA start
   const int blk = tile / C::TILES_PER_BLOCK, half = tile % C::TILES_PER_BLOCK;
   const int kt_begin = split * p.kt_per_split;
   const int kt_end = min(kt_begin + p.kt_per_split, p.kt_total);
@@ -172,7 +150,7 @@ __global__ void __launch_bounds__(kGemmThreads, 1) block_grad_umma_kernel(
   const uint32_t smem_base = (smem_u32(smem_raw) + 1023u) & ~1023u;
   uint8_t* smem_gen = smem_raw + (smem_base - smem_u32(smem_raw));
   auto a_addr = [&](int stage) { return smem_base + stage * C::STAGE_BYTES; };
-  auto b_addr = [&](int stage) { return smem_base + stage * C::STAGE_BYTES + C::A_SLOTS * C::CHUNK_BYTES; };
+  auto b_addr = [&](int stage) { return smem_base + stage * C::STAGE_BYTES + C::A_LOAD * C::CHUNK_BYTES; };
 
   int row, col;
   const CUtensorMap* map_x = &tmap_x;
@@ -209,7 +187,6 @@ __global__ void __launch_bounds__(kGemmThreads, 1) block_grad_umma_kernel(
   tc_fence_after();
   const uint32_t tmem_base = tmem_slot;
   if (threadIdx.x == 0) pdl_launch_dependents();   // the split-K reduce grid may get scheduled (it waits for us)
-  if (threadIdx.x == 0) SMT_TRACE(1);                       // barriers + TMEM ready
 
   if (warp == 0) {
     // ===== TMA producer =====
@@ -223,7 +200,7 @@ __global__ void __launch_bounds__(kGemmThreads, 1) block_grad_umma_kernel(
         mbar_expect_tx(fb, C::TX_BYTES);
         const int t0 = (kt_begin + it) * C::KT;
 #pragma unroll
-        for (int c = 0; c < C::A_ISSUE; ++c)
+        for (int c = 0; c < C::A_LOAD; ++c)
           tma_load_2d(a_addr(stage) + c * C::CHUNK_BYTES, map_dy, fb, a_col0 + c * 64, t0);
 #pragma unroll
         for (int c = 0; c < C::B_LOAD; ++c)
@@ -239,7 +216,6 @@ __global__ void __launch_bounds__(kGemmThreads, 1) block_grad_umma_kernel(
         const uint32_t phase = (uint32_t)(it / C::STAGES) & 1u;
         mbar_wait(smem_u32(&full_bar[stage]), phase);
         tc_fence_after();
-        if (it == 0) SMT_TRACE(2);                          // first operands landed
 #pragma unroll
         for (int k = 0; k < C::KT / 16; ++k) {
           // 16 tokens = two 8-row swizzle atoms = 2048 B further down every chunk
@@ -263,7 +239,6 @@ __global__ void __launch_bounds__(kGemmThreads, 1) block_grad_umma_kernel(
     constexpr int ROWS_PER_MH = B < 128 ? B : 128;
     mbar_wait(smem_u32(&tmem_full_bar), 0);
     tc_fence_after();
-    if (ew == 0) SMT_TRACE(3);                              // accumulators complete
     float sq0 = 0.f, sq1 = 0.f;
     if (q * 32 < ROWS_PER_MH) {
       // all MMAs have retired => the pipeline buffers are dead; reuse them as transpose staging
@@ -296,7 +271,6 @@ __global__ void __launch_bounds__(kGemmThreads, 1) block_grad_umma_kernel(
 
   tc_fence_before();
   __syncthreads();
-  if (threadIdx.x == 0) SMT_TRACE(4);                       // epilogue done
   if (warp == 1) {
     tc_fence_after();
     tmem_dealloc(tmem_base, C::TMEM_COLS);
@@ -330,7 +304,6 @@ __global__ void __launch_bounds__(kGemmThreads, 1) block_grad_umma_kernel(
           __trap();
         }
       }
-      SMT_TRACE(5);                                         // all sibling partials arrived
     }
     __syncthreads();
     const int chunk = ((C::TILE_ELEMS / 8 + p.splits - 1) / p.splits) * 8;
@@ -342,7 +315,6 @@ __global__ void __launch_bounds__(kGemmThreads, 1) block_grad_umma_kernel(
     else fused_reduce_slice<SMT_F16>(part0, p.splits, C::TILE_ELEMS, e_begin, e_end, p.out, out_off, acc_out, B, p.ld_out);
     __syncthreads();
     if (threadIdx.x == 0) {
-      SMT_TRACE(6);                                         // slice reduced
       if (atomicAdd(arrive + 1, 1) == p.splits - 1) {   // every sibling has passed its wait: safe to re-arm
         arrive[0] = 0;
         arrive[1] = 0;
@@ -648,7 +620,7 @@ int env_int(const char* name, int dflt) {
 //
 //     cost = 4 + waves * (5 + kt * c_kt + epilogue) + [splits > 1] * (8 + partial_bytes / 4 MB/us)
 //
-// fitted on B200 over tools/sweep_plan.py (profiles/r01_plan_sweep_raw.txt; typical error < 8 %).  c_kt is the
+// fitted on B200 over a plan sweep (profiles/r01_plan_sweep_raw.txt; typical error < 8 %; DESIGN.md section 3.1).  c_kt is the
 // measured time per 64-token K tile: 0.64 us for a whole 256-block per CTA (two M=128 UMMAs per K step, 84 % of the
 // UMMA issue rate), 0.41 us for a half block, 0.27 / 0.22 us for b = 128 / 64 with their taller stages.  Splitting K costs a
 // second (reduce) kernel plus writing and re-reading the fp32 partial tiles, so small launches prefer half-block
@@ -659,9 +631,7 @@ Plan make_plan(int n_blocks, int block, int64_t T) {
   const int ktile = ktile_for(block);
   const int kt_total = (int)((T + ktile - 1) / ktile);
   double best_cost = 1e30;
-  const int force_mh = env_int("SMT_GEMM_FORCE_MH", 0), force_splits = env_int("SMT_GEMM_FORCE_SPLITS", 0);
   for (int mh = 1; mh <= (block == 256 ? 2 : 1); ++mh) {
-    if (force_mh && mh != force_mh && block == 256) continue;
     const int tpb = (block == 256 && mh == 1) ? 2 : 1;
     const int tiles = n_blocks * tpb;
     const int tile_rows = block >= 128 ? 128 * mh : block;
@@ -672,7 +642,6 @@ Plan make_plan(int n_blocks, int block, int64_t T) {
     if (max_splits < 1) max_splits = 1;
     if (max_splits > 64) max_splits = 64;
     for (int s = 1; s <= max_splits; ++s) {
-      if (force_splits && s != (force_splits > max_splits ? max_splits : force_splits)) continue;
       const int kt = (kt_total + s - 1) / s;
       const int s_eff = (kt_total + kt - 1) / kt;
       const long ctas = (long)tiles * s_eff;
@@ -775,9 +744,6 @@ int launch_reduce(const float* ws, void* out, const smt_gemm_item* items, int bl
 
 inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
-unsigned long long* g_trace = nullptr;   // debug only, see smt_debug_set_gemm_trace
-int g_trace_ctas = 0;
-
 size_t plan_workspace_bytes(const Plan& pl) {
   return pl.splits > 1 ? kCounterBytes + (size_t)pl.tiles * pl.splits * pl.tile_elems * sizeof(float) : 0;
 }
@@ -879,7 +845,6 @@ extern "C" SMT_API int smt_block_grad_gemm(const void* x, int64_t ldx, int in_fe
   gp.out = G;
   gp.ws = need > 0 ? reinterpret_cast<float*>(reinterpret_cast<char*>(workspace) + kCounterBytes) : nullptr;
   gp.counters = use_fused_reduce(pl) ? reinterpret_cast<int*>(workspace) : nullptr;
-  gp.trace = (g_trace != nullptr && pl.tiles * pl.splits <= g_trace_ctas) ? g_trace : nullptr;
   gp.splits = pl.splits;
   gp.kt_total = pl.kt_total;
   gp.kt_per_split = pl.kt_per_split;
@@ -897,15 +862,6 @@ extern "C" SMT_API int smt_block_grad_gemm(const void* x, int64_t ldx, int in_fe
 }
 
 // ---- grouped entry point: blocks of several (x, dy) problems in one launch ----------------------------------
-
-// Debug facility: when a buffer of 8 * max_ctas uint64 is registered, every CTA of the single-problem GEMM stamps
-// %globaltimer at: 0 start, 1 setup done, 2 first operands landed, 3 accumulators complete, 4 epilogue done,
-// 5 split-K siblings arrived, 6 slice reduced.  Pass NULL to switch it off.
-extern "C" SMT_API int smt_debug_set_gemm_trace(void* dev_buf, int max_ctas) {
-  g_trace = reinterpret_cast<unsigned long long*>(dev_buf);
-  g_trace_ctas = dev_buf ? max_ctas : 0;
-  return SMT_OK;
-}
 
 extern "C" SMT_API int smt_encode_operand_map(void* map_host, const void* base, int64_t features, int64_t T,
                                               int64_t ld, int dtype, int block) {

@@ -7,20 +7,19 @@
 // against the 128 of a 256-block, which is why those sizes sat at 1/4 and 1/2 of the whole-block rate (round-1 profile,
 // section 1c/1d).  Blocks of one block ROW share their dy strip, so here a tile is a RUN: one block row and up to
 // kRunWidth(b) of its selected block columns.  The dy strip is loaded once per stage and the x strips of the run sit side by
-// side in shared memory, forming one UMMA B operand of N = ncols*b columns (b = 256: two N = 256 instructions that share
-// the A descriptor, one TMEM accumulator each):
+// side in shared memory, forming one UMMA B operand of N = ncols*b columns:
 //
 //     b = 64   up to 4 blocks per tile   1 + 4 TMA boxes of 96 tokens per stage, 3 stages   M = 128 (upper half unused), N <= 256
 //     b = 128  up to 2 blocks per tile   2 + 4 boxes of 64 tokens, 4 stages                 M = 128, N <= 256
-//     b = 256  up to 2 blocks per tile   2 + 8 boxes of 64 tokens, 2 stages                 M = 128 (one half of the block row), 2 x N = 256
-//              (two stages of 80 KiB cannot hide HBM latency: the host only takes this form for b = 256 when forced)
+//
+// There is no b = 256 form: a run of two 256-blocks needs 80 KiB per 64-token stage, and two such stages cannot hide HBM
+// latency (measured 37.8 us against 29.6 us for the plain kernel's whole-block tiles on 12 clustered blocks).
 //
 // Split-K over tokens for few tiles: one wave of CTAs, cooperative launch, partial tiles in an fp32 workspace, every
 // sibling CTA reduces its slice in the fixed order 0..splits-1 (deterministic, no atomics on data) - the same scheme as
 // the plain kernel.  The host (ops.block_grad_gemm) forms the runs from the Python index list, keeps the device copy
 // cached per list, and takes this path when enough blocks share a row.
 #include <cuda.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include "common.cuh"
@@ -41,26 +40,23 @@ constexpr size_t kRunCounterBytes = 16384;
 // on 716 blocks x T 8192, against 140.0 with 64-token and 119.6 with 80-token stages); b = 128: 64 tokens (6 boxes,
 // 48 KiB, 4 stages; 80 tokens x 3 stages measured the same).  128-token stages (two stages only) were no better than
 // the plain kernel.
-#ifndef SMT_RUNS_KT_64
-#define SMT_RUNS_KT_64 96       // b = 64
-#endif
-#ifndef SMT_RUNS_KT_128
-#define SMT_RUNS_KT_128 64      // b = 128
-#endif
+constexpr int kRunKTile64 = 96;
+constexpr int kRunKTile128 = 64;
 
 template <int B>
 struct RunCfg {
+  static_assert(B == 64 || B == 128, "run tiles exist for b = 64 / 128 only");
   static constexpr int NW = B == 64 ? 4 : 2;                 // blocks per run
-  static constexpr int KT = B == 256 ? 64 : (B == 128 ? SMT_RUNS_KT_128 : SMT_RUNS_KT_64);   // tokens per pipeline stage
+  static constexpr int KT = B == 128 ? kRunKTile128 : kRunKTile64;   // tokens per pipeline stage
   static constexpr int CHUNK = KT * 128;                     // one {64 features x KT tokens} TMA box
   static constexpr int A_LOAD = B == 64 ? 1 : 2;             // dy chunks (the M = 128 operand of b = 64 aliases the next chunk)
   static constexpr int B_PER_BLOCK = B / 64;
-  static constexpr int B_MAX = NW * B_PER_BLOCK;             // 4, 4, 8
-  static constexpr int STAGE_BYTES = (A_LOAD + B_MAX) * CHUNK;   // 60 / 48 / 80 KiB
-  static constexpr int STAGES = (200 * 1024) / STAGE_BYTES;      // 3 / 4 / 2
+  static constexpr int B_MAX = NW * B_PER_BLOCK;             // 4, 4
+  static constexpr int STAGE_BYTES = (A_LOAD + B_MAX) * CHUNK;   // 60 / 48 KiB
+  static constexpr int STAGES = (200 * 1024) / STAGE_BYTES;      // 3 / 4
   static constexpr int TILE_ROWS = B == 64 ? 64 : 128;       // output rows of one block that a tile produces
   static constexpr int SLOT = TILE_ROWS * B;                 // elements of one block's part of a tile
-  static constexpr int TMEM_COLS = B == 256 ? 512 : 256;
+  static constexpr int TMEM_COLS = 256;
   static constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + 1024;
   static_assert(STAGES * STAGE_BYTES >= kRunEpiWarps * 32 * kStageRow * 4, "epilogue staging must fit");
 };
@@ -120,7 +116,7 @@ __global__ void __launch_bounds__(kRunThreads, 1) block_grad_runs_kernel(const _
   if (warp == 0) {
     // ===== TMA producer: the dy strip once, then the x strip of every block of the run =====
     if (lane == 0) {
-      const int a_col0 = run.row * B + (B == 256 ? run.half * 128 : 0);
+      const int a_col0 = run.row * B;
       const uint32_t tx = (uint32_t)((C::A_LOAD + ncols * C::B_PER_BLOCK) * C::CHUNK);
       for (int it = 0; it < n_kt; ++it) {
         const int stage = it % C::STAGES;
@@ -140,11 +136,9 @@ __global__ void __launch_bounds__(kRunThreads, 1) block_grad_runs_kernel(const _
       }
     }
   } else if (warp == 1) {
-    // ===== MMA issuer =====
+    // ===== MMA issuer: ONE instruction over all the run's columns =====
     if (lane == 0) {
-      // b <= 128: ONE instruction over all the run's columns; b = 256: one N = 256 instruction per block
-      const int n_inst = B == 256 ? ncols : 1;
-      const uint32_t idesc = make_idesc(p.in_fmt, 128, B == 256 ? 256 : ncols * B);
+      const uint32_t idesc = make_idesc(p.in_fmt, 128, ncols * B);
       for (int it = 0; it < n_kt; ++it) {
         const int stage = it % C::STAGES;
         const uint32_t phase = (uint32_t)(it / C::STAGES) & 1u;
@@ -153,10 +147,8 @@ __global__ void __launch_bounds__(kRunThreads, 1) block_grad_runs_kernel(const _
 #pragma unroll
         for (int k = 0; k < C::KT / 16; ++k) {
           const uint64_t adesc = make_desc_mn_sw128(a_addr(stage) + k * 2048, C::CHUNK, 1024);
-          for (int i = 0; i < n_inst; ++i) {
-            const uint64_t bdesc = make_desc_mn_sw128(b_addr(stage) + i * 4 * C::CHUNK + k * 2048, C::CHUNK, 1024);
-            umma_f16(tmem_base + i * 256, adesc, bdesc, idesc, (it > 0 || k > 0) ? 1u : 0u);
-          }
+          const uint64_t bdesc = make_desc_mn_sw128(b_addr(stage) + k * 2048, C::CHUNK, 1024);
+          umma_f16(tmem_base, adesc, bdesc, idesc, (it > 0 || k > 0) ? 1u : 0u);
         }
         umma_commit(smem_u32(&empty_bar[stage]));
       }
@@ -170,7 +162,7 @@ __global__ void __launch_bounds__(kRunThreads, 1) block_grad_runs_kernel(const _
     if (q * 32 < C::TILE_ROWS) {
       float* stage = reinterpret_cast<float*>(smem_gen) + ew * 32 * kStageRow;
       const bool final_out = (p.splits == 1);
-      const int row_in_block = (B == 256 ? run.half * 128 : 0) + q * 32;
+      const int row_in_block = q * 32;
 #pragma unroll 1
       for (int j = 0; j < ncols; ++j) {
         float* part = p.ws + ((int64_t)(tile * C::NW + j) * p.splits + split) * C::SLOT;
@@ -217,7 +209,6 @@ __global__ void __launch_bounds__(kRunThreads, 1) block_grad_runs_kernel(const _
     const int total = ncols * C::SLOT;
     const int chunk = ((total / 8 + p.splits - 1) / p.splits) * 8;
     const int e_begin = split * chunk, e_end = min(e_begin + chunk, total);
-    const int row0 = B == 256 ? run.half * 128 : 0;
     for (int e = e_begin + (int)threadIdx.x * 8; e < e_end; e += (int)blockDim.x * 8) {
       const int j = e / C::SLOT, within = e - j * C::SLOT;
       const float* src0 = p.ws + (int64_t)(tile * C::NW + j) * p.splits * C::SLOT + within;
@@ -227,7 +218,7 @@ __global__ void __launch_bounds__(kRunThreads, 1) block_grad_runs_kernel(const _
         acc[0] += a.x; acc[1] += a.y; acc[2] += a.z; acc[3] += a.w;
         acc[4] += b4.x; acc[5] += b4.y; acc[6] += b4.z; acc[7] += b4.w;
       }
-      const int64_t o = (int64_t)run.out_blk[j] * B * B + (int64_t)row0 * B + within;
+      const int64_t o = (int64_t)run.out_blk[j] * B * B + within;
       const float4 v0 = make_float4(acc[0], acc[1], acc[2], acc[3]), v1 = make_float4(acc[4], acc[5], acc[6], acc[7]);
       if (p.out_dtype == SMT_F32) {
         if (p.accumulate) { store4<SMT_F32, true>(p.out, o, v0); store4<SMT_F32, true>(p.out, o + 4, v1); }
@@ -260,8 +251,9 @@ struct RunPlan {
   int splits, kt_total, kt_per_split;
 };
 
-int run_ktile(int block) { return block == 256 ? 64 : (block == 128 ? SMT_RUNS_KT_128 : SMT_RUNS_KT_64); }
+int run_ktile(int block) { return block == 128 ? kRunKTile128 : kRunKTile64; }
 int run_width(int block) { return block == 64 ? 4 : 2; }
+bool runs_block_ok(int block) { return block == 64 || block == 128; }
 int run_slot(int block) { return (block == 64 ? 64 : 128) * block; }
 
 // One wave: the token range is split so that n_runs * splits CTAs fill the SMs once (the reduction is fused into the
@@ -275,8 +267,6 @@ RunPlan make_run_plan(int n_runs, int block, int64_t T) {
   if (s > max_s) s = max_s;
   if (s < 1) s = 1;
   if (s > 64) s = 64;
-  const char* v = getenv("SMT_GEMM_RUNS_FORCE_SPLITS");
-  if (v && *v && n_runs * atoi(v) <= sm_count() && atoi(v) >= 1) s = atoi(v);
   pl.kt_per_split = (pl.kt_total + s - 1) / s;
   pl.splits = (pl.kt_total + pl.kt_per_split - 1) / pl.kt_per_split;
   return pl;
@@ -311,10 +301,10 @@ inline bool al16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) 
 
 using namespace smt;
 
-extern "C" SMT_API int smt_block_grad_gemm_run_width(int block) { return block_ok(block) ? run_width(block) : 0; }
+extern "C" SMT_API int smt_block_grad_gemm_run_width(int block) { return runs_block_ok(block) ? run_width(block) : 0; }
 
 extern "C" SMT_API size_t smt_block_grad_gemm_runs_workspace_bytes(int n_runs, int block, int64_t T) {
-  if (n_runs <= 0 || T <= 0 || !block_ok(block)) return 0;
+  if (n_runs <= 0 || T <= 0 || !runs_block_ok(block)) return 0;
   return run_workspace_bytes(n_runs, block, make_run_plan(n_runs, block, T));
 }
 
@@ -324,7 +314,8 @@ extern "C" SMT_API int smt_block_grad_gemm_runs(const void* x, int64_t ldx, int 
                                                 void* workspace, size_t workspace_bytes, void* stream) {
   SMT_CHECK_ARG(n_runs >= 0 && T > 0, "smt_block_grad_gemm_runs: needs T > 0 and n_runs >= 0");
   if (n_runs == 0) return SMT_OK;
-  SMT_CHECK_ARG(block_ok(block), "smt_block_grad_gemm_runs: block size %d not in {64,128,256}", block);
+  SMT_CHECK_ARG(runs_block_ok(block), "smt_block_grad_gemm_runs: block size %d not in {64,128} (b = 256 has no run tiles)",
+                block);
   SMT_CHECK_ARG(x && dy && G && runs, "smt_block_grad_gemm_runs: null pointer");
   SMT_CHECK_ARG((in_dtype == SMT_BF16 || in_dtype == SMT_F16) && out_dtype >= SMT_F32 && out_dtype <= SMT_F16,
                 "smt_block_grad_gemm_runs: 16-bit inputs only");
@@ -359,8 +350,7 @@ extern "C" SMT_API int smt_block_grad_gemm_runs(const void* x, int64_t ldx, int 
   rp.in_fmt = in_dtype == SMT_BF16 ? 1 : 0;
   cudaStream_t st = (cudaStream_t)stream;
   int rc;
-  if (block == 256) rc = launch_runs<256>(mx, mdy, rp, n_runs, st);
-  else if (block == 128) rc = launch_runs<128>(mx, mdy, rp, n_runs, st);
+  if (block == 128) rc = launch_runs<128>(mx, mdy, rp, n_runs, st);
   else rc = launch_runs<64>(mx, mdy, rp, n_runs, st);
   if (rc) return rc;
   set_launch_count(1);

@@ -13,12 +13,11 @@
 // Kernel shape (both directions): CTA pairs (cta_group::2), tile 256 x 256 per pair (M = 256 across the pair, each CTA
 // owns 128 rows and loads half of the B tile), K step 64 per pipeline stage (32 KiB per CTA and stage, 6 stages),
 // two 256-column TMEM accumulators so that the epilogue of tile i overlaps the main loop of tile i + 1, static
-// persistent schedule rasterised in groups of 8 M tiles for L2 reuse of the weights.  Warp 0 = TMA producer (both CTAs),
+// persistent schedule rasterised in groups of 16 M tiles for L2 reuse of the weights.  Warp 0 = TMA producer (both CTAs),
 // warp 1 = UMMA issuer (leader CTA), warps 2-5 = epilogue (TMEM -> registers -> bf16 -> per-warp shared-memory transpose
 // -> 128-byte row stores).  A is always K-major; B is K-major in forward (W[n, k], k contiguous) and MN-major in dgrad
 // (W[k, n], n contiguous): same TMA boxes / UMMA descriptors as the block-gradient kernel for the MN-major side.
 #include <cuda.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include "common.cuh"
@@ -31,10 +30,9 @@ namespace {
 constexpr int kDenseBK = 64;                           // K elements per stage (one 128-byte swizzle row)
 constexpr int kDenseTileM = 256, kDenseTileN = 256;    // per CTA pair
 constexpr int kDenseStageBytes = 2 * 128 * kDenseBK * 2;   // A: 128 rows x 64, B half: 128 n x 64  = 32 KiB
-#ifndef SMT_DENSE_STAGES
-#define SMT_DENSE_STAGES 6
-#endif
-constexpr int kDenseStages = SMT_DENSE_STAGES;
+constexpr int kDenseStages = 6;                        // 4 stages measured 2 % slower, 5 the same (profiles/r02_fused_qkv.md)
+// M tiles per raster group: 16 measured fastest of 2 / 4 / 8 / 16 / 32 (profiles/r02_fused_qkv.md)
+constexpr int kDenseGroupM = 16;
 constexpr int kDenseEpiWarps = 4;
 constexpr int kDenseThreads = 64 + 32 * kDenseEpiWarps;
 constexpr int kDenseStagingPitch = 144;                // bytes per staged row: 128 B of bf16 + 16 B pad (conflict-free v4)
@@ -295,13 +293,6 @@ int encode_dense_map(CUtensorMap* map, const void* base, int64_t cols, int64_t r
 
 inline bool al16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
-// M tiles per raster group (SMT_DENSE_GROUP_M overrides the default for experiments)
-int dense_group_m() {
-  const char* v = getenv("SMT_DENSE_GROUP_M");
-  const int g = (v && *v) ? atoi(v) : 16;
-  return g > 0 ? g : 16;
-}
-
 template <bool DGRAD>
 int launch_dense(const DenseMaps& maps, const DenseParams& p, cudaStream_t st) {
   auto kern = fused_dense_umma_2sm_kernel<DGRAD>;
@@ -393,7 +384,7 @@ extern "C" SMT_API int smt_fused_linear_forward(const void* x, int64_t ldx, int6
   p.seg_tile0[n_seg] = tiles;
   p.n_tiles = tiles;
   p.m_tiles = (int)((T + kDenseTileM - 1) / kDenseTileM);
-  p.group_m = dense_group_m();
+  p.group_m = kDenseGroupM;
   if (int rc = launch_dense<false>(maps, p, (cudaStream_t)stream)) return rc;
   set_launch_count(1);
   return SMT_OK;
@@ -424,7 +415,7 @@ extern "C" SMT_API int smt_fused_linear_dgrad(const void* const* dy_host, const 
   p.ld_out[0] = lddx;
   p.n_tiles = (K + kDenseTileN - 1) / kDenseTileN;
   p.m_tiles = (int)((T + kDenseTileM - 1) / kDenseTileM);
-  p.group_m = dense_group_m();
+  p.group_m = kDenseGroupM;
   if (int rc = launch_dense<true>(maps, p, (cudaStream_t)stream)) return rc;
   set_launch_count(1);
   return SMT_OK;

@@ -19,12 +19,8 @@ constexpr int kThreads = 256;
 
 // ---- acc += grad ---------------------------------------------------------------------------
 
-#ifndef SMT_SCORE_UNROLL
-#define SMT_SCORE_UNROLL 2     // vec8 groups in flight per thread (measured best of {1, 2, 4}: profiles/r01_kernels.md)
-#endif
-#ifndef SMT_SCORE_CTAS
-#define SMT_SCORE_CTAS 4       // grid cap in CTAs per SM for the streaming kernels (2 x 4 measured best: 6 125 GB/s)
-#endif
+constexpr int kScoreUnroll = 2;     // vec8 groups in flight per thread (measured best of {1, 2, 4}: profiles/r01_kernels.md)
+constexpr int kScoreCtas = 4;       // grid cap in CTAs per SM for the streaming kernels (2 x 4 measured best: 6 125 GB/s)
 
 template <int DT>
 __device__ __forceinline__ void load_grad8(const void* __restrict__ grad, int64_t i, float (&g)[8]) {
@@ -42,7 +38,7 @@ template <int DT>
 __global__ void __launch_bounds__(kThreads) score_accumulate_vec_kernel(
     float* __restrict__ acc, const void* __restrict__ grad, int64_t n_vec8) {
   // one "vec8" = 8 consecutive elements: 32 B of fp32 accumulator, 16 B (16-bit) or 32 B (fp32) of grad
-  constexpr int U = SMT_SCORE_UNROLL;
+  constexpr int U = kScoreUnroll;
   const int64_t stride = (int64_t)gridDim.x * blockDim.x;
   int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   for (; i + (U - 1) * stride < n_vec8; i += U * stride) {
@@ -242,9 +238,7 @@ __global__ void __launch_bounds__(kThreads) channel_score_reduce_kernel(
 //   sum_{o in r, k in c} dW[o, k] = sum_t Dy[t, r] * X[t, c],  Dy / X = per-token segment sums of dy / x.
 // token_block_sums_kernel makes Dy and X (one read of the activation), block_outer_* contracts them.
 
-#ifndef SMT_TBS_UNROLL
-#define SMT_TBS_UNROLL 4       // segment groups in flight per thread
-#endif
+constexpr int kTbsUnroll = 4;       // segment groups in flight per thread
 
 // out[t, j] = sum_{k < B} src[t, j*B + k].  L lanes of a warp share one segment (L = min(vectors per segment, 32)),
 // each lane loads P = vectors / L 128-bit vectors of it; the lane sums run in a fixed order, then an xor butterfly over
@@ -258,7 +252,7 @@ __global__ void __launch_bounds__(kThreads) token_block_sums_kernel(
   constexpr int L = NV < 32 ? NV : 32;                  // lanes per segment
   constexpr int P = NV / L;                             // vectors per lane per segment
   constexpr int SPW = 32 / L;                           // segments per warp and group
-  constexpr int U = SMT_TBS_UNROLL;
+  constexpr int U = kTbsUnroll;
   const int lane = threadIdx.x & 31, sub = lane / L, l = lane % L;
   const int64_t n_seg = T * seg_per_row;
   const int64_t n_groups = (n_seg + SPW - 1) / SPW;
@@ -371,7 +365,7 @@ void launch_token_block_sums(const void* src, int64_t ld, int64_t T, int seg_per
 inline int streaming_grid(int64_t work_items) {
   // enough CTAs for ~8 resident per SM, capped by the work
   int64_t want = (work_items + kThreads - 1) / kThreads;
-  int64_t cap = (int64_t)sm_count() * SMT_SCORE_CTAS;
+  int64_t cap = (int64_t)sm_count() * kScoreCtas;
   return (int)(want < cap ? (want < 1 ? 1 : want) : cap);
 }
 
@@ -491,7 +485,7 @@ extern "C" SMT_API int smt_token_block_sums(const void* src, int dtype, int64_t 
   const int vec = dtype == SMT_F32 ? 4 : 8;
   const int lanes = block / vec < 32 ? block / vec : 32;
   const int64_t groups = (T * seg_per_row + 32 / lanes - 1) / (32 / lanes);   // one warp per group
-  const int64_t want = (groups + (kThreads / 32) * SMT_TBS_UNROLL - 1) / ((kThreads / 32) * SMT_TBS_UNROLL);
+  const int64_t want = (groups + (kThreads / 32) * kTbsUnroll - 1) / ((kThreads / 32) * kTbsUnroll);
   cudaStream_t st = (cudaStream_t)stream;
 #define SMT_LAUNCH_TBS(B)                                                                                            \
   do {                                                                                                               \

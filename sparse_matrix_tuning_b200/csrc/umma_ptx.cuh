@@ -106,17 +106,6 @@ __device__ __forceinline__ void tmem_ld_32x32(uint32_t taddr, uint32_t (&r)[32])
 }
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 
-__device__ __forceinline__ unsigned long long globaltimer_ns() {
-  unsigned long long t;
-  asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
-  return t;
-}
-#define SMT_TRACE(slot)                                                                                   \
-  do {                                                                                                    \
-    if (p.trace != nullptr && (threadIdx.x & 31) == 0)                                                    \
-      p.trace[((size_t)blockIdx.y * gridDim.x + blockIdx.x) * 8 + (slot)] = globaltimer_ns();             \
-  } while (0)
-
 // Shared-memory matrix descriptor, MN-major, SWIZZLE_128B (see header comment for the layout).
 __device__ __forceinline__ uint64_t make_desc_mn_sw128(uint32_t smem_addr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
   uint64_t d = 0;

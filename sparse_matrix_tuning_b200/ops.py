@@ -397,7 +397,7 @@ LAST_SINGLE: dict = {}    # which kernel the last single-problem block_grad_gemm
 
 def _runs_for(index_list, block: int, device):
     """Strip-sharing runs of an index list (cached per list object, validated by value): blocks grouped by block row,
-    columns ascending, cut into runs of at most `run width` blocks; b = 256 yields one run per 128-row half.
+    columns ascending, cut into runs of at most `run width` blocks (b = 64 / 128).
     Returns (device tensor of smt_gemm_run, number of runs, fraction of the blocks that sit in a run of >= 2)."""
     import numpy as np
     snap = _snapshot_index_list(index_list)
@@ -416,13 +416,12 @@ def _runs_for(index_list, block: int, device):
             part = cols[k:k + width]
             if len(part) >= 2:
                 shared += len(part)
-            for half in ((0, 1) if block == 256 else (0,)):
-                cs = [c for c, _ in part] + [0] * (4 - len(part))
-                bs = [i for _, i in part] + [0] * (4 - len(part))
-                rows.append((r, half, len(part), *cs, *bs, 0))
-    arr = np.array(rows, dtype=np.int32).reshape(-1, 12)
+            cs = [c for c, _ in part] + [0] * (4 - len(part))
+            bs = [i for _, i in part] + [0] * (4 - len(part))
+            rows.append((r, len(part), *cs, *bs))
+    arr = np.array(rows, dtype=np.int32).reshape(-1, 10)
     assert arr.shape[1] * 4 == C.sizeof(_lib.GemmRun)
-    dev = torch.from_numpy(arr).to(device) if len(rows) else torch.empty((0, 12), dtype=torch.int32, device=device)
+    dev = torch.from_numpy(arr).to(device) if len(rows) else torch.empty((0, 10), dtype=torch.int32, device=device)
     res = (dev, len(rows), shared / max(len(snap), 1))
     if len(_runs_cache) > 4096:
         _runs_cache.clear()
@@ -436,9 +435,9 @@ def block_grad_gemm(x2d: torch.Tensor, dy2d: torch.Tensor, block_rc: torch.Tenso
     """G[i*b+o, k] (+)= sum_t dy[t, r_i*b+o] * x[t, c_i*b+k]. smt.py:386-404.
 
     x2d: [T, in], dy2d: [T, out] (unit column stride, same dtype); block_rc: int32 [n, 2] on device.
-    `index_list` (optional): the host-side list `block_rc` was made from.  With it, 16-bit launches in which enough
-    blocks share a block row run the strip-sharing kernel (`smt_block_grad_gemm_runs`: the dy strip is fetched once per
-    run of up to 4 / 2 / 2 blocks for b = 64 / 128 / 256).  SMT_GEMM_RUNS=0 disables that, =2 forces it.
+    `index_list` (optional): the host-side list `block_rc` was made from.  With it, 16-bit launches of b = 64 / 128 in
+    which enough blocks share a block row run the strip-sharing kernel (`smt_block_grad_gemm_runs`: the dy strip is
+    fetched once per run of up to 4 / 2 blocks for b = 64 / 128).
     """
     require_cuda(x2d, dy2d, block_rc)
     _req(x2d.dim() == 2 and dy2d.dim() == 2 and x2d.shape[0] == dy2d.shape[0],
@@ -454,32 +453,48 @@ def block_grad_gemm(x2d: torch.Tensor, dy2d: torch.Tensor, block_rc: torch.Tenso
         accumulate = False
     _req(out.is_contiguous() and out.numel() == n * block * block,
          "out.is_contiguous() and out.numel() == n * block * block")
-    lib = load()
-    in_id = dtype_id(x2d.dtype)
-    import os
-    mode = os.environ.get("SMT_GEMM_RUNS", "1")
-    if index_list is not None and mode != "0" and n > 0 and T > 0 and x2d.dtype != torch.float32:
+    if index_list is not None and block != 256 and n > 0 and T > 0 and x2d.dtype != torch.float32:
         _req(len(index_list) == n, "len(index_list) == block_rc.shape[0]")
-        runs, n_runs, shared = _runs_for(index_list, block, x2d.device)
+        runs = _runs_for(index_list, block, x2d.device)
+        n_runs = runs[1]
         # Measured rule (profiles/r02_kernel_sweep.md): run tiles pay when the launch is big enough for the operand feed
-        # to matter (>= 148 blocks), the runs are wide (singles are better off on the plain kernel's taller stages;
-        # two 80 KiB stages of a b = 256 pair tile cannot hide HBM latency) and the run tiles (times their one-wave
-        # split factor) still fill the GPU.  Small launches are bound by fixed costs either way.
+        # to matter (>= 148 blocks), the runs are wide (singles are better off on the plain kernel's taller stages)
+        # and the run tiles (times their one-wave split factor) still fill the GPU.  Small launches are bound by fixed
+        # costs either way.
         width = n / max(n_runs, 1)
         sms = 148
         fill = n_runs if n_runs >= sms else n_runs * (sms // max(n_runs, 1))      # CTAs of the (one-wave) split plan
-        if mode == "2" or (block != 256 and n >= 148 and width >= (2.0 if block == 64 else 1.5) and fill >= 80):
-            ws_bytes = lib.smt_block_grad_gemm_runs_workspace_bytes(n_runs, block, T)
-            ws = _workspace(ws_bytes, x2d.device, tag="gemm_runs")
-            with _timed("block_grad_gemm", x2d.device, (n, block, T)):
-                check(lib.smt_block_grad_gemm_runs(ptr(x2d), x2d.stride(0), x2d.shape[1], ptr(dy2d), dy2d.stride(0),
-                                                   dy2d.shape[1], T, in_id, ptr(runs), n_runs, block, ptr(out),
-                                                   dtype_id(out.dtype), 1 if accumulate else 0, ptr(ws), ws_bytes,
-                                                   _st(x2d)), "smt_block_grad_gemm_runs")
-            _count(lib.smt_last_launch_count())
-            LAST_SINGLE.update(kernel="runs", runs=n_runs, shared_fraction=shared)
-            return out
+        if n >= 148 and width >= (2.0 if block == 64 else 1.5) and fill >= 80:
+            return _gemm_runs(x2d, dy2d, runs, block, out, accumulate)
+    return _gemm_blocks(x2d, dy2d, block_rc, block, out, accumulate)
+
+
+def _gemm_runs(x2d: torch.Tensor, dy2d: torch.Tensor, runs, block: int, out: torch.Tensor,
+               accumulate: bool) -> torch.Tensor:
+    """The strip-sharing kernel on checked operands (see block_grad_gemm); `runs` = _runs_for(index_list, ...).
+    Needs T > 0, 16-bit inputs and b = 64 / 128."""
+    lib = load()
+    dev_runs, n_runs, shared = runs
+    n, T = out.numel() // (block * block), x2d.shape[0]
+    ws_bytes = lib.smt_block_grad_gemm_runs_workspace_bytes(n_runs, block, T)
+    ws = _workspace(ws_bytes, x2d.device, tag="gemm_runs")
+    with _timed("block_grad_gemm", x2d.device, (n, block, T)):
+        check(lib.smt_block_grad_gemm_runs(ptr(x2d), x2d.stride(0), x2d.shape[1], ptr(dy2d), dy2d.stride(0),
+                                           dy2d.shape[1], T, dtype_id(x2d.dtype), ptr(dev_runs), n_runs, block,
+                                           ptr(out), dtype_id(out.dtype), 1 if accumulate else 0, ptr(ws), ws_bytes,
+                                           _st(x2d)), "smt_block_grad_gemm_runs")
+    _count(lib.smt_last_launch_count())
+    LAST_SINGLE.update(kernel="runs", runs=n_runs, shared_fraction=shared)
+    return out
+
+
+def _gemm_blocks(x2d: torch.Tensor, dy2d: torch.Tensor, block_rc: torch.Tensor, block: int, out: torch.Tensor,
+                 accumulate: bool) -> torch.Tensor:
+    """The one-tile-per-block kernel on checked operands (see block_grad_gemm)."""
+    lib = load()
     LAST_SINGLE.update(kernel="blocks", runs=0, shared_fraction=0.0)
+    n, T = block_rc.shape[0], x2d.shape[0]
+    in_id = dtype_id(x2d.dtype)
     ws_bytes = lib.smt_block_grad_gemm_workspace_bytes(n, block, T, in_id)
     ws = _workspace(ws_bytes, x2d.device)
     with _timed("block_grad_gemm", x2d.device, (n, block, T)):

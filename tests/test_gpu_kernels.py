@@ -645,34 +645,39 @@ def _run_patterns(block):
 
 @pytest.mark.parametrize("T", [1000, 4096])
 @pytest.mark.parametrize("block", [64, 128, 256])
-def test_block_grad_gemm_runs_vs_truth_and_block_tiles(ops, monkeypatch, block, T):
-    """Strip-sharing kernel (a tile = one block row x up to 4 / 2 / 2 of its blocks): against fp64 truth and against
-    the plain one-tile-per-block kernel, for whole block rows, an unsorted mixed list (runs + singles, output order =
-    list order) and a single block; ragged token counts; bf16 and fp32 outputs; accumulate."""
+def test_block_grad_gemm_run_launcher_vs_truth_and_block_tiles(ops, block, T):
+    """Strip-sharing kernel through its private launcher (a tile = one block row x up to 4 / 2 of its blocks,
+    b = 64 / 128): against fp64 truth and against the plain one-tile-per-block launcher, for whole block rows, an
+    unsorted mixed list (runs + singles, output order = list order) and a single block; ragged token counts; bf16 and
+    fp32 outputs; accumulate.  Then the automatic choice of the public op between the two kernels, for every block
+    size."""
     torch.manual_seed(block + T)
     x = torch.randn(T, 1024).bfloat16()
     dy = torch.randn(T, 1024).bfloat16()
     xd, dyd = x.cuda(), dy.cuda()
-    for name, idx in _run_patterns(block).items():
+    patterns = _run_patterns(block) if block != 256 else {}                        # b = 256 has no run tiles
+    for name, idx in patterns.items():
         rc = ops.make_block_rc(idx, "cuda")
+        runs = ops._runs_for(idx, block, xd.device)
         truth = O.block_grad_truth(x.reshape(1, T, -1), dy.reshape(1, T, -1), idx, block)
         scale = truth.abs().max().item()
-        monkeypatch.setenv("SMT_GEMM_RUNS", "2")                                 # force the run kernel
-        got32 = ops.block_grad_gemm(xd, dyd, rc, block, out_dtype=torch.float32, index_list=idx)
+
+        def out(dtype):
+            return torch.empty((len(idx) * block, block), dtype=dtype, device="cuda")
+
+        got32 = ops._gemm_runs(xd, dyd, runs, block, out(torch.float32), False)
         assert ops.LAST_SINGLE["kernel"] == "runs", name
         assert (got32.cpu().double() - truth).abs().max().item() <= 3e-5 * scale, name
-        got16 = ops.block_grad_gemm(xd, dyd, rc, block, out_dtype=torch.bfloat16, index_list=idx)
+        got16 = ops._gemm_runs(xd, dyd, runs, block, out(torch.bfloat16), False)
         assert (got16.cpu().double() - truth).abs().max().item() <= 2 ** -7 * scale, name
-        assert torch.equal(got32, ops.block_grad_gemm(xd, dyd, rc, block, out_dtype=torch.float32, index_list=idx))
+        assert torch.equal(got32, ops._gemm_runs(xd, dyd, runs, block, out(torch.float32), False))
         base = torch.randn_like(got32)
         acc = base.clone()
-        ops.block_grad_gemm(xd, dyd, rc, block, out=acc, accumulate=True, index_list=idx)
+        ops._gemm_runs(xd, dyd, runs, block, acc, True)
         assert (acc - base - got32).abs().max().item() <= 3e-5 * scale, name
-        monkeypatch.setenv("SMT_GEMM_RUNS", "0")
-        plain = ops.block_grad_gemm(xd, dyd, rc, block, out_dtype=torch.float32, index_list=idx)
+        plain = ops._gemm_blocks(xd, dyd, rc, block, out(torch.float32), False)
         assert ops.LAST_SINGLE["kernel"] == "blocks"
         assert (got32 - plain).abs().max().item() <= 3e-5 * scale, name           # different split points, same math
-    monkeypatch.delenv("SMT_GEMM_RUNS", raising=False)
     # automatic choice: a big launch of wide runs => run tiles (b = 64 / 128); scattered singles / small launches => blocks
     nb = 1024 // block
     everything = [(r, c) for r in range(nb) for c in range(nb)]
@@ -683,15 +688,15 @@ def test_block_grad_gemm_runs_vs_truth_and_block_tiles(ops, monkeypatch, block, 
     assert ops.LAST_SINGLE["kernel"] == "blocks"
 
 
-def test_block_grad_gemm_runs_many_tiles_no_split(ops, monkeypatch):
+def test_block_grad_gemm_runs_many_tiles_no_split(ops):
     """More run tiles than SMs: several waves, no split-K, direct epilogue (b = 64, every block of a 2048 x 2048 weight)."""
     torch.manual_seed(5)
     T, b = 512, 64
     x = torch.randn(T, 2048, device="cuda").bfloat16()
     dy = torch.randn(T, 2048, device="cuda").bfloat16()
     idx = [(r, c) for r in range(32) for c in range(32)]
-    monkeypatch.setenv("SMT_GEMM_RUNS", "2")
-    got = ops.block_grad_gemm(x, dy, ops.make_block_rc(idx, "cuda"), b, out_dtype=torch.float32, index_list=idx)
+    out = torch.empty((len(idx) * b, b), dtype=torch.float32, device="cuda")
+    got = ops._gemm_runs(x, dy, ops._runs_for(idx, b, x.device), b, out, False)
     assert ops.LAST_SINGLE["kernel"] == "runs" and ops.LAST_SINGLE["runs"] == 256
     ref = dy.float().t() @ x.float()
     want = torch.stack([ref[r * b:(r + 1) * b, c * b:(c + 1) * b] for r, c in idx]).reshape(-1, b)

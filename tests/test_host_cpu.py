@@ -49,6 +49,9 @@ def test_argument_validation_needs_no_gpu(built_library):
     assert lib.smt_score_accumulate(None, None, 1, 8, None) == -1
     assert lib.smt_block_grad_gemm(p, 512, 500, p, 512, 512, 64, 1, p, 1, 256, p, 1, 0, None, 0, None) == -1
     assert b"multiples of block" in lib.smt_last_error()
+    assert lib.smt_block_grad_gemm_run_width(256) == 0                                   # b = 256 has no run tiles
+    assert lib.smt_block_grad_gemm_runs(p, 512, 512, p, 512, 512, 64, 1, p, 1, 256, p, 1, 0, None, 0, None) == -1
+    assert b"block size 256" in lib.smt_last_error()
     assert lib.smt_compact_adam(p, p, p, p, 1, 12, 1e-3, .9, .95, 1e-8, 0., .1, .05, 1., None, 0, 0., None, 1, None, 0, 0, 1, None) == -1
     assert lib.smt_topk_blocks(p, p, None, 8, p, p, p, 1, p, p, 1 << 20, None) == -1      # rank without inverse
     assert lib.smt_topk_workspace_bytes(1000) >= 16000

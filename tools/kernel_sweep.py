@@ -64,11 +64,13 @@ def main():
                             idx = [(1, c) for c in range(n)]
                         rc = ops.make_block_rc(idx, "cuda")
                         out = torch.empty(n * b, b, device="cuda", dtype=torch.bfloat16)
-                        os.environ["SMT_GEMM_RUNS"] = "0"                       # round-1 kernel: one tile per block
-                        t_blocks = timeit(lambda: ops.block_grad_gemm(x, dy, rc, b, out=out, index_list=idx))
-                        os.environ["SMT_GEMM_RUNS"] = "2"
-                        t_runs = timeit(lambda: ops.block_grad_gemm(x, dy, rc, b, out=out, index_list=idx))
-                        os.environ["SMT_GEMM_RUNS"] = "1"                       # default: strip-sharing runs when they pay
+                        # round-1 kernel: one tile per block; run tiles forced (b = 64 / 128 only)
+                        t_blocks = timeit(lambda: ops._gemm_blocks(x, dy, rc, b, out, False))
+                        runs_us = "-"
+                        if b != 256:
+                            t_runs = timeit(lambda: ops._gemm_runs(x, dy, ops._runs_for(idx, b, x.device), b, out, False))
+                            runs_us = f"{t_runs * 1e6:.1f}"
+                        # default: strip-sharing runs when they pay
                         t = timeit(lambda: ops.block_grad_gemm(x, dy, rc, b, out=out, index_list=idx))
                         kern = ops.LAST_SINGLE.get("kernel", "?")
                         flops = 2.0 * b * b * T * n
@@ -77,7 +79,7 @@ def main():
                         t_tensor = flops / (PEAKS["bf16_tflops"] * 1e12)
                         t_hbm = min_bytes / (PEAKS["hbm_gbs"] * 1e9)
                         bound = "tensor" if t_tensor >= t_hbm else "hbm"
-                        print(f"| {label} | {b} | {sp * 100:g}% | {pattern} | {T} | {n} | {kern} | {t * 1e6:.1f} | {t_blocks * 1e6:.1f} | {t_runs * 1e6:.1f} | "
+                        print(f"| {label} | {b} | {sp * 100:g}% | {pattern} | {T} | {n} | {kern} | {t * 1e6:.1f} | {t_blocks * 1e6:.1f} | {runs_us} | "
                               f"{flops / t / 1e12:.1f} | {flops / t / 1e12 / PEAKS['bf16_tflops']:.3f} | {bound} | "
                               f"{max(t_tensor, t_hbm) / t:.3f} |", flush=True)
             del x, dy

@@ -65,12 +65,11 @@ for b in (64, 128, 256):
     dy = torch.randn(T, fin, device=dev).bfloat16()
     nb = fin // b
     idx = [(r, c) for r in range(min(nb, 3)) for c in range(nb)]
-    rc = ops.make_block_rc(idx, dev)
-    os.environ["SMT_GEMM_RUNS"] = "2"
-    got = ops.block_grad_gemm(x, dy, rc, b, out_dtype=torch.float32, index_list=idx)
-    os.environ["SMT_GEMM_RUNS"] = "1"
-    ref = dy.float()[:, :b].t() @ x.float()[:, :b]
-    assert (got[:b] - ref).abs().max() <= 3e-5 * ref.abs().max()
+    if b != 256:                                                    # run tiles exist for b = 64 / 128
+        got = ops._gemm_runs(x, dy, ops._runs_for(idx, b, x.device), b,
+                             torch.empty(len(idx) * b, b, device=dev), False)
+        ref = dy.float()[:, :b].t() @ x.float()[:, :b]
+        assert (got[:b] - ref).abs().max() <= 3e-5 * ref.abs().max()
     flat = torch.zeros(len(idx) * b * b, device=dev, dtype=torch.bfloat16)
     sqp = torch.zeros(2 * len(idx), device=dev)
     batch = ops.BlockGradBatch()
