@@ -232,8 +232,6 @@ int launch_adam_c(int c_dtype, int w_dtype, int grid, cudaStream_t st, float* ma
   return launch_adam_w<GDT, SMT_F16>(w_dtype, grid, st, master, m, v, grad, n_vec8, a, sqnorm, n_sq, compact_out, table, shift);
 }
 
-inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
-
 }  // namespace
 }  // namespace smt
 

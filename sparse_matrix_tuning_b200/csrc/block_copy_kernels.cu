@@ -42,7 +42,7 @@ int launch_copy(bool gather, const smt_block_ref* table, int n_blocks, int block
   SMT_CHECK_ARG(table && compact, "%s: null pointer", who);
   SMT_CHECK_ARG(block_ok(block), "%s: block size %d not in {64,128,256}", who, block);
   SMT_CHECK_ARG(elem_bytes == 2 || elem_bytes == 4, "%s: elem_bytes must be 2 or 4", who);
-  SMT_CHECK_ARG((reinterpret_cast<uintptr_t>(compact) & 15u) == 0, "%s: compact must be 16-byte aligned", who);
+  SMT_CHECK_ARG(aligned16(compact), "%s: compact must be 16-byte aligned", who);
   dim3 grid(n_blocks, kRowSplit);
   const int row_bytes = block * elem_bytes;
   if (gather)

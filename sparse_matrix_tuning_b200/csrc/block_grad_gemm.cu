@@ -55,7 +55,6 @@ constexpr int kEpiWarps = 8;                  // multiple of 4 (one TMEM lane qu
 constexpr int kGemmThreads = 64 + 32 * kEpiWarps;   // warp 0 TMA, warp 1 MMA + TMEM alloc, warps 2-9 epilogue
 constexpr int kSmemBudget = 200 * 1024;       // pipeline stages (dynamic smem), leaves room for barriers
 constexpr int kMinTokensPerSplit = 256;
-constexpr size_t kCounterBytes = 16384;       // head of the workspace: self-resetting split-K arrival counters
 
 template <int B, int MH_>
 struct Cfg {
@@ -97,35 +96,6 @@ struct GemmParams {
   int accumulate;
   int in_fmt;                     // 0 = f16, 1 = bf16
 };
-
-// Fused split-K reduction (cooperative launch: every CTA of the grid is resident, so waiting on siblings is safe).
-// Each of the `splits` CTAs of a tile has written its fp32 partial; after a per-tile arrival counter reaches
-// `splits`, CTA `split` sums ITS slice of the tile over all partials in the fixed order 0..splits-1 and writes the
-// final output.  The last CTA to finish resets the two counters, so the buffer is all-zero again at kernel end.
-template <int ODT>
-__device__ __forceinline__ void fused_reduce_slice(const float* __restrict__ part0, int splits, int tile_elems,
-                                                   int e_begin, int e_end, void* out, int64_t out_off, bool acc_out,
-                                                   int b, int64_t ldo) {
-  for (int e = e_begin + (int)threadIdx.x * 8; e < e_end; e += (int)blockDim.x * 8) {
-    float acc[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-    for (int sp = 0; sp < splits; ++sp) {
-      const float* src = part0 + (int64_t)sp * tile_elems + e;
-      const float4 a = ld_cg_f4(src), b4 = ld_cg_f4(src + 4);
-      acc[0] += a.x; acc[1] += a.y; acc[2] += a.z; acc[3] += a.w;
-      acc[4] += b4.x; acc[5] += b4.y; acc[6] += b4.z; acc[7] += b4.w;
-    }
-    // element e of the (row-major, pitch b) tile lives at row e / b, column e % b of the output (pitch ldo); an
-    // 8-element vector never crosses a row (b is a multiple of 8)
-    const int64_t o = out_off + (int64_t)(e / b) * ldo + (e % b);
-    if (acc_out) {
-      store4<ODT, true>(out, o, make_float4(acc[0], acc[1], acc[2], acc[3]));
-      store4<ODT, true>(out, o + 4, make_float4(acc[4], acc[5], acc[6], acc[7]));
-    } else {
-      store4<ODT, false>(out, o, make_float4(acc[0], acc[1], acc[2], acc[3]));
-      store4<ODT, false>(out, o + 4, make_float4(acc[4], acc[5], acc[6], acc[7]));
-    }
-  }
-}
 
 template <int B, int MH, bool GROUPED>
 __global__ void __launch_bounds__(kGemmThreads, 1) block_grad_umma_kernel(
@@ -290,36 +260,10 @@ __global__ void __launch_bounds__(kGemmThreads, 1) block_grad_umma_kernel(
   }
 
   if (p.counters != nullptr) {
-    // ===== fused split-K reduction =====
-    __threadfence();                     // this thread's partial-tile stores are visible device-wide ...
-    __syncthreads();                     // ... for every thread of the CTA, before the CTA announces itself
-    int* arrive = p.counters + 2 * tile;
-    if (threadIdx.x == 0) {
-      atomicAdd(arrive, 1);
-      const long long t0 = clock64();
-      while (ld_acquire_gpu(arrive) < p.splits) {
-        __nanosleep(64);
-        if (clock64() - t0 > 4000000000ll) {
-          printf("smt_block_grad_gemm: split-K arrival wait timed out (tile %d split %d)\n", tile, split);
-          __trap();
-        }
-      }
-    }
-    __syncthreads();
-    const int chunk = ((C::TILE_ELEMS / 8 + p.splits - 1) / p.splits) * 8;
-    const int e_begin = split * chunk;
-    const int e_end = min(e_begin + chunk, C::TILE_ELEMS);
-    const float* part0 = p.ws + (int64_t)tile * p.splits * C::TILE_ELEMS;
-    if (p.out_dtype == SMT_F32) fused_reduce_slice<SMT_F32>(part0, p.splits, C::TILE_ELEMS, e_begin, e_end, p.out, out_off, acc_out, B, p.ld_out);
-    else if (p.out_dtype == SMT_BF16) fused_reduce_slice<SMT_BF16>(part0, p.splits, C::TILE_ELEMS, e_begin, e_end, p.out, out_off, acc_out, B, p.ld_out);
-    else fused_reduce_slice<SMT_F16>(part0, p.splits, C::TILE_ELEMS, e_begin, e_end, p.out, out_off, acc_out, B, p.ld_out);
-    __syncthreads();
-    if (threadIdx.x == 0) {
-      if (atomicAdd(arrive + 1, 1) == p.splits - 1) {   // every sibling has passed its wait: safe to re-arm
-        arrive[0] = 0;
-        arrive[1] = 0;
-      }
-    }
+    // element e of the (row-major, pitch B) tile lives at row e / B, column e % B of the output (pitch ld_out)
+    fused_splitk_reduce(p.counters + 2 * tile, split, p.splits, p.ws + (int64_t)tile * p.splits * C::TILE_ELEMS,
+                        C::TILE_ELEMS, C::TILE_ELEMS, p.out, p.out_dtype, acc_out,
+                        [&](int e) { return out_off + (int64_t)(e / B) * p.ld_out + e % B; }, "smt_block_grad_gemm");
   }
 }
 
@@ -499,14 +443,8 @@ __global__ void __launch_bounds__(256) splitk_reduce_kernel(const float* __restr
     const int64_t e = vec * 8;
     const int64_t tile = e / tile_elems;
     const int within = (int)(e - tile * tile_elems);
-    const float* src = ws + tile * splits * tile_elems + within;
-    float acc[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-    for (int s = 0; s < splits; ++s) {
-      const float4 a = ld_stream_f4(src + (int64_t)s * tile_elems);
-      const float4 b = ld_stream_f4(src + (int64_t)s * tile_elems + 4);
-      acc[0] += a.x; acc[1] += a.y; acc[2] += a.z; acc[3] += a.w;
-      acc[4] += b.x; acc[5] += b.y; acc[6] += b.z; acc[7] += b.w;
-    }
+    float acc[8];
+    sum_partials8<ld_stream_f4>(ws + tile * splits * tile_elems + within, splits, tile_elems, acc);
     int64_t o = e;
     int accumulate = accumulate_all;
     if (items != nullptr) {
@@ -668,20 +606,8 @@ int encode_operand_map(CUtensorMap* map, const void* base, int64_t features, int
 
 template <int B, int MH, bool GROUPED>
 int launch_umma_cfg(const CUtensorMap& mx, const CUtensorMap& mdy, const GemmParams& gp, const Plan& pl, cudaStream_t st) {
-  using C = Cfg<B, MH>;
-  auto kern = block_grad_umma_kernel<B, MH, GROUPED>;
-  SMT_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES));
-  dim3 grid(pl.tiles, pl.splits);
-  if (gp.counters != nullptr) {
-    // fused reduction: CTAs wait on their siblings, which is only legal when all of them are co-resident
-    void* args[3] = {const_cast<CUtensorMap*>(&mx), const_cast<CUtensorMap*>(&mdy), const_cast<GemmParams*>(&gp)};
-    SMT_CHECK_CUDA(cudaLaunchCooperativeKernel(reinterpret_cast<void*>(kern), grid, dim3(kGemmThreads), args,
-                                               (size_t)C::SMEM_BYTES, st));
-    return SMT_OK;
-  }
-  kern<<<grid, kGemmThreads, C::SMEM_BYTES, st>>>(mx, mdy, gp);
-  SMT_CHECK_LAUNCH();
-  return SMT_OK;
+  return launch_tiles(block_grad_umma_kernel<B, MH, GROUPED>, dim3(pl.tiles, pl.splits), kGemmThreads,
+                      Cfg<B, MH>::SMEM_BYTES, gp.counters != nullptr, st, mx, mdy, gp);
 }
 
 template <bool GROUPED>
@@ -742,10 +668,8 @@ int launch_reduce(const float* ws, void* out, const smt_gemm_item* items, int bl
   return SMT_OK;
 }
 
-inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
-
 size_t plan_workspace_bytes(const Plan& pl) {
-  return pl.splits > 1 ? kCounterBytes + (size_t)pl.tiles * pl.splits * pl.tile_elems * sizeof(float) : 0;
+  return pl.splits > 1 ? kSplitCounterBytes + (size_t)pl.tiles * pl.splits * pl.tile_elems * sizeof(float) : 0;
 }
 
 // The fused (in-kernel) reduction needs every CTA resident at once: one CTA per SM (shared memory), one wave.
@@ -757,7 +681,7 @@ bool use_fused_reduce(const Plan& pl) {
     coop = (cudaGetDevice(&dev) == cudaSuccess &&
             cudaDeviceGetAttribute(&v, cudaDevAttrCooperativeLaunch, dev) == cudaSuccess && v) ? 1 : 0;
   }
-  return coop == 1 && (long)pl.tiles * pl.splits <= sm_count() && (size_t)pl.tiles * 2 * sizeof(int) <= kCounterBytes;
+  return coop == 1 && (long)pl.tiles * pl.splits <= sm_count() && (size_t)pl.tiles * 2 * sizeof(int) <= kSplitCounterBytes;
 }
 
 }  // namespace
@@ -829,12 +753,11 @@ extern "C" SMT_API int smt_block_grad_gemm(const void* x, int64_t ldx, int in_fe
 
   SMT_CHECK_ARG(T < (1ll << 31) - kMaxKTile, "smt_block_grad_gemm: T too large");
   const Plan pl = make_plan(n_blocks, block, T);
-  const size_t need = plan_workspace_bytes(pl);
-  if (need > 0 && (workspace == nullptr || workspace_bytes < need)) {
-    set_error("smt_block_grad_gemm: workspace too small (%zu < %zu)", workspace_bytes, need);
-    return SMT_ERR_WORKSPACE;
-  }
-  if (need > 0) SMT_CHECK_ARG(aligned16(workspace), "smt_block_grad_gemm: workspace must be 16-byte aligned");
+  int* counters;
+  float* partials;
+  if (int rc = carve_split_workspace("smt_block_grad_gemm", workspace, workspace_bytes, plan_workspace_bytes(pl),
+                                     &counters, &partials))
+    return rc;
 
   CUtensorMap mx, mdy;
   if (int rc = encode_operand_map(&mx, x, in_features, T, ldx, in_dtype, ktile_for(block))) return rc;
@@ -843,8 +766,8 @@ extern "C" SMT_API int smt_block_grad_gemm(const void* x, int64_t ldx, int in_fe
   GemmParams gp{};
   gp.block_rc = block_rc;
   gp.out = G;
-  gp.ws = need > 0 ? reinterpret_cast<float*>(reinterpret_cast<char*>(workspace) + kCounterBytes) : nullptr;
-  gp.counters = use_fused_reduce(pl) ? reinterpret_cast<int*>(workspace) : nullptr;
+  gp.ws = partials;
+  gp.counters = use_fused_reduce(pl) ? counters : nullptr;
   gp.splits = pl.splits;
   gp.kt_total = pl.kt_total;
   gp.kt_per_split = pl.kt_per_split;
@@ -916,11 +839,12 @@ extern "C" SMT_API int smt_block_grad_gemm_grouped(const void* maps, const smt_g
   SMT_CHECK_ARG(T < (1ll << 31) - kMaxKTile, "smt_block_grad_gemm_grouped: T too large");
   SMT_CHECK_ARG(ld_out == 0 || (ld_out >= block && ld_out % 8 == 0 && ld_out < (1ll << 31)),
                 "smt_block_grad_gemm_grouped: ld_out must be 0 (compact tiles) or a multiple of 8 that is >= block");
-  const size_t need_total = smt_block_grad_gemm_grouped_workspace_bytes(n_items, block, T);
-  if (need_total > 0 && (workspace == nullptr || workspace_bytes < need_total)) {
-    set_error("smt_block_grad_gemm_grouped: workspace too small (%zu < %zu)", workspace_bytes, need_total);
-    return SMT_ERR_WORKSPACE;
-  }
+  const Plan pl = make_plan(n_items, block, T);
+  int* counters;
+  float* partials;
+  if (int rc = carve_split_workspace("smt_block_grad_gemm_grouped", workspace, workspace_bytes,
+                                     plan_workspace_bytes(pl), &counters, &partials))
+    return rc;
   cudaStream_t st = (cudaStream_t)stream;
   int launches = 0;
   GemmParams gp{};
@@ -941,11 +865,9 @@ extern "C" SMT_API int smt_block_grad_gemm_grouped(const void* maps, const smt_g
     set_launch_count(1);
     return SMT_OK;
   }
-  const Plan pl = make_plan(n_items, block, T);
-  const size_t need = plan_workspace_bytes(pl);
   gp.items = items;
-  gp.ws = need > 0 ? reinterpret_cast<float*>(reinterpret_cast<char*>(workspace) + kCounterBytes) : nullptr;
-  gp.counters = use_fused_reduce(pl) ? reinterpret_cast<int*>(workspace) : nullptr;
+  gp.ws = partials;
+  gp.counters = use_fused_reduce(pl) ? counters : nullptr;
   gp.splits = pl.splits;
   gp.kt_total = pl.kt_total;
   gp.kt_per_split = pl.kt_per_split;

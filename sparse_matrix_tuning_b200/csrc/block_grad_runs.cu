@@ -15,10 +15,11 @@
 // There is no b = 256 form: a run of two 256-blocks needs 80 KiB per 64-token stage, and two such stages cannot hide HBM
 // latency (measured 37.8 us against 29.6 us for the plain kernel's whole-block tiles on 12 clustered blocks).
 //
-// Split-K over tokens for few tiles: one wave of CTAs, cooperative launch, partial tiles in an fp32 workspace, every
-// sibling CTA reduces its slice in the fixed order 0..splits-1 (deterministic, no atomics on data) - the same scheme as
-// the plain kernel.  The host (ops.block_grad_gemm) forms the runs from the Python index list, keeps the device copy
-// cached per list, and takes this path when enough blocks share a row.
+// Split-K over tokens for few tiles: one wave of CTAs, cooperative launch, partial tiles in an fp32 workspace, reduced in
+// the kernel by the split-K reduction that the plain kernel also calls (fused_splitk_reduce in gemm_epilogue.cuh: every
+// sibling CTA sums its slice in the fixed order 0..splits-1; deterministic, no atomics on data).  The host
+// (ops.block_grad_gemm) forms the runs from the Python index list, keeps the device copy cached per list, and takes this
+// path when enough blocks share a row.
 #include <cuda.h>
 #include <string.h>
 
@@ -32,7 +33,6 @@ namespace {
 
 constexpr int kRunThreads = 64 + 32 * 8;        // warp 0 TMA, warp 1 MMA + TMEM, warps 2-9 epilogue
 constexpr int kRunEpiWarps = 8;
-constexpr size_t kRunCounterBytes = 16384;
 
 // Tokens per pipeline stage for b = 64 / 128 (measured: profiles/r02_runs_variants_raw.txt).  A launch whose strips
 // come from HBM needs >= 3 stages to hide the load latency, and every TMA box costs the producer ~70 clk whatever its
@@ -64,7 +64,7 @@ struct RunCfg {
 struct RunParams {
   const smt_gemm_run* runs;
   void* out;
-  float* ws;             // fp32 partial slots when splits > 1: [(run * NW + j) * splits + split][SLOT]
+  float* ws;             // fp32 partial slots when splits > 1: [(run * splits + split) * NW + j][SLOT]
   int* counters;         // 2 self-resetting ints per run (splits > 1)
   int splits;
   int kt_total, kt_per_split;
@@ -165,7 +165,7 @@ __global__ void __launch_bounds__(kRunThreads, 1) block_grad_runs_kernel(const _
       const int row_in_block = q * 32;
 #pragma unroll 1
       for (int j = 0; j < ncols; ++j) {
-        float* part = p.ws + ((int64_t)(tile * C::NW + j) * p.splits + split) * C::SLOT;
+        float* part = p.ws + (((int64_t)tile * p.splits + split) * C::NW + j) * C::SLOT;
         const int64_t out0 = (int64_t)run.out_blk[j] * B * B + (int64_t)row_in_block * B;
 #pragma unroll 1
         for (int cc = par; cc < B / 32; cc += kRunEpiWarps / 4) {
@@ -189,55 +189,11 @@ __global__ void __launch_bounds__(kRunThreads, 1) block_grad_runs_kernel(const _
   }
 
   if (p.counters != nullptr) {
-    // ===== fused split-K reduction (cooperative launch: all CTAs are resident) =====
-    __threadfence();
-    __syncthreads();
-    int* arrive = p.counters + 2 * tile;
-    if (threadIdx.x == 0) {
-      atomicAdd(arrive, 1);
-      const long long t0 = clock64();
-      while (ld_acquire_gpu(arrive) < p.splits) {
-        __nanosleep(64);
-        if (clock64() - t0 > 4000000000ll) {
-          printf("smt_block_grad_gemm_runs: split-K arrival wait timed out (tile %d split %d)\n", tile, split);
-          __trap();
-        }
-      }
-    }
-    __syncthreads();
-    // my slice of the run's ncols * SLOT elements, summed over the partials in the fixed order 0..splits-1
-    const int total = ncols * C::SLOT;
-    const int chunk = ((total / 8 + p.splits - 1) / p.splits) * 8;
-    const int e_begin = split * chunk, e_end = min(e_begin + chunk, total);
-    for (int e = e_begin + (int)threadIdx.x * 8; e < e_end; e += (int)blockDim.x * 8) {
-      const int j = e / C::SLOT, within = e - j * C::SLOT;
-      const float* src0 = p.ws + (int64_t)(tile * C::NW + j) * p.splits * C::SLOT + within;
-      float acc[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-      for (int sp = 0; sp < p.splits; ++sp) {
-        const float4 a = ld_cg_f4(src0 + (int64_t)sp * C::SLOT), b4 = ld_cg_f4(src0 + (int64_t)sp * C::SLOT + 4);
-        acc[0] += a.x; acc[1] += a.y; acc[2] += a.z; acc[3] += a.w;
-        acc[4] += b4.x; acc[5] += b4.y; acc[6] += b4.z; acc[7] += b4.w;
-      }
-      const int64_t o = (int64_t)run.out_blk[j] * B * B + within;
-      const float4 v0 = make_float4(acc[0], acc[1], acc[2], acc[3]), v1 = make_float4(acc[4], acc[5], acc[6], acc[7]);
-      if (p.out_dtype == SMT_F32) {
-        if (p.accumulate) { store4<SMT_F32, true>(p.out, o, v0); store4<SMT_F32, true>(p.out, o + 4, v1); }
-        else { store4<SMT_F32, false>(p.out, o, v0); store4<SMT_F32, false>(p.out, o + 4, v1); }
-      } else if (p.out_dtype == SMT_BF16) {
-        if (p.accumulate) { store4<SMT_BF16, true>(p.out, o, v0); store4<SMT_BF16, true>(p.out, o + 4, v1); }
-        else { store4<SMT_BF16, false>(p.out, o, v0); store4<SMT_BF16, false>(p.out, o + 4, v1); }
-      } else {
-        if (p.accumulate) { store4<SMT_F16, true>(p.out, o, v0); store4<SMT_F16, true>(p.out, o + 4, v1); }
-        else { store4<SMT_F16, false>(p.out, o, v0); store4<SMT_F16, false>(p.out, o + 4, v1); }
-      }
-    }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-      if (atomicAdd(arrive + 1, 1) == p.splits - 1) {   // every sibling has passed its wait: safe to re-arm
-        arrive[0] = 0;
-        arrive[1] = 0;
-      }
-    }
+    // a split's partial of the run is one tile of NW slots; element e lives in slot e / SLOT of the run
+    fused_splitk_reduce(p.counters + 2 * tile, split, p.splits, p.ws + (int64_t)tile * p.splits * C::NW * C::SLOT,
+                        C::NW * C::SLOT, ncols * C::SLOT, p.out, p.out_dtype, p.accumulate != 0,
+                        [&](int e) { return (int64_t)run.out_blk[e / C::SLOT] * B * B + e % C::SLOT; },
+                        "smt_block_grad_gemm_runs");
   }
 }
 
@@ -274,27 +230,8 @@ RunPlan make_run_plan(int n_runs, int block, int64_t T) {
 
 size_t run_workspace_bytes(int n_runs, int block, const RunPlan& pl) {
   if (pl.splits <= 1) return 0;
-  return kRunCounterBytes + (size_t)n_runs * run_width(block) * pl.splits * run_slot(block) * sizeof(float);
+  return kSplitCounterBytes + (size_t)n_runs * run_width(block) * pl.splits * run_slot(block) * sizeof(float);
 }
-
-template <int B>
-int launch_runs(const CUtensorMap& mx, const CUtensorMap& mdy, const RunParams& rp, int n_runs, cudaStream_t st) {
-  using C = RunCfg<B>;
-  auto kern = block_grad_runs_kernel<B>;
-  SMT_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES));
-  dim3 grid(n_runs, rp.splits);
-  if (rp.counters != nullptr) {
-    void* args[3] = {const_cast<CUtensorMap*>(&mx), const_cast<CUtensorMap*>(&mdy), const_cast<RunParams*>(&rp)};
-    SMT_CHECK_CUDA(cudaLaunchCooperativeKernel(reinterpret_cast<void*>(kern), grid, dim3(kRunThreads), args,
-                                               (size_t)C::SMEM_BYTES, st));
-    return SMT_OK;
-  }
-  kern<<<grid, kRunThreads, C::SMEM_BYTES, st>>>(mx, mdy, rp);
-  SMT_CHECK_LAUNCH();
-  return SMT_OK;
-}
-
-inline bool al16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
 }  // namespace
 }  // namespace smt
@@ -322,17 +259,17 @@ extern "C" SMT_API int smt_block_grad_gemm_runs(const void* x, int64_t ldx, int 
   SMT_CHECK_ARG(in_features > 0 && out_features > 0 && in_features % block == 0 && out_features % block == 0,
                 "smt_block_grad_gemm_runs: features (%d in, %d out) must be multiples of block %d", in_features,
                 out_features, block);
-  SMT_CHECK_ARG(ldx >= in_features && lddy >= out_features && al16(x) && al16(dy) && al16(G) && (ldx * 2) % 16 == 0 &&
-                    (lddy * 2) % 16 == 0,
+  SMT_CHECK_ARG(ldx >= in_features && lddy >= out_features && aligned16(x) && aligned16(dy) && aligned16(G) &&
+                    (ldx * 2) % 16 == 0 && (lddy * 2) % 16 == 0,
                 "smt_block_grad_gemm_runs: operands must be 16-byte aligned (pointer and row pitch)");
   SMT_CHECK_ARG(T < (1ll << 31) - 256, "smt_block_grad_gemm_runs: T too large");
   const RunPlan pl = make_run_plan(n_runs, block, T);
-  const size_t need = run_workspace_bytes(n_runs, block, pl);
-  if (need > 0 && (workspace == nullptr || workspace_bytes < need)) {
-    set_error("smt_block_grad_gemm_runs: workspace too small (%zu < %zu)", workspace_bytes, need);
-    return SMT_ERR_WORKSPACE;
-  }
-  SMT_CHECK_ARG(need == 0 || ((size_t)n_runs * 2 * sizeof(int) <= kRunCounterBytes && al16(workspace)),
+  int* counters;
+  float* partials;
+  if (int rc = carve_split_workspace("smt_block_grad_gemm_runs", workspace, workspace_bytes,
+                                     run_workspace_bytes(n_runs, block, pl), &counters, &partials))
+    return rc;
+  SMT_CHECK_ARG(counters == nullptr || (size_t)n_runs * 2 * sizeof(int) <= kSplitCounterBytes,
                 "smt_block_grad_gemm_runs: too many runs for a split launch");
   CUtensorMap mx, mdy;
   if (int rc = encode_strip_map(&mx, x, in_features, T, ldx, in_dtype, run_ktile(block))) return rc;
@@ -340,8 +277,8 @@ extern "C" SMT_API int smt_block_grad_gemm_runs(const void* x, int64_t ldx, int 
   RunParams rp{};
   rp.runs = runs;
   rp.out = G;
-  rp.ws = need > 0 ? reinterpret_cast<float*>(reinterpret_cast<char*>(workspace) + kRunCounterBytes) : nullptr;
-  rp.counters = need > 0 ? reinterpret_cast<int*>(workspace) : nullptr;
+  rp.ws = partials;
+  rp.counters = counters;
   rp.splits = pl.splits;
   rp.kt_total = pl.kt_total;
   rp.kt_per_split = pl.kt_per_split;
@@ -349,9 +286,11 @@ extern "C" SMT_API int smt_block_grad_gemm_runs(const void* x, int64_t ldx, int 
   rp.accumulate = accumulate;
   rp.in_fmt = in_dtype == SMT_BF16 ? 1 : 0;
   cudaStream_t st = (cudaStream_t)stream;
-  int rc;
-  if (block == 128) rc = launch_runs<128>(mx, mdy, rp, n_runs, st);
-  else rc = launch_runs<64>(mx, mdy, rp, n_runs, st);
+  const dim3 grid(n_runs, pl.splits);
+  const bool coop = counters != nullptr;
+  const int rc = block == 128
+                     ? launch_tiles(block_grad_runs_kernel<128>, grid, kRunThreads, RunCfg<128>::SMEM_BYTES, coop, st, mx, mdy, rp)
+                     : launch_tiles(block_grad_runs_kernel<64>, grid, kRunThreads, RunCfg<64>::SMEM_BYTES, coop, st, mx, mdy, rp);
   if (rc) return rc;
   set_launch_count(1);
   return SMT_OK;

@@ -51,6 +51,7 @@ inline int sm_count() {
 
 inline bool block_ok(int b) { return b == 64 || b == 128 || b == 256; }
 inline int dtype_bytes(int dt) { return dt == SMT_F32 ? 4 : 2; }
+inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
 
 // ---- device helpers ------------------------------------------------------------------------
 

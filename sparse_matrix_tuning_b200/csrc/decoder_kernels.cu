@@ -129,8 +129,6 @@ int row_threads(int nvec) {
   return t < 32 ? 32 : t;
 }
 
-bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
-
 // ---- rotary position embedding ---------------------------------------------------------------------------------
 // Rows of 128 (head_dim) elements; work item j (0..7) of a row owns elements [8j, 8j+8) and their rotation partners
 // [64+8j, 64+8j+8).  q rows come first, then k rows; row r of q belongs to token r / Hq (token = b*S + s).

@@ -291,8 +291,6 @@ int encode_dense_map(CUtensorMap* map, const void* base, int64_t cols, int64_t r
   return encode_2d_sw128(map, base, cols, rows, ld, dtype, box_rows, "smt_fused_linear");
 }
 
-inline bool al16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
-
 template <bool DGRAD>
 int launch_dense(const DenseMaps& maps, const DenseParams& p, cudaStream_t st) {
   auto kern = fused_dense_umma_2sm_kernel<DGRAD>;
@@ -330,7 +328,7 @@ int check_common(const char* who, int64_t T, int n_seg, const void* const* W, co
   SMT_CHECK_ARG(K > 0 && K % 64 == 0, "%s: in_features %d must be a multiple of 64", who, K);
   SMT_CHECK_ARG(W && ldw && N, "%s: null pointer", who);
   for (int j = 0; j < n_seg; ++j) {
-    SMT_CHECK_ARG(W[j] && al16(W[j]) && ldw[j] >= K && (ldw[j] * 2) % 16 == 0,
+    SMT_CHECK_ARG(W[j] && aligned16(W[j]) && ldw[j] >= K && (ldw[j] * 2) % 16 == 0,
                   "%s: weight %d must be 16-byte aligned with a row pitch >= in_features", who, j);
     SMT_CHECK_ARG(N[j] > 0 && N[j] % 64 == 0, "%s: out_features %d of segment %d must be a multiple of 64", who, N[j], j);
   }
@@ -357,7 +355,7 @@ extern "C" SMT_API int smt_fused_linear_forward(const void* x, int64_t ldx, int6
                                                 void* const* y_host, const int64_t* ldy_host, int dtype, void* stream) {
   if (int rc = check_common("smt_fused_linear_forward", T, n_seg, W_host, ldw_host, N_host, K, dtype)) return rc;
   if (T == 0) return SMT_OK;
-  SMT_CHECK_ARG(x && al16(x) && ldx >= K && (ldx * 2) % 16 == 0, "smt_fused_linear_forward: x must be 16-byte aligned");
+  SMT_CHECK_ARG(x && aligned16(x) && ldx >= K && (ldx * 2) % 16 == 0, "smt_fused_linear_forward: x must be 16-byte aligned");
   SMT_CHECK_ARG(y_host && ldy_host, "smt_fused_linear_forward: null pointer");
   DenseMaps maps;
   memset(&maps, 0, sizeof(maps));
@@ -372,7 +370,7 @@ extern "C" SMT_API int smt_fused_linear_forward(const void* x, int64_t ldx, int6
     SMT_CHECK_ARG(N_host[j] % kDenseTileN == 0,
                   "smt_fused_linear_forward: out_features %d of segment %d must be a multiple of %d", N_host[j], j,
                   kDenseTileN);
-    SMT_CHECK_ARG(y_host[j] && al16(y_host[j]) && ldy_host[j] >= N_host[j] && (ldy_host[j] * 2) % 16 == 0,
+    SMT_CHECK_ARG(y_host[j] && aligned16(y_host[j]) && ldy_host[j] >= N_host[j] && (ldy_host[j] * 2) % 16 == 0,
                   "smt_fused_linear_forward: output %d must be 16-byte aligned with a row pitch >= out_features", j);
     if (int rc = encode_dense_map(&maps.b[j], W_host[j], K, N_host[j], ldw_host[j], dtype, 128)) return rc;
     p.seg_len[j] = N_host[j];
@@ -396,7 +394,7 @@ extern "C" SMT_API int smt_fused_linear_dgrad(const void* const* dy_host, const 
   if (int rc = check_common("smt_fused_linear_dgrad", T, n_seg, W_host, ldw_host, N_host, K, dtype)) return rc;
   if (T == 0) return SMT_OK;
   SMT_CHECK_ARG(dy_host && lddy_host, "smt_fused_linear_dgrad: null pointer");
-  SMT_CHECK_ARG(dx && al16(dx) && lddx >= K && (lddx * 2) % 16 == 0, "smt_fused_linear_dgrad: dx must be 16-byte aligned");
+  SMT_CHECK_ARG(dx && aligned16(dx) && lddx >= K && (lddx * 2) % 16 == 0, "smt_fused_linear_dgrad: dx must be 16-byte aligned");
   DenseMaps maps;
   memset(&maps, 0, sizeof(maps));
   DenseParams p{};
@@ -405,7 +403,7 @@ extern "C" SMT_API int smt_fused_linear_dgrad(const void* const* dy_host, const 
   p.k_or_n = K;
   p.in_fmt = dtype == SMT_BF16 ? 1 : 0;
   for (int j = 0; j < n_seg; ++j) {
-    SMT_CHECK_ARG(dy_host[j] && al16(dy_host[j]) && lddy_host[j] >= N_host[j] && (lddy_host[j] * 2) % 16 == 0,
+    SMT_CHECK_ARG(dy_host[j] && aligned16(dy_host[j]) && lddy_host[j] >= N_host[j] && (lddy_host[j] * 2) % 16 == 0,
                   "smt_fused_linear_dgrad: dy %d must be 16-byte aligned with a row pitch >= out_features", j);
     if (int rc = encode_dense_map(&maps.a[j], dy_host[j], N_host[j], T, lddy_host[j], dtype, 128)) return rc;
     if (int rc = encode_dense_map(&maps.b[j], W_host[j], K, N_host[j], ldw_host[j], dtype, 64)) return rc;

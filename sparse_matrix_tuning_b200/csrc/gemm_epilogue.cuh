@@ -1,5 +1,6 @@
 // Epilogue helpers shared by the block-gradient kernels: accumulator sub-tile -> global memory through a per-warp
-// shared-memory transpose (every store instruction writes whole rows), and the L2-coherent loads of the split-K fix-up.
+// shared-memory transpose (every store instruction writes whole rows), and the split-K reduction of partial tiles
+// (device side and the host's workspace layout and launch).
 #pragma once
 
 #include "common.cuh"
@@ -96,6 +97,118 @@ __device__ __forceinline__ int ld_acquire_gpu(const int* p) {
   int v;
   asm volatile("ld.acquire.gpu.global.s32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
   return v;
+}
+
+// ---- split-K: fp32 partial tiles in a workspace, summed in the fixed split order ----------------------------------
+
+// acc = sum over s = 0..splits-1, in that order, of the 8 floats at src + s * stride.  Every split-K reduction (fused
+// and separate) sums through this loop, which is what makes their results bit-identical.  LOAD is ld_cg_f4 for
+// partials written by sibling CTAs of the same grid, ld_stream_f4 for partials of an earlier grid.
+template <auto LOAD>
+__device__ __forceinline__ void sum_partials8(const float* src, int splits, int64_t stride, float (&acc)[8]) {
+#pragma unroll
+  for (int j = 0; j < 8; ++j) acc[j] = 0.f;
+  // unrolled 4 deep: left to itself the compiler unrolls 8 deep, +18 registers in the b = 64 block kernels
+#pragma unroll 4
+  for (int s = 0; s < splits; ++s) {
+    const float4 a = LOAD(src + s * stride), b = LOAD(src + s * stride + 4);
+    acc[0] += a.x; acc[1] += a.y; acc[2] += a.z; acc[3] += a.w;
+    acc[4] += b.x; acc[5] += b.y; acc[6] += b.z; acc[7] += b.w;
+  }
+}
+
+template <int ODT, class OutOff>
+__device__ __forceinline__ void fused_reduce_slice(const float* part0, int64_t stride, int splits, int e_begin, int e_end,
+                                                   void* out, bool acc_out, const OutOff& out_off) {
+  for (int e = e_begin + (int)threadIdx.x * 8; e < e_end; e += (int)blockDim.x * 8) {
+    float acc[8];
+    sum_partials8<ld_cg_f4>(part0 + e, splits, stride, acc);
+    const int64_t o = out_off(e);
+    const float4 v0 = make_float4(acc[0], acc[1], acc[2], acc[3]), v1 = make_float4(acc[4], acc[5], acc[6], acc[7]);
+    if (acc_out) {
+      store4<ODT, true>(out, o, v0);
+      store4<ODT, true>(out, o + 4, v1);
+    } else {
+      store4<ODT, false>(out, o, v0);
+      store4<ODT, false>(out, o + 4, v1);
+    }
+  }
+}
+
+// Fused split-K reduction, called by every CTA of a tile once its epilogue has stored the CTA's fp32 partial.  CTAs
+// wait on their siblings, so the grid must have been launched cooperatively (all CTAs resident).  When the tile's
+// arrival counter reaches `splits`, CTA `split` sums its slice of the tile's `total` elements over all partials
+// (partial s at part0 + s * stride) and stores element e at out_off(e) of `out`; out_off must map 8 consecutive
+// elements to 8 consecutive outputs.  The last CTA to finish re-arms the tile's two counters, so the counters are all
+// zero again when the kernel ends.  `who` names the kernel's entry point in the timeout message; the callers' grids
+// are (tile, split).
+template <class OutOff>
+__device__ __forceinline__ void fused_splitk_reduce(int* counters, int split, int splits, const float* part0,
+                                                    int64_t stride, int total, void* out, int out_dtype, bool acc_out,
+                                                    const OutOff& out_off, const char* who) {
+  __threadfence();                     // this thread's partial-tile stores are visible device-wide ...
+  __syncthreads();                     // ... for every thread of the CTA, before the CTA announces itself
+  if (threadIdx.x == 0) {
+    atomicAdd(counters, 1);
+    const long long t0 = clock64();
+    while (ld_acquire_gpu(counters) < splits) {
+      __nanosleep(64);
+      if (clock64() - t0 > 4000000000ll) {
+        printf("%s: split-K arrival wait timed out (tile %d split %d)\n", who, (int)blockIdx.x, split);
+        __trap();
+      }
+    }
+  }
+  __syncthreads();
+  const int chunk = ((total / 8 + splits - 1) / splits) * 8;
+  const int e_begin = split * chunk, e_end = min(e_begin + chunk, total);
+  if (out_dtype == SMT_F32) fused_reduce_slice<SMT_F32>(part0, stride, splits, e_begin, e_end, out, acc_out, out_off);
+  else if (out_dtype == SMT_BF16) fused_reduce_slice<SMT_BF16>(part0, stride, splits, e_begin, e_end, out, acc_out, out_off);
+  else fused_reduce_slice<SMT_F16>(part0, stride, splits, e_begin, e_end, out, acc_out, out_off);
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    if (atomicAdd(counters + 1, 1) == splits - 1) {   // every sibling has passed its wait: safe to re-arm
+      counters[0] = 0;
+      counters[1] = 0;
+    }
+  }
+}
+
+// Head of a split-K workspace: 2 self-resetting arrival counters per tile (zero when the workspace is handed over).
+constexpr size_t kSplitCounterBytes = 16384;
+
+// Checks the workspace of a launch that needs `need` bytes of it (0: no split) and splits it into the arrival
+// counters and the fp32 partials that follow them.
+inline int carve_split_workspace(const char* who, void* workspace, size_t workspace_bytes, size_t need, int** counters,
+                                 float** partials) {
+  *counters = nullptr;
+  *partials = nullptr;
+  if (need == 0) return SMT_OK;
+  if (workspace == nullptr || workspace_bytes < need) {
+    set_error("%s: workspace too small (%zu < %zu)", who, workspace_bytes, need);
+    return SMT_ERR_WORKSPACE;
+  }
+  SMT_CHECK_ARG(aligned16(workspace), "%s: workspace must be 16-byte aligned", who);
+  *counters = static_cast<int*>(workspace);
+  *partials = reinterpret_cast<float*>(static_cast<char*>(workspace) + kSplitCounterBytes);
+  return SMT_OK;
+}
+
+// Launches a grid of tile CTAs: cooperatively when they run fused_splitk_reduce (which is only safe when the whole grid
+// is resident), with <<<>>> otherwise.
+template <class... Args>
+int launch_tiles(void (*kern)(Args...), dim3 grid, int threads, int smem_bytes, bool cooperative, cudaStream_t st,
+                 const Args&... args) {
+  SMT_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
+  if (cooperative) {
+    void* argv[] = {const_cast<Args*>(&args)...};
+    SMT_CHECK_CUDA(cudaLaunchCooperativeKernel(reinterpret_cast<void*>(kern), grid, dim3(threads), argv,
+                                               (size_t)smem_bytes, st));
+    return SMT_OK;
+  }
+  kern<<<grid, threads, smem_bytes, st>>>(args...);
+  SMT_CHECK_LAUNCH();
+  return SMT_OK;
 }
 
 }  // namespace

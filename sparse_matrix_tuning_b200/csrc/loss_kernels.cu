@@ -142,7 +142,7 @@ extern "C" SMT_API int smt_cross_entropy_rows(void* logits, int64_t ldl, int64_t
                 (long long)ldl);
   if (T == 0) return SMT_OK;
   SMT_CHECK_ARG(logits && labels && scale && loss_rows, "smt_cross_entropy_rows: null pointer");
-  SMT_CHECK_ARG((reinterpret_cast<uintptr_t>(logits) & 15u) == 0, "smt_cross_entropy_rows: logits must be 16-byte aligned");
+  SMT_CHECK_ARG(smt::aligned16(logits), "smt_cross_entropy_rows: logits must be 16-byte aligned");
   smt::ce_rows_kernel<<<(unsigned)T, smt::kCeThreads, 0, (cudaStream_t)stream>>>(
       (uint16_t*)logits, ldl, V, labels, ignore_index, scale, loss_rows);
   SMT_CHECK_LAUNCH();

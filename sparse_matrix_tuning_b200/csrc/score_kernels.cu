@@ -369,8 +369,6 @@ inline int streaming_grid(int64_t work_items) {
   return (int)(want < cap ? (want < 1 ? 1 : want) : cap);
 }
 
-inline bool aligned16(const void* p) { return (reinterpret_cast<uintptr_t>(p) & 15u) == 0; }
-
 }  // namespace
 }  // namespace smt
 

@@ -572,10 +572,20 @@ def test_fused_and_separate_split_k_reduction_are_bit_identical(api, monkeypatch
         plain = [ops.block_grad_gemm(x, dy, rc, b, out_dtype=dt) for dt in (torch.float32, torch.bfloat16)]
         monkeypatch.delenv("SMT_GEMM_NO_FUSED_REDUCE", raising=False)
         assert torch.equal(fused[0], plain[0]) and torch.equal(fused[1], plain[1]) and torch.equal(fused[0], again)
-    # many back-to-back launches re-arm the arrival counters correctly
+    # many back-to-back launches re-arm the arrival counters correctly, in the block-tile kernel and in the run-tile
+    # kernel (b = 64 / 128; runs of 1 to 4 / 2 blocks), which calls the same fused reduction; launches interleaved
+    runs = []
+    for rb in (64, 128):
+        nb = 1024 // rb
+        idx = list(dict.fromkeys([(0, 3), (0, 1), (3, 0), (0, 0), (2, 2), (0, 2), (3, 3), (1, 1), (3, 1), (0, nb - 1)]))
+        args = (x, dy, ops._runs_for(idx, rb, x.device), rb)
+        assert ops.load().smt_block_grad_gemm_runs_workspace_bytes(args[2][1], rb, T) > 0          # split-K
+        runs.append((args, ops._gemm_runs(*args, torch.empty((len(idx) * rb, rb), device="cuda"), False)))
     ref = ops.block_grad_gemm(x, dy, rc, b, out_dtype=torch.float32)
     for _ in range(50):
         assert torch.equal(ops.block_grad_gemm(x, dy, rc, b, out_dtype=torch.float32), ref)
+        for args, want in runs:
+            assert torch.equal(ops._gemm_runs(*args, torch.empty_like(want), False), want)
 
 
 def test_config1_bf16_steady_state_vs_reference_golden(api):
