@@ -324,7 +324,7 @@ int check_common(const char* who, int64_t T, int n_seg, const void* const* W, co
                  int dtype) {
   SMT_CHECK_ARG(n_seg >= 1 && n_seg <= kMaxSeg, "%s: 1..3 segments, got %d", who, n_seg);
   SMT_CHECK_ARG(dtype == SMT_BF16 || dtype == SMT_F16, "%s: 16-bit operands only", who);
-  SMT_CHECK_ARG(T >= 0 && T < (1ll << 31) - 512, "%s: bad token count", who);
+  SMT_CHECK_ARG(T >= 0 && T < (1ll << 31) - 512, "%s: token count %lld outside [0, 2^31 - 512)", who, (long long)T);
   SMT_CHECK_ARG(K > 0 && K % 64 == 0, "%s: in_features %d must be a multiple of 64", who, K);
   SMT_CHECK_ARG(W && ldw && N, "%s: null pointer", who);
   for (int j = 0; j < n_seg; ++j) {
@@ -355,8 +355,18 @@ extern "C" SMT_API int smt_fused_linear_forward(const void* x, int64_t ldx, int6
                                                 void* const* y_host, const int64_t* ldy_host, int dtype, void* stream) {
   if (int rc = check_common("smt_fused_linear_forward", T, n_seg, W_host, ldw_host, N_host, K, dtype)) return rc;
   if (T == 0) return SMT_OK;
-  SMT_CHECK_ARG(x && aligned16(x) && ldx >= K && (ldx * 2) % 16 == 0, "smt_fused_linear_forward: x must be 16-byte aligned");
+  // every argument is checked before the first map is encoded, so a rejection never depends on the driver
+  SMT_CHECK_ARG(x && aligned16(x) && ldx >= K && (ldx * 2) % 16 == 0,
+                "smt_fused_linear_forward: x must be 16-byte aligned with a 16-byte row pitch >= in_features");
   SMT_CHECK_ARG(y_host && ldy_host, "smt_fused_linear_forward: null pointer");
+  for (int j = 0; j < n_seg; ++j) {
+    SMT_CHECK_ARG(N_host[j] % kDenseTileN == 0,
+                  "smt_fused_linear_forward: out_features %d of segment %d must be a multiple of %d", N_host[j], j,
+                  kDenseTileN);
+    SMT_CHECK_ARG(y_host[j] && aligned16(y_host[j]) && ldy_host[j] >= N_host[j] && (ldy_host[j] * 2) % 16 == 0,
+                  "smt_fused_linear_forward: output %d must be 16-byte aligned with a 16-byte row pitch >= out_features",
+                  j);
+  }
   DenseMaps maps;
   memset(&maps, 0, sizeof(maps));
   DenseParams p{};
@@ -367,11 +377,6 @@ extern "C" SMT_API int smt_fused_linear_forward(const void* x, int64_t ldx, int6
   if (int rc = encode_dense_map(&maps.a[0], x, K, T, ldx, dtype, 128)) return rc;
   int tiles = 0;
   for (int j = 0; j < n_seg; ++j) {
-    SMT_CHECK_ARG(N_host[j] % kDenseTileN == 0,
-                  "smt_fused_linear_forward: out_features %d of segment %d must be a multiple of %d", N_host[j], j,
-                  kDenseTileN);
-    SMT_CHECK_ARG(y_host[j] && aligned16(y_host[j]) && ldy_host[j] >= N_host[j] && (ldy_host[j] * 2) % 16 == 0,
-                  "smt_fused_linear_forward: output %d must be 16-byte aligned with a row pitch >= out_features", j);
     if (int rc = encode_dense_map(&maps.b[j], W_host[j], K, N_host[j], ldw_host[j], dtype, 128)) return rc;
     p.seg_len[j] = N_host[j];
     p.seg_tile0[j] = tiles;
@@ -393,8 +398,13 @@ extern "C" SMT_API int smt_fused_linear_dgrad(const void* const* dy_host, const 
                                               const int* N_host, void* dx, int64_t lddx, int dtype, void* stream) {
   if (int rc = check_common("smt_fused_linear_dgrad", T, n_seg, W_host, ldw_host, N_host, K, dtype)) return rc;
   if (T == 0) return SMT_OK;
+  // every argument is checked before the first map is encoded, so a rejection never depends on the driver
   SMT_CHECK_ARG(dy_host && lddy_host, "smt_fused_linear_dgrad: null pointer");
-  SMT_CHECK_ARG(dx && aligned16(dx) && lddx >= K && (lddx * 2) % 16 == 0, "smt_fused_linear_dgrad: dx must be 16-byte aligned");
+  for (int j = 0; j < n_seg; ++j)
+    SMT_CHECK_ARG(dy_host[j] && aligned16(dy_host[j]) && lddy_host[j] >= N_host[j] && (lddy_host[j] * 2) % 16 == 0,
+                  "smt_fused_linear_dgrad: dy %d must be 16-byte aligned with a 16-byte row pitch >= out_features", j);
+  SMT_CHECK_ARG(dx && aligned16(dx) && lddx >= K && (lddx * 2) % 16 == 0,
+                "smt_fused_linear_dgrad: dx must be 16-byte aligned with a 16-byte row pitch >= in_features");
   DenseMaps maps;
   memset(&maps, 0, sizeof(maps));
   DenseParams p{};
@@ -403,8 +413,6 @@ extern "C" SMT_API int smt_fused_linear_dgrad(const void* const* dy_host, const 
   p.k_or_n = K;
   p.in_fmt = dtype == SMT_BF16 ? 1 : 0;
   for (int j = 0; j < n_seg; ++j) {
-    SMT_CHECK_ARG(dy_host[j] && aligned16(dy_host[j]) && lddy_host[j] >= N_host[j] && (lddy_host[j] * 2) % 16 == 0,
-                  "smt_fused_linear_dgrad: dy %d must be 16-byte aligned with a row pitch >= out_features", j);
     if (int rc = encode_dense_map(&maps.a[j], dy_host[j], N_host[j], T, lddy_host[j], dtype, 128)) return rc;
     if (int rc = encode_dense_map(&maps.b[j], W_host[j], K, N_host[j], ldw_host[j], dtype, 64)) return rc;
     p.seg_len[j] = N_host[j];
