@@ -328,6 +328,31 @@ SMT_API int smt_compact_adam(float* master, float* exp_avg, float* exp_avg_sq,
                      const smt_block_ref* table, int n_blocks, int block, int w_dtype,
                      void* stream);
 
+/* One selected weight column (channel sparsity, smt.py:185-217 with column semantics): arena elements
+ * [off, off + n_out) hold W[0 .. n_out), col]. */
+typedef struct smt_column_ref {
+  uint64_t w_ptr;   /* device address of the dense weight W                                    */
+  int64_t  ldw;     /* leading dimension of W, elements                                         */
+  int64_t  off;     /* arena element offset of this channel's row, a multiple of 8                */
+  int32_t  col;     /* weight column (input channel), 0 <= col < ldw                            */
+  int32_t  n_out;   /* rows of W written (out_features), a multiple of 8                       */
+} smt_column_ref;
+/* The AdamW step of smt_compact_adam over the arena rows of `columns` (n_columns entries, any number of weights), with
+ * the write-back of every updated element into its weight column: element off + o is rounded to `w_dtype` into
+ * W[o, col] (and to `compact_dtype` into compact_out[off + o] when compact_out != NULL).  Same arithmetic, clip and
+ * argument checks as smt_compact_adam: given the same inputs, master / exp_avg / exp_avg_sq of the covered elements are
+ * bit-identical to its result.  Arena elements no entry covers are not touched.  The table is device memory the entry
+ * point cannot read: an entry outside [0, n_elems), with an unaligned `off` / `n_out` or a column outside [0, ldw) is
+ * skipped by the kernel.  Entries must not overlap. */
+SMT_API int smt_compact_adam_columns(float* master, float* exp_avg, float* exp_avg_sq,
+                     const void* grad, int grad_dtype, int64_t n_elems,
+                     float lr, float beta1, float beta2, float eps, float weight_decay,
+                     float bias_correction1, float bias_correction2,
+                     float grad_scale, const float* sqnorm, int n_sqnorm, float max_norm,
+                     void* compact_out, int compact_dtype,
+                     const smt_column_ref* columns, int n_columns, int w_dtype,
+                     void* stream);
+
 #ifdef __cplusplus
 }
 #endif

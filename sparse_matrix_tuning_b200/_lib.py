@@ -26,6 +26,12 @@ class BlockRef(C.Structure):
     _fields_ = [("w_ptr", C.c_uint64), ("ldw", C.c_int64), ("row", C.c_int32), ("col", C.c_int32)]
 
 
+class ColumnRef(C.Structure):
+    """Mirror of `smt_column_ref`."""
+    _fields_ = [("w_ptr", C.c_uint64), ("ldw", C.c_int64), ("off", C.c_int64), ("col", C.c_int32),
+                ("n_out", C.c_int32)]
+
+
 class GemmItem(C.Structure):
     """Mirror of `smt_gemm_item`."""
     _fields_ = [("map_dy", C.c_uint32), ("map_x", C.c_uint32), ("row", C.c_int32), ("col", C.c_int32),
@@ -96,6 +102,10 @@ _SIGNATURES = {
     "smt_compact_adam": (C.c_int, [_P, _P, _P, _P, C.c_int, C.c_int64,
                                    C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float,
                                    C.c_float, _P, C.c_int, C.c_float, _P, C.c_int, _P, C.c_int, C.c_int, C.c_int, _P]),
+    "smt_compact_adam_columns": (C.c_int, [_P, _P, _P, _P, C.c_int, C.c_int64,
+                                           C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float,
+                                           C.c_float, C.c_float, _P, C.c_int, C.c_float, _P, C.c_int, _P, C.c_int,
+                                           C.c_int, _P]),
 }
 EXPORTS = tuple(_SIGNATURES)
 

@@ -11,7 +11,7 @@ from typing import Optional, Sequence, Tuple
 import torch
 
 from . import _lib
-from ._lib import BlockRef, check, dtype_id, load, ptr, require_cuda, stream_ptr
+from ._lib import BlockRef, ColumnRef, check, dtype_id, load, ptr, require_cuda, stream_ptr
 
 STRATEGY_IDS = _lib.STRATEGY_IDS
 
@@ -91,6 +91,28 @@ def make_block_table(entries: Sequence[Tuple[torch.Tensor, int, int]], device) -
         arr[i].row = int(r)
         arr[i].col = int(c)
     host = torch.frombuffer(bytearray(bytes(arr)), dtype=torch.uint8)[: n * C.sizeof(BlockRef)].clone()
+    return host.to(device)
+
+
+def make_column_table(entries: Sequence[Tuple[torch.Tensor, int, int]], device) -> torch.Tensor:
+    """Device array of `smt_column_ref` for [(weight, column, arena offset), ...]: arena elements
+    [offset, offset + weight.shape[0]) hold column `column` of `weight` (uint8 tensor view)."""
+    n = len(entries)
+    arr = (ColumnRef * max(n, 1))()
+    for i, (w, col, off) in enumerate(entries):
+        if w.dim() != 2 or w.stride(1) != 1:
+            raise _lib.SMTLibraryError("column table: weights must be 2-D with unit column stride")
+        if not 0 <= int(col) < w.shape[1]:
+            raise _lib.SMTLibraryError(f"column table: column {col} outside a weight with {w.shape[1]} columns")
+        if int(off) < 0 or int(off) % 8 or w.shape[0] % 8:
+            raise _lib.SMTLibraryError("column table: arena offsets and out_features must be multiples of 8; got offset "
+                                       f"{off}, out_features {w.shape[0]}")
+        arr[i].w_ptr = w.data_ptr()
+        arr[i].ldw = w.stride(0)
+        arr[i].off = int(off)
+        arr[i].col = int(col)
+        arr[i].n_out = w.shape[0]
+    host = torch.frombuffer(bytearray(bytes(arr)), dtype=torch.uint8)[: n * C.sizeof(ColumnRef)].clone()
     return host.to(device)
 
 
@@ -326,14 +348,33 @@ _ws_cache: dict = {}
 _channel_items: dict = {}
 
 
-def channel_grad_gemm(partial: torch.Tensor, n: int, dy2d: torch.Tensor) -> torch.Tensor:
+def channel_grad_block(n: int, out_f: int) -> int:
+    """Tile size of the channel-gradient launches: [n, out_f] is covered by ceil(n/b) x out_f/b tiles of b x b."""
+    return 128 if (out_f % 128 == 0 and n > 64) else 64
+
+
+def _channel_tiles(rows: int, cols: int) -> tuple:
+    key = ("tiles", rows, cols)
+    hit = _channel_items.get(key)
+    if hit is None:
+        hit = tuple((r, c) for r in range(rows) for c in range(cols))
+        if len(_channel_items) > 64:
+            _channel_items.clear()
+        _channel_items[key] = hit
+    return hit
+
+
+def channel_grad_gemm(partial: torch.Tensor, n: int, dy2d: torch.Tensor, out: Optional[torch.Tensor] = None,
+                      accumulate: bool = False) -> torch.Tensor:
     """grad[i, o] = sum_t partial[t, i] * dy[t, o] for the n selected input channels - the weight gradient of
     linearChannel.backward (smt.py:283-284: `partial_input^T @ grad_output`, summed over the batch) on the tcgen05
     block-gradient pipeline: the packed channels play the `dy` operand (their row blocks are padded by TMA zero fill),
     grad_output the `x` operand, and every (row block, column block) tile is stored with the row pitch of the result, so
     the tiles assemble the row-major [n, out_features] gradient directly.  fp32 accumulation over all tokens, ONE
-    rounding.  `partial`: [T, n8] (n8 >= n, row pitch a multiple of 16 bytes, columns >= n zero); returns [n, out]."""
-    require_cuda(partial, dy2d)
+    rounding.  `partial`: [T, n8] (n8 >= n, row pitch a multiple of 16 bytes, columns >= n zero); returns [n, out].
+    `out` (optional): contiguous [ceil(n/b)*b, out_features] destination (b = channel_grad_block(n, out_features)); its
+    rows past n receive zeros.  `accumulate` adds into it instead of overwriting it."""
+    require_cuda(partial, dy2d, out)
     _req(partial.dim() == 2 and dy2d.dim() == 2 and partial.shape[0] == dy2d.shape[0] and partial.dtype == dy2d.dtype,
          "partial.dim() == 2 and dy2d.dim() == 2 and partial.shape[0] == dy2d.shape[0] and partial.dtype == dy2d.dtype")
     _req(partial.stride(1) == 1 and dy2d.stride(1) == 1 and partial.dtype in (torch.bfloat16, torch.float16),
@@ -342,17 +383,24 @@ def channel_grad_gemm(partial: torch.Tensor, n: int, dy2d: torch.Tensor) -> torc
     _req(0 < n <= partial.shape[1] and (partial.stride(0) * 2) % 16 == 0 and (dy2d.stride(0) * 2) % 16 == 0,
          "0 < n <= partial.shape[1] and 16-byte row pitches")
     _req(out_f % 64 == 0, "out_features % 64 == 0")
-    block = 128 if (out_f % 128 == 0 and n > 64) else 64
+    block = channel_grad_block(n, out_f)
     rows, cols = (n + block - 1) // block, out_f // block
     dev = dy2d.device
-    out = torch.empty(rows * block, out_f, dtype=dy2d.dtype, device=dev)
+    if out is None:
+        out = torch.empty(rows * block, out_f, dtype=dy2d.dtype, device=dev)
+        accumulate = False
+    _req(out.is_contiguous() and out.shape == (rows * block, out_f) and out.dtype == dy2d.dtype,
+         "out: contiguous [ceil(n/b)*b, out_features] of dy's dtype")
     if T == 0:
-        return out.zero_()[:n]
+        if not accumulate:
+            out.zero_()
+        return out[:n]
     import numpy as np
-    key = (rows, cols, block, out_f)
+    key = (rows, cols, block, out_f, bool(accumulate))
     arr = _channel_items.get(key)
     if arr is None:
-        arr = np.array([(0, 1, r, c, r * block * out_f + c * block, _lib.ITEM_OVERWRITE, -1)
+        flags = 0 if accumulate else _lib.ITEM_OVERWRITE
+        arr = np.array([(0, 1, r, c, r * block * out_f + c * block, flags, -1)
                         for r in range(rows) for c in range(cols)], dtype=_item_dtype())
         if len(_channel_items) > 64:
             _channel_items.clear()
@@ -371,8 +419,8 @@ def channel_grad_gemm(partial: torch.Tensor, n: int, dy2d: torch.Tensor) -> torc
     ws = _workspace(ws_bytes, dev)
     with _timed("channel_grad_gemm", dev, (n, out_f, T)):
         check(lib.smt_block_grad_gemm_grouped(dev_buf.data_ptr(), dev_buf.data_ptr() + 256, n_items, T, block, in_id,
-                                              out.data_ptr(), dtype_id(out.dtype), 0, out_f, 0, ptr(ws), ws_bytes,
-                                              stream_ptr(dev)), "smt_block_grad_gemm_grouped")
+                                              out.data_ptr(), dtype_id(out.dtype), 1 if accumulate else 0, out_f, 0,
+                                              ptr(ws), ws_bytes, stream_ptr(dev)), "smt_block_grad_gemm_grouped")
     _count(lib.smt_last_launch_count())
     return out[:n]
 
@@ -731,13 +779,18 @@ def compact_adam(master: torch.Tensor, exp_avg: torch.Tensor, exp_avg_sq: torch.
                  *, lr: float, beta1: float, beta2: float, eps: float, weight_decay: float, step: int,
                  grad_scale: float = 1.0, sqnorm: Optional[torch.Tensor] = None, max_norm: float = 0.0,
                  compact_out: Optional[torch.Tensor] = None, table: Optional[torch.Tensor] = None,
-                 n_blocks: int = 0, block: int = 0, w_dtype: Optional[torch.dtype] = None) -> None:
-    """One fused AdamW step over flat compact state (+ clip, + dense write-back). See smt_b200.h."""
-    require_cuda(master, exp_avg, exp_avg_sq, grad, sqnorm, compact_out, table)
+                 n_blocks: int = 0, block: int = 0, w_dtype: Optional[torch.dtype] = None,
+                 columns: Optional[torch.Tensor] = None, n_columns: int = 0) -> None:
+    """One fused AdamW step over flat compact state (+ clip, + dense write-back). See smt_b200.h.
+    The write-back goes to weight blocks (`table` of make_block_table, `n_blocks`, `block`) or to weight columns
+    (`columns` of make_column_table, `n_columns`: smt_compact_adam_columns, which updates only the arena rows the
+    table covers)."""
+    require_cuda(master, exp_avg, exp_avg_sq, grad, sqnorm, compact_out, table, columns)
     for t in (master, exp_avg, exp_avg_sq):
         _req(t.dtype == torch.float32 and t.is_contiguous() and t.numel() == grad.numel(),
              "t.dtype == torch.float32 and t.is_contiguous() and t.numel() == grad.numel()")
     _req(grad.is_contiguous(), "grad.is_contiguous()")
+    _req(table is None or columns is None, "a block table or a column table, not both")
     n_sq = 0
     if sqnorm is not None:
         # one scalar (smt_grad_sqnorm) or several partial sums (GEMM epilogue slots, per-chunk norms of a
@@ -750,11 +803,17 @@ def compact_adam(master: torch.Tensor, exp_avg: torch.Tensor, exp_avg_sq: torch.
     _count()
     c_dt = dtype_id(compact_out.dtype) if compact_out is not None else _lib.BF16
     w_dt = dtype_id(w_dtype) if w_dtype is not None else _lib.BF16
+    head = (ptr(master), ptr(exp_avg), ptr(exp_avg_sq), ptr(grad), dtype_id(grad.dtype), grad.numel(), lr, beta1,
+            beta2, eps, weight_decay, bc1, bc2, grad_scale, ptr(sqnorm), n_sq, max_norm, ptr(compact_out), c_dt)
+    if columns is not None:
+        _req(columns.dtype == torch.uint8 and columns.numel() >= n_columns * C.sizeof(ColumnRef),
+             "columns: a make_column_table tensor with n_columns entries")
+        with _timed("compact_adam_columns", master.device, grad.numel()):
+            check(load().smt_compact_adam_columns(*head, ptr(columns), n_columns, w_dt, _st(master)),
+                  "smt_compact_adam_columns")
+        return
     with _timed("compact_adam", master.device, grad.numel()):
-        check(load().smt_compact_adam(ptr(master), ptr(exp_avg), ptr(exp_avg_sq), ptr(grad), dtype_id(grad.dtype),
-                                      grad.numel(), lr, beta1, beta2, eps, weight_decay, bc1, bc2, grad_scale,
-                                      ptr(sqnorm), n_sq, max_norm, ptr(compact_out), c_dt, ptr(table), n_blocks, block,
-                                      w_dt, _st(master)), "smt_compact_adam")
+        check(load().smt_compact_adam(*head, ptr(table), n_blocks, block, w_dt, _st(master)), "smt_compact_adam")
 
 
 
@@ -778,11 +837,12 @@ def _item_dtype():
 
 
 class _Problem:
-    __slots__ = ("x", "dy", "idx", "idx_id", "out", "block", "accumulate", "sq", "sq_slot0", "sink")
+    __slots__ = ("x", "dy", "idx", "idx_id", "out", "block", "accumulate", "sq", "sq_slot0", "sink", "ld_out")
 
-    def __init__(self, x, dy, idx, idx_id, out, block, accumulate, sq, sq_slot0, sink):
+    def __init__(self, x, dy, idx, idx_id, out, block, accumulate, sq, sq_slot0, sink, ld_out=0):
         self.x, self.dy, self.idx, self.idx_id, self.out, self.block = x, dy, idx, idx_id, out, block
         self.accumulate, self.sq, self.sq_slot0, self.sink = accumulate, sq, sq_slot0, sink
+        self.ld_out = ld_out          # 0: compact b x b tiles; > 0: tiles of a row-major matrix with this row pitch
 
 
 _idx_snap: dict = {}      # id(index_list) -> tuple snapshot (validated by value on every use)
@@ -807,8 +867,10 @@ class BlockGradBatch:
 
     add() keeps references to the operands; flush() encodes one TMA descriptor per distinct operand on the host,
     ships descriptors + per-block work items with a single pinned H2D copy and launches
-    `smt_block_grad_gemm_grouped`.  Problems must share T, the input dtype, the output dtype and the block size
-    (flush() launches one group per distinct combination).  The sorted / paired work-item array of a given set of
+    `smt_block_grad_gemm_grouped`.  Problems must share T, the input dtype, the output dtype, the block size and the
+    output row pitch (flush() launches one group per distinct combination).  Channel problems (`add_channel`) are the
+    tiles of `channel_grad_gemm`; their output pitch is the module's out_features, so each distinct width is a launch of
+    its own.  The sorted / paired work-item array of a given set of
     problems is cached, so steady-state steps only re-encode the (pointer-dependent) TMA descriptors."""
 
     def __init__(self):
@@ -841,6 +903,31 @@ class BlockGradBatch:
         self.problems.append(_Problem(x2d, dy2d, _snapshot_index_list(index_list), id(index_list), out, int(block),
                                       bool(accumulate), sq, int(sq_slot0), sink))
 
+    def add_channel(self, partial: torch.Tensor, dy2d: torch.Tensor, n: int, out: torch.Tensor, accumulate: bool = True,
+                    sq: Optional[torch.Tensor] = None, sq_slot0: int = -1, sink=None) -> None:
+        """The channel gradient `partial[:, :n]^T @ dy2d` (see channel_grad_gemm) into `out`, a contiguous
+        [ceil(n/b)*b, out_features] region whose rows past n receive zeros (b = channel_grad_block(n, out_features)).
+        Tile i of the row-major (row block, column block) order gets the sum-of-squares slots [sq_slot0 + 2 i, + 1]."""
+        require_cuda(partial, dy2d, out, sq)
+        _req(partial.dim() == 2 and dy2d.dim() == 2 and partial.shape[0] == dy2d.shape[0] and partial.dtype == dy2d.dtype
+             and partial.dtype in (torch.bfloat16, torch.float16),
+             "16-bit partial [T, n8] and dy [T, out_features] of one dtype")
+        _req(partial.stride(1) == 1 and dy2d.stride(1) == 1 and (partial.stride(0) * 2) % 16 == 0
+             and (dy2d.stride(0) * 2) % 16 == 0 and partial.data_ptr() % 16 == 0 and dy2d.data_ptr() % 16 == 0,
+             "unit column strides and 16-byte aligned rows")
+        out_f = dy2d.shape[1]
+        _req(0 < n <= partial.shape[1] and out_f % 64 == 0, "0 < n <= partial.shape[1] and out_features % 64 == 0")
+        block = channel_grad_block(n, out_f)
+        rows = (n + block - 1) // block
+        _req(out.is_contiguous() and out.shape == (rows * block, out_f) and out.dtype == dy2d.dtype,
+             "out: contiguous [ceil(n/b)*b, out_features] of dy's dtype")
+        if out.data_ptr() in self._out_ptrs:
+            self.flush()
+        self._out_ptrs.add(out.data_ptr())
+        # the packed channels are the `dy` operand, grad_output the `x` operand (see channel_grad_gemm)
+        self.problems.append(_Problem(dy2d, partial, _channel_tiles(rows, out_f // block), None, out, block,
+                                      bool(accumulate), sq, int(sq_slot0), sink, ld_out=out_f))
+
     def flush(self, accumulate: bool = True) -> int:
         """Launches everything collected so far; returns the number of grouped launches.  `last_flushed` keeps the
         problems of this flush (their sinks have been updated)."""
@@ -858,16 +945,16 @@ class BlockGradBatch:
             if len(pr.idx) == 0 or pr.x.shape[0] == 0:
                 continue
             key = (pr.x.shape[0], pr.x.dtype, pr.out.dtype, pr.block, pr.x.device,
-                   pr.sq.data_ptr() if pr.sq is not None else 0)
+                   pr.sq.data_ptr() if pr.sq is not None else 0, pr.ld_out)
             groups.setdefault(key, []).append(pr)
-        for (T, in_dt, out_dt, block, dev, _sq), prs in groups.items():
-            self._launch_group(T, in_dt, out_dt, block, dev, prs, accumulate)
+        for (T, in_dt, out_dt, block, dev, _sq, ld_out), prs in groups.items():
+            self._launch_group(T, in_dt, out_dt, block, dev, prs, accumulate, ld_out)
         HOST_TIME["flush_s"] += time.perf_counter() - t0
         HOST_TIME["flushes"] += 1
         self.last_flushed = problems
         return len(groups)
 
-    def _items_for(self, T, block, prs, maps_of, base_ptr, esize):
+    def _items_for(self, T, block, prs, maps_of, base_ptr, esize, ld_out=0):
         """Work-item array for this set of problems (cached: index lists, output offsets and the sharing pattern of
         the operands do not change from step to step).
         Work-item order = execution order (CTAs / CTA pairs are dispatched in item order):
@@ -877,7 +964,7 @@ class BlockGradBatch:
           * a module's unpaired blocks follow its pairs immediately (their strips are still in L2), not at the end of
             the launch; an odd one out is carried over to the next module to keep the even alignment."""
         import numpy as np
-        key = (T, block, tuple((pr.idx, (pr.out.data_ptr() - base_ptr) // esize, pr.accumulate,
+        key = (T, block, ld_out, tuple((pr.idx, (pr.out.data_ptr() - base_ptr) // esize, pr.accumulate,
                                 pr.sq_slot0 if pr.sq is not None else -1, mx, mdy)
                                for pr, (mx, mdy) in zip(prs, maps_of)))
         hit = self._plans.get(key)
@@ -887,7 +974,7 @@ class BlockGradBatch:
         for pr, (mx, mdy) in zip(prs, maps_of):
             off0 = (pr.out.data_ptr() - base_ptr) // esize
             flags = 0 if pr.accumulate else _lib.ITEM_OVERWRITE
-            entries = [(mdy, mx, r, c, off0 + i * block * block, flags,
+            entries = [(mdy, mx, r, c, off0 + (r * block * ld_out + c * block if ld_out else i * block * block), flags,
                         (pr.sq_slot0 + 2 * i) if (pr.sq is not None and pr.sq_slot0 >= 0) else -1)
                        for i, (r, c) in sorted(enumerate(pr.idx), key=lambda t: (t[1][0], t[1][1]))]
             pairs, singles, i = [], list(carry), 0
@@ -909,7 +996,7 @@ class BlockGradBatch:
         self._plans[key] = (arr, n_pairs)
         return arr, n_pairs
 
-    def _launch_group(self, T, in_dt, out_dt, block, dev, prs, accumulate) -> None:
+    def _launch_group(self, T, in_dt, out_dt, block, dev, prs, accumulate, ld_out=0) -> None:
         lib = load()
         maps: dict = {}
 
@@ -922,7 +1009,7 @@ class BlockGradBatch:
         esize = prs[0].out.element_size()
         base_ptr = min(pr.out.data_ptr() for pr in prs)
         maps_of = [(map_index(pr.x), map_index(pr.dy)) for pr in prs]
-        arr, n_pairs = self._items_for(T, block, prs, maps_of, base_ptr, esize)
+        arr, n_pairs = self._items_for(T, block, prs, maps_of, base_ptr, esize, ld_out)
         n_items, n_maps = len(arr), len(maps)
         sq = prs[0].sq
         emits = bool(sq is not None and lib.smt_block_grad_gemm_grouped_emits_sq(n_items, block, T))
@@ -943,7 +1030,7 @@ class BlockGradBatch:
         with _timed("block_grad_gemm", dev, (n_items, block, T)):
             check(lib.smt_block_grad_gemm_grouped(dev_buf.data_ptr(), dev_buf.data_ptr() + n_maps * 128, n_items,
                                                   T, block, in_id, base_ptr, dtype_id(out_dt), 1 if accumulate else 0,
-                                                  0, ptr(sq) if emits else 0, ptr(ws), ws_bytes, stream_ptr(dev)),
+                                                  ld_out, ptr(sq) if emits else 0, ptr(ws), ws_bytes, stream_ptr(dev)),
                   "smt_block_grad_gemm_grouped")
         _count(lib.smt_last_launch_count())
         for pr in prs:

@@ -20,7 +20,10 @@ fp32 masters, rounding to the parameter dtype into `flat_param`, and the write-b
 its dense weight matrix.
 
 Gradient delivery protocol (`GradSink`).  Every `selected_weight` of an arena owns a `GradSink`: the view of
-`flat_grad` that `linearZ.backward` writes into, plus three host-side flags.  `zero_grad()` is LAZY for those
+`flat_grad` that `linearZ.backward` writes into, plus three host-side flags.  bf16 channel layers
+(`LinearLayer_ChannelSparsity`) take part the same way: `linearChannel.backward` delivers into the arena, whose region for
+such a parameter has the padding rows of the gradient launch's last row tile, and one `smt_compact_adam_columns` launch
+writes the updated channels into their weight columns.  `zero_grad()` is LAZY for those
 parameters: it only sets `sink.overwrite`, and the first block-gradient GEMM that delivers afterwards overwrites the
 view instead of accumulating (per-work-item flag) - the 114 MB memset and the read-modify-write of the GEMM epilogue
 disappear from the step.  Further backward passes before the next `step()` accumulate (gradient accumulation).  The
@@ -42,17 +45,48 @@ from ._lib import SMTLibraryError
 
 
 def _owner_of(p):
+    """The SMT layer whose dense weight SMTAdam writes `p` back into, or None.  An owner provides (smt/smt.py):
+    `_arena_layout()` -> (elements the arena reserves, sum-of-squares slots), `_writeback(offset)` -> (key, table
+    entries), `_writeback_args(key, entries, device)` -> ops.compact_adam keyword arguments, `mark_synced()` and
+    `sync_weight(force)`."""
     ref = getattr(p, "_smt_owner", None)
-    return ref() if ref is not None else None
+    owner = ref() if ref is not None else None
+    return owner if owner is not None and owner._arena_ok() else None
+
+
+def _writeback_args(owners_offs, device):
+    """ops.compact_adam keyword arguments of ONE launch that writes back the parameters [(owner, arena offset)], or
+    None when they need different kinds of table (blocks of another size or dtype, columns)."""
+    key, entries = None, []
+    for owner, off in owners_offs:
+        k, e = owner._writeback(off)
+        if key is not None and k != key:
+            return None
+        key = k
+        entries += e
+    return type(owners_offs[0][0])._writeback_args(key, entries, device)
+
+
+def _cached_writeback_args(cache: dict, slot, owners_offs, device):
+    """`_writeback_args`, rebuilt only when a dense weight's storage moved."""
+    wkey = tuple((o.weight.data_ptr(), o.weight.stride(0)) for o, _ in owners_offs)
+    hit = cache.get(slot)
+    if hit is None or hit[0] != wkey:
+        hit = (wkey, _writeback_args(owners_offs, device))
+        cache[slot] = hit
+    return hit[1]
 
 
 class GradSink:
-    """Where `linearZ.backward` delivers the block gradients of one `selected_weight` in native mode."""
-    __slots__ = ("view", "sq", "sq_slot0", "overwrite", "touched", "sq_ok", "__weakref__")
+    """Where `linearZ.backward` / `linearChannel.backward` deliver the gradient of one `selected_weight` in native
+    mode."""
+    __slots__ = ("view", "store", "sq", "sq_slot0", "overwrite", "touched", "sq_ok", "__weakref__")
 
-    def __init__(self, view: torch.Tensor, sq: Optional[torch.Tensor], sq_slot0: int):
-        self.view = view              # [n*b, b] view of the arena's flat_grad
-        self.sq = sq                  # the arena's per-block sum-of-squares slots (2 per block) or None
+    def __init__(self, view: torch.Tensor, sq: Optional[torch.Tensor], sq_slot0: int, store: Optional[torch.Tensor] = None):
+        self.view = view              # the parameter's .grad: a view of the arena's flat_grad
+        self.store = view if store is None else store   # what the GEMM writes: `view` plus the padding rows of a
+                                                        # channel parameter ([ceil(n/b)*b, out_features])
+        self.sq = sq                  # the arena's per-tile sum-of-squares slots (2 per block / channel tile) or None
         self.sq_slot0 = sq_slot0
         self.overwrite = False        # the next delivery replaces the contents (lazy zero_grad)
         self.touched = False          # a gradient was delivered since the last zero_grad
@@ -80,28 +114,31 @@ class _Arena:
         self.params = params
         self.device = first.device
         self.dtype = first.dtype
-        offs, total = [], 0
+        offs, sizes, slots, total = [], [], [], 0
         for p in params:
             if p.device != self.device or p.dtype != self.dtype:
                 raise SMTLibraryError("SMTAdam: all parameters of a group must share device and dtype")
+            owner = _owner_of(p)
+            size, n_sq = owner._arena_layout() if owner is not None else (p.numel(), 0)
             offs.append(total)
-            total += (p.numel() + 7) // 8 * 8              # kernels work on 8-element vectors
-        self.offsets, self.total = offs, total
+            sizes.append((size + 7) // 8 * 8)               # kernels work on 8-element vectors
+            slots.append(n_sq)
+            total += sizes[-1]
+        self.offsets, self.sizes, self.sq_counts, self.total = offs, sizes, slots, total
         self.flat_param = torch.zeros(total, dtype=self.dtype, device=self.device)
         self.flat_grad = torch.zeros(total, dtype=self.dtype, device=self.device)
         self.master = torch.zeros(total, dtype=torch.float32, device=self.device)
         self.exp_avg = torch.zeros(total, dtype=torch.float32, device=self.device)
         self.exp_avg_sq = torch.zeros(total, dtype=torch.float32, device=self.device)
         self.sqnorm = torch.zeros(1, dtype=torch.float32, device=self.device)
-        # two sum-of-squares slots per selected block (written by the block-gradient GEMM epilogue)
-        n_slots = sum(2 * len(_owner_of(p).index_list) for p in params if _owner_of(p) is not None)
-        self.block_sq = torch.zeros(max(n_slots, 1), dtype=torch.float32, device=self.device)
+        # two sum-of-squares slots per selected block / channel tile (written by the gradient GEMM epilogue)
+        self.block_sq = torch.zeros(max(sum(slots), 1), dtype=torch.float32, device=self.device)
         self.sq_dirty = True                                # the buffer was modified by something else (all-reduce, copy)
         self.sq_override: Optional[torch.Tensor] = None     # partial sums supplied by a data-parallel exchange
         self.sinks: List[Optional[GradSink]] = []
         self.grad_views: List[torch.Tensor] = []
         slot = 0
-        for p, off in zip(params, offs):
+        for p, off, size, n_sq in zip(params, offs, sizes, slots):
             n = p.numel()
             view = self.flat_param[off:off + n].view(p.shape)
             view.copy_(p.data)
@@ -112,32 +149,30 @@ class _Arena:
                 g.copy_(p.grad)
             p.grad = g
             self.grad_views.append(g)
-            owner = _owner_of(p)
-            if owner is not None:
-                sink = GradSink(g, self.block_sq, slot)
-                slot += 2 * len(owner.index_list)
-                p._smt_sink = sink                          # linearZ.backward delivers here directly
+            if _owner_of(p) is not None:
+                store = self.flat_grad[off:off + size].view(-1, *p.shape[1:]) if size != n else g
+                sink = GradSink(g, self.block_sq, slot, store)
+                slot += n_sq
+                p._smt_sink = sink                          # linearZ / linearChannel.backward deliver here directly
                 self.sinks.append(sink)
             else:
                 self.sinks.append(None)
         self.all_sinks = all(sk is not None for sk in self.sinks)
-        self._table = None
-        self._table_key = None
+        self._writeback_cache: dict = {}
 
     def reconcile_grads(self) -> None:
         """Before a step: every parameter's gradient must be what the arena holds.
         * sink parameters that received nothing since zero_grad(): their slice (and slots) become zero;
         * parameters without a sink (e.g. layer norms in mixture mode) whose `.grad` is no longer the arena view
           (autograd created a fresh tensor after `set_to_none`): copied in and re-attached; None -> zeros."""
-        for p, view, sink in zip(self.params, self.grad_views, self.sinks):
+        for p, view, sink, n_slots in zip(self.params, self.grad_views, self.sinks, self.sq_counts):
             if sink is not None:
                 if p.grad is None or p.grad.data_ptr() != view.data_ptr():
                     if not sink.touched:                    # dropped and never delivered again: no gradient this step
                         sink.overwrite = True
                     p.grad = view
                 if sink.overwrite:                          # nothing was delivered since the (lazy) zero_grad
-                    view.zero_()
-                    n_slots = 2 * (view.numel() // (_owner_of(p).block ** 2))
+                    view.zero_()                            # (padding rows of a channel parameter only ever hold zeros)
                     self.block_sq[sink.sq_slot0:sink.sq_slot0 + n_slots].zero_()
                     sink.overwrite = False
                     sink.sq_ok = True
@@ -159,24 +194,21 @@ class _Arena:
             return None
         return self.block_sq
 
-    def fused_table(self):
-        """One block table covering the whole arena, or None when the group is not purely SMT blocks of one
-        block size / weight dtype (then the step falls back to per-parameter launches)."""
+    def fused_writeback(self):
+        """ops.compact_adam write-back arguments of ONE launch over the whole arena, or None when the group is not
+        purely SMT parameters with one kind of table (blocks of one size and weight dtype, or channels of one weight
+        dtype); the step then falls back to per-parameter launches."""
         owners = [_owner_of(p) for p in self.params]
         if any(o is None for o in owners):
             return None
-        blocks = {o.block for o in owners}
-        wdt = {o.weight.dtype for o in owners}
-        if len(blocks) != 1 or len(wdt) != 1:
+        return _cached_writeback_args(self._writeback_cache, "all", list(zip(owners, self.offsets)), self.device)
+
+    def writeback(self, i: int):
+        """ops.compact_adam write-back arguments of parameter i alone (offsets relative to its slice), or None."""
+        owner = _owner_of(self.params[i])
+        if owner is None:
             return None
-        key = tuple((o.weight.data_ptr(), o.weight.stride(0)) for o in owners)
-        if self._table is None or self._table_key != key:
-            entries = []
-            for o in owners:
-                entries += [(o.weight.data, r, c) for r, c in o.index_list]
-            self._table = (ops.make_block_table(entries, self.device), len(entries), blocks.pop(), wdt.pop())
-            self._table_key = key
-        return self._table
+        return _cached_writeback_args(self._writeback_cache, i, [(owner, 0)], self.device)
 
 
 class SMTAdam(torch.optim.Optimizer):
@@ -193,6 +225,7 @@ class SMTAdam(torch.optim.Optimizer):
         self.grad_scale = float(grad_scale)                # e.g. 1/world_size after a SUM all-reduce
         self.steps_done = 0                                # serial number of the gradient state (bumped by every step())
         self.flatten = bool(flatten)
+        self._loose_writeback: dict = {}                   # flatten=False: write-back tables per parameter
         self._arenas: List[Optional[_Arena]] = []
         for group in self.param_groups:
             group.setdefault("step", 0)
@@ -364,27 +397,20 @@ class SMTAdam(torch.optim.Optimizer):
         return loss
 
     def _step_arena(self, arena: _Arena, common) -> None:
-        fused = arena.fused_table()
+        fused = arena.fused_writeback()
         if fused is not None:
-            table, n_blocks, block, w_dtype = fused
             ops.compact_adam(arena.master, arena.exp_avg, arena.exp_avg_sq, arena.flat_grad,
-                             compact_out=arena.flat_param, table=table, n_blocks=n_blocks, block=block,
-                             w_dtype=w_dtype, **common)
+                             compact_out=arena.flat_param, **fused, **common)
             for p in arena.params:
                 _owner_of(p).mark_synced()
             return
-        for p, off in zip(arena.params, arena.offsets):
-            n = (p.numel() + 7) // 8 * 8
+        for i, (p, off, n) in enumerate(zip(arena.params, arena.offsets, arena.sizes)):
             sl = slice(off, off + n)
-            owner = _owner_of(p)
-            kw = dict(common)
-            if owner is not None and len(owner.index_list) * owner.block * owner.block == n:
-                kw.update(table=owner._block_table(), n_blocks=len(owner.index_list), block=owner.block,
-                          w_dtype=owner.weight.dtype)
+            wb = arena.writeback(i)
             ops.compact_adam(arena.master[sl], arena.exp_avg[sl], arena.exp_avg_sq[sl], arena.flat_grad[sl],
-                             compact_out=arena.flat_param[sl], **kw)
-            if owner is not None and "table" in kw:
-                owner.mark_synced()
+                             compact_out=arena.flat_param[sl], **(wb or {}), **common)
+            if wb is not None:
+                _owner_of(p).mark_synced()
             else:
                 torch.autograd.graph.increment_version(p)   # forward() must re-scatter / autograd must notice
 
@@ -408,8 +434,7 @@ class SMTAdam(torch.optim.Optimizer):
         owner = _owner_of(p)
         kw = dict(common)
         if owner is not None:
-            kw.update(table=owner._block_table(), n_blocks=len(owner.index_list), block=owner.block,
-                      w_dtype=owner.weight.dtype)
+            kw.update(_cached_writeback_args(self._loose_writeback, id(p), [(owner, 0)], p.device))
         ops.compact_adam(master, st["exp_avg"].reshape(-1), st["exp_avg_sq"].reshape(-1), g, compact_out=out, **kw)
         if owner is not None:
             owner.mark_synced()

@@ -112,7 +112,8 @@ def _block_rc_for(index_list, device) -> torch.Tensor:
 # ---- deferred, grouped block-gradient launches (native mode only) ------------------------------------------------
 #
 # With a gradient sink (SMTAdam's flat buffer) nothing has to be RETURNED by linearZ.backward, so the contraction can
-# be postponed: every module's backward only enqueues its (x, dy, blocks, sink) problem and ONE grouped tcgen05
+# be postponed: every module's backward only enqueues its (x, dy, blocks, sink) problem (linearChannel: its
+# (partial, dy, n, sink) problem, whose tiles are stored with the row pitch out_features) and ONE grouped tcgen05
 # launch runs when the autograd engine finishes the backward pass (a queue_callback), i.e. before
 # `loss.backward()` returns.  Per-module launches of ~9-30 blocks cannot fill 148 SMs; the grouped launch of all
 # 869 blocks can.  `flush_block_grads()` is also called by SMTAdam.step() / dp.allreduce_compact_grads as a guard.
@@ -173,19 +174,25 @@ def flush_block_grads() -> int:
         return _flush_locked()
 
 
-def _enqueue_block_grad(x2, dy2, index_list, sink, block, accumulate) -> None:
+def _enqueue(xkey, device, add) -> None:
+    """Queue one module's gradient problem (`add()` puts it into `_pending`); `xkey` identifies the module's input, so
+    that a chunked flush happens at a layer boundary."""
     with _pending_lock:
         chunk = _grouped["chunk_blocks"]
-        xkey = (x2.data_ptr(), x2.shape[0])
         if chunk > 0 and _pending_state["last_x"] not in (None, xkey) and _pending.n_blocks() >= chunk:
             _flush_locked()                                     # layer boundary with a GPU-filling chunk pending
         _pending_state["last_x"] = xkey
-        _pending.add(x2, dy2, index_list, sink.view, block, accumulate=accumulate, sq=sink.sq, sq_slot0=sink.sq_slot0,
-                     sink=sink)
-        _pending_state["stream"] = torch.cuda.current_stream(x2.device)
+        add()
+        _pending_state["stream"] = torch.cuda.current_stream(device)
         if not _pending_state["callback_queued"]:
             _pending_state["callback_queued"] = True
             torch.autograd.Variable._execution_engine.queue_callback(flush_block_grads)
+
+
+def _enqueue_block_grad(x2, dy2, index_list, sink, block, accumulate) -> None:
+    _enqueue((x2.data_ptr(), x2.shape[0]), x2.device,
+             lambda: _pending.add(x2, dy2, index_list, sink.view, block, accumulate=accumulate, sq=sink.sq,
+                                  sq_slot0=sink.sq_slot0, sink=sink))
 
 
 class linearZ(torch.autograd.Function):
@@ -291,6 +298,24 @@ class LinearLayer_MatrixSparsity(nn.Module):
         self._synced = None
         return out
 
+    # -- what SMTAdam's arena (optim._Arena) asks of the layer that owns a parameter --
+    def _arena_ok(self) -> bool:
+        return True
+
+    def _arena_layout(self):
+        """(elements the arena reserves for selected_weight, sum-of-squares slots its gradient launches fill)"""
+        n = len(self.index_list)
+        return n * self.block * self.block, 2 * n
+
+    def _writeback(self, off: int):
+        """(key, entries) of the dense write-back of selected_weight stored at arena offset `off`: owners with equal keys
+        share one fused Adam launch, whose table `_writeback_args` builds from their concatenated entries."""
+        return ("blocks", self.block, self.weight.dtype), [(self.weight.data, r, c) for r, c in self.index_list]
+
+    @staticmethod
+    def _writeback_args(key, entries, device) -> dict:
+        return dict(table=ops.make_block_table(entries, device), n_blocks=len(entries), block=key[1], w_dtype=key[2])
+
     def mark_synced(self) -> None:
         """Called by the fused optimizer (SMTAdam) right after it has written the updated blocks into `weight`
         itself.  The mark is tied to the parameter's storage pointer and version counter: re-pointing `.data`
@@ -325,14 +350,16 @@ class LinearLayer_MatrixSparsity(nn.Module):
 # results autograd adds with two elementwise kernels.  `fuse_qkv_projections(model)` ties the three modules of every
 # layer into a group: the first call (q_proj) runs ONE hand-written tcgen05 GEMM over [Wq; Wk; Wv] and hands k_proj /
 # v_proj their slices when they are called with the same tensor; backward runs ONE GEMM over K = 4096 + 1024 + 1024
-# for the input gradient and feeds the block-gradient path of each sparse member.  Module names, parameters and
-# state dicts are untouched (the override is a method bound to the instance); members may be LinearLayer_MatrixSparsity
-# or frozen, bias-free nn.Linear.  Anything the kernel does not support falls back to the members' own forward.
+# for the input gradient and feeds the weight-gradient path of each sparse member.  Module names, parameters and
+# state dicts are untouched (the override is a method bound to the instance); members may be LinearLayer_MatrixSparsity,
+# bf16 LinearLayer_ChannelSparsity or frozen, bias-free nn.Linear.  Anything the kernel does not support falls back to
+# the members' own forward.
 # The same call also moves the layer's elementwise ops (norms, residual add, RoPE, SwiGLU) onto native kernels
 # (decoder_fusion.py).
 
 class fusedLinearZ(torch.autograd.Function):
-    """forward(ctx, input, group, *selected_weights of the sparse members) -> one output per member."""
+    """forward(ctx, input, group, *selected_weights of the sparse members) -> one output per member.
+    Block members keep `input` for their gradient; channel members keep only their packed input channels (linearChannel)."""
 
     @staticmethod
     def forward(ctx, input, group, *selected_weights):
@@ -341,25 +368,41 @@ class fusedLinearZ(torch.autograd.Function):
         ys = ops.fused_linear_forward(x2, [w.data for w in weights])
         ctx.group = group
         ctx.block = Block_dimension
-        ctx.save_for_backward(input, *weights)
+        ctx.x_shape = input.shape
+        ctx.xkey = (x2.data_ptr(), x2.shape[0])
+        partials = []
+        sparse = [m for m in group.members if isinstance(m, _SPARSE_LAYERS)]
+        for k, m in enumerate(sparse):
+            if isinstance(m, LinearLayer_ChannelSparsity):
+                partials.append(ops.channel_gather(x2, _channel_idx_for(m.index_list, x2.device, 8))
+                                if ctx.needs_input_grad[2 + k] and len(m.index_list) else None)   # smt.py:240-247
+        keep_x = any(isinstance(m, LinearLayer_MatrixSparsity) for m in sparse)
+        ctx.n_partials = len(partials)
+        ctx.save_for_backward(input if keep_x else None, *partials, *weights)
         lead = input.shape[:-1]
         return tuple(y.view(*lead, y.shape[-1]) for y in ys)
 
     @staticmethod
     def backward(ctx, *grad_outputs):
-        x, *weights = ctx.saved_tensors
+        x, *saved = ctx.saved_tensors
+        partials, weights = saved[:ctx.n_partials], saved[ctx.n_partials:]
         members = ctx.group.members
         dys = [_as_operand(g.reshape(-1, g.shape[-1])) for g in grad_outputs]
         grad_input = None
         if ctx.needs_input_grad[0]:
-            grad_input = ops.fused_linear_dgrad(dys, [w.data for w in weights]).view(x.shape)   # smt.py:406, all members
-        grads, k = [], 0
+            grad_input = ops.fused_linear_dgrad(dys, [w.data for w in weights]).view(ctx.x_shape)   # smt.py:406, all members
+        grads, k, j = [], 0, 0
         x2 = None
         for m, dy2 in zip(members, dys):
-            if not isinstance(m, LinearLayer_MatrixSparsity):
+            if not isinstance(m, _SPARSE_LAYERS):
                 continue
             g = None
-            if ctx.needs_input_grad[2 + k]:
+            if isinstance(m, LinearLayer_ChannelSparsity):
+                partial = partials[j]
+                j += 1
+                if ctx.needs_input_grad[2 + k]:
+                    g = _channel_weight_grad(m.selected_weight, partial, len(m.index_list), dy2, ctx.xkey)
+            elif ctx.needs_input_grad[2 + k]:
                 if x2 is None:
                     x2 = _as_operand(x.reshape(-1, x.shape[-1]))
                 g = _block_weight_grad(m.selected_weight, m.index_list, x2, dy2, ctx.block, dy2.dtype)
@@ -397,9 +440,9 @@ class _SharedInputGroup:
                 self._cache = None
             return y
         if role == 0 and self._supported(x):
-            sparse = [m for m in self.members if isinstance(m, LinearLayer_MatrixSparsity)]
+            sparse = [m for m in self.members if isinstance(m, _SPARSE_LAYERS)]
             for m in sparse:
-                m.sync_weight()                                        # smt.py:332-341, unless SMTAdam vouches
+                m.sync_weight()                         # smt.py:332-341 / 208-211, unless SMTAdam vouches
             outs = list(fusedLinearZ.apply(x, self, *[m.selected_weight for m in sparse]))
             y, outs[0] = outs[0], None
             self._cache = (x, outs)
@@ -410,6 +453,8 @@ class _SharedInputGroup:
 def _fusable_member(m) -> bool:
     if isinstance(m, LinearLayer_MatrixSparsity):
         return True
+    if isinstance(m, LinearLayer_ChannelSparsity):
+        return m.weight.dtype == torch.bfloat16 and m.selected_weight.dtype == torch.bfloat16
     return isinstance(m, nn.Linear) and m.bias is None and not m.weight.requires_grad
 
 
@@ -422,8 +467,9 @@ def fuse_qkv_projections(model) -> int:
     one fused dense GEMM per direction (see above), and in a LLaMA decoder layer whose projections were fused the
     elementwise ops around them - the two RMSNorms with the residual add, RoPE and SwiGLU - run on the native kernels of
     `decoder_fusion` (the model's final norm too).  Returns the number of layers whose projections were fused.  Call
-    after `convert_linear_layer_to_matrix_sparsity`; undone by `unfuse_qkv_projections` (and automatically by
-    `convert_matrix_sparsity_to_linear_layer`).  The overrides are methods bound to each module, so a `copy.deepcopy`
+    after `convert_linear_layer_to_matrix_sparsity` / `convert_linear_layer_to_channel_sparsity`; undone by
+    `unfuse_qkv_projections` (and automatically by `convert_matrix_sparsity_to_linear_layer` /
+    `convert_channel_sparsity_to_linear_layer`).  The overrides are methods bound to each module, so a `copy.deepcopy`
     of the model computes with the copy's weights."""
     fused = 0
     for parent in model.modules():
@@ -661,6 +707,8 @@ class linearChannel(torch.autograd.Function):
         pad = 64 if x2.dtype == torch.float32 else 8
         partial = ops.channel_gather(x2, _channel_idx_for(channel_index_list, x2.device, pad))
         ctx.n_channels = len(channel_index_list)
+        ctx.sw_ref = selected_weight                      # only for the optional gradient sink (no data use)
+        ctx.xkey = (x2.data_ptr(), x2.shape[0])
         ctx.save_for_backward(partial, weight)
         return torch.matmul(input, weight.t())            # smt.py:257
 
@@ -669,24 +717,41 @@ class linearChannel(torch.autograd.Function):
         partial, weight = ctx.saved_tensors
         grad_input = grad_weight = None
         if ctx.needs_input_grad[1]:
-            n = ctx.n_channels
             dy2 = grad_output.reshape(-1, grad_output.shape[-1])
             if dy2.stride(-1) != 1 or (dy2.stride(0) * dy2.element_size()) % 16 != 0:
                 dy2 = dy2.contiguous()
-            if partial.dtype != dy2.dtype:
-                partial = partial.to(dy2.dtype)
-            out_f = dy2.shape[1]
-            # smt.py:283-284: sum over the batch of partial^T @ dy == ONE contraction over all tokens, on the same
-            # tcgen05 pipeline as the block gradients (fp32 accumulation, one rounding)
-            if n == 0:
-                grad_weight = torch.zeros(0, out_f, dtype=dy2.dtype, device=dy2.device)
-            elif dy2.dtype == torch.float32 or out_f % 64 != 0:
-                grad_weight = _channel_grad_by_blocks(partial, n, dy2)
-            else:
-                grad_weight = ops.channel_grad_gemm(partial, n, dy2)
+            grad_weight = _channel_weight_grad(ctx.sw_ref, partial, ctx.n_channels, dy2, ctx.xkey)
         if ctx.needs_input_grad[0]:
             grad_input = torch.matmul(grad_output, weight)                                      # smt.py:286
         return grad_input, grad_weight, None, None
+
+
+def _channel_weight_grad(sw_param, partial, n, dy2, xkey):
+    """The channel gradient of one module (smt.py:283-284).  Native mode (the parameter owns a GradSink): delivered
+    into the padded arena region of the parameter - grouped with the other modules of the backward pass when grouping
+    is enabled - and None is returned; otherwise the [n, out_features] gradient is returned.  `xkey` identifies the
+    module's input (chunked flushes happen at layer boundaries)."""
+    if partial.dtype != dy2.dtype:
+        partial = partial.to(dy2.dtype)
+    sink = getattr(sw_param, "_smt_sink", None)
+    if sink is not None:
+        dy2 = _as_operand(dy2)
+        accumulate = sink.begin_delivery(sw_param)
+        if _grouped["enabled"]:
+            _enqueue(xkey, dy2.device, lambda: _pending.add_channel(partial, dy2, n, sink.store, accumulate=accumulate,
+                                                                    sq=sink.sq, sq_slot0=sink.sq_slot0, sink=sink))
+        else:
+            ops.channel_grad_gemm(partial, n, dy2, out=sink.store, accumulate=accumulate)
+            sink.sq_ok = False
+        return None
+    out_f = dy2.shape[1]
+    # smt.py:283-284: sum over the batch of partial^T @ dy == ONE contraction over all tokens, on the same tcgen05
+    # pipeline as the block gradients (fp32 accumulation, one rounding)
+    if n == 0:
+        return torch.zeros(0, out_f, dtype=dy2.dtype, device=dy2.device)
+    if dy2.dtype == torch.float32 or out_f % 64 != 0:
+        return _channel_grad_by_blocks(partial, n, dy2)
+    return ops.channel_grad_gemm(partial, n, dy2)
 
 
 def _channel_grad_by_blocks(partial, n, dy2):
@@ -733,11 +798,58 @@ class LinearLayer_ChannelSparsity(nn.Module):
         if n:
             ops.column_gather(weight.data, _channel_idx_for(index_list, weight.device), compact)
         self.selected_weight = nn.Parameter(compact, requires_grad=True)
+        self.selected_weight._smt_owner = weakref.ref(self)   # lets SMTAdam find the dense weight to write back
         self.fn = linearChannel.apply
+        # Set ONLY by `mark_synced()` (SMTAdam after its fused column write-back); see LinearLayer_MatrixSparsity.
+        self._synced = None
+
+    def _apply(self, fn, *args, **kwargs):
+        out = super()._apply(fn, *args, **kwargs)
+        self._synced = None
+        return out
+
+    # -- what SMTAdam's arena (optim._Arena) asks of the layer that owns a parameter (see LinearLayer_MatrixSparsity) --
+    def _arena_ok(self) -> bool:
+        """bf16 layers with selected channels and out_features % 64 == 0 take the native path (gradients delivered into
+        the arena, fused column write-back); any other channel layer is an ordinary arena parameter, as before."""
+        w = self.weight
+        return len(self.index_list) > 0 and w.dtype == torch.bfloat16 and self.selected_weight.dtype == w.dtype \
+            and w.shape[0] % 64 == 0
+
+    def _grad_tiles(self):
+        """(b, row tiles, column tiles) of this layer's channel-gradient launches (ops.channel_grad_gemm)."""
+        n, out_f = len(self.index_list), self.weight.shape[0]
+        b = ops.channel_grad_block(n, out_f)
+        return b, (n + b - 1) // b, out_f // b
+
+    def _arena_layout(self):
+        """The last row tile of the gradient launch stores ceil(n/b)*b rows (the rows past n are zero), so the arena
+        reserves them: selected_weight and its .grad are the first n rows of the region."""
+        b, rows, cols = self._grad_tiles()
+        return rows * b * self.weight.shape[0], 2 * rows * cols
+
+    def _writeback(self, off: int):
+        w = self.weight.data
+        out_f = w.shape[0]
+        return ("columns", w.dtype), [(w, int(c), off + i * out_f) for i, c in enumerate(self.index_list)]
+
+    @staticmethod
+    def _writeback_args(key, entries, device) -> dict:
+        return dict(columns=ops.make_column_table(entries, device), n_columns=len(entries), w_dtype=key[1])
+
+    def mark_synced(self) -> None:
+        """Called by SMTAdam right after it has written the updated channels into the columns of `weight` itself; the
+        same rule as LinearLayer_MatrixSparsity.mark_synced (storage pointer + version counter of selected_weight)."""
+        self._synced = (self.selected_weight.data_ptr(), self.selected_weight._version)
 
     def sync_weight(self, force: bool = False) -> None:
-        """compact -> dense write-back (smt.py:208-211): one launch on EVERY forward, like the reference's loop —
-        whatever optimizer updated `selected_weight` (also through `.data` or an aliased flat buffer) is seen."""
+        """compact -> dense write-back (smt.py:208-211): one launch on every forward, like the reference's loop —
+        whatever optimizer updated `selected_weight` (also through `.data` or an aliased flat buffer) is seen.  The only
+        exception is right after an SMTAdam step that wrote the columns itself (see `mark_synced`)."""
+        if not force and self._synced is not None and \
+                self._synced == (self.selected_weight.data_ptr(), self.selected_weight._version):
+            return
+        self._synced = None
         if len(self.index_list):
             sw = self.selected_weight.data
             if sw.dtype != self.weight.dtype:
@@ -748,6 +860,9 @@ class LinearLayer_ChannelSparsity(nn.Module):
     def forward(self, x):
         self.sync_weight()
         return self.fn(x, self.selected_weight, self.index_list, self.weight)   # smt.py:213
+
+
+_SPARSE_LAYERS = (LinearLayer_MatrixSparsity, LinearLayer_ChannelSparsity)
 
 
 def convert_linear_layer_to_channel_sparsity(model,
@@ -776,6 +891,7 @@ def convert_linear_layer_to_channel_sparsity(model,
 def convert_channel_sparsity_to_linear_layer(model, part_module_name=['.layers']):
     """Write the trained channels back and restore plain nn.Linear modules (the channel twin of smt.py:416-457; the
     reference has no such function for channels)."""
+    unfuse_qkv_projections(model)
     names = [name for name, module in model.named_modules()
              if isinstance(module, LinearLayer_ChannelSparsity) and any(part in name for part in part_module_name)]
     for name in names:
