@@ -281,6 +281,23 @@ SMT_API int smt_rope_forward(const void* q, const void* k, const void* cos_, con
                              int Hk, int64_t cs_bstride, void* q_out, void* k_out, void* stream);
 SMT_API int smt_rope_backward(const void* dq_out, const void* dk_out, const void* cos_, const void* sin_, int B, int S,
                               int Hq, int Hk, int64_t cs_bstride, void* dq, void* dk, void* stream);
+/* Per-head RMSNorm of q and k followed by the rotary embedding above, in one launch: transformers' Qwen3Attention
+ * `q_norm` / `k_norm` (Qwen3RMSNorm over head_dim 128) + apply_rotary_pos_emb.  q [B, S, Hq, 128], k [B, S, Hk, 128]
+ * and the outputs in the projections' layout; wq / wk: the frozen norm weights [128]; cos / sin as for smt_rope_*.
+ *   forward   rstd = rsqrt(mean(x^2) + eps)  (fp32, one per head row: rstd_q [B*S*Hq], rstd_k [B*S*Hk])
+ *             y = bf16(w * bf16(x * rstd)),  out = smt_rope_forward(y)
+ *   backward  dy = smt_rope_backward(dq_out) (bf16),  g = dy * w,  xhat = x * rstd,
+ *             dx = bf16(rstd * (g - xhat * mean(g * xhat)))      (input gradient only: the weights are frozen)
+ * Each row's sum is reduced in a fixed order, so a recomputed forward reproduces the first one bit for bit.
+ * rstd: 4-byte aligned; every other tensor 16-byte aligned. */
+SMT_API int smt_qk_norm_rope_forward(const void* q, const void* k, const void* wq, const void* wk, float eps_q,
+                                     float eps_k, const void* cos_, const void* sin_, int B, int S, int Hq, int Hk,
+                                     int64_t cs_bstride, void* q_out, void* k_out, float* rstd_q, float* rstd_k,
+                                     void* stream);
+SMT_API int smt_qk_norm_rope_backward(const void* q, const void* k, const void* wq, const void* wk,
+                                      const float* rstd_q, const float* rstd_k, const void* cos_, const void* sin_,
+                                      const void* dq_out, const void* dk_out, int B, int S, int Hq, int Hk,
+                                      int64_t cs_bstride, void* dq, void* dk, void* stream);
 /* SwiGLU over n elements (n % 8 == 0):
  *   forward   h  = bf16(bf16(silu(g)) * u)
  *   backward  du = bf16(dh * bf16(silu(g))),  dg = bf16(silu'(g) * bf16(dh * u))   (torch's silu_backward formula) */

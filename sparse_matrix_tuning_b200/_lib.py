@@ -94,6 +94,10 @@ _SIGNATURES = {
     "smt_rmsnorm_backward": (C.c_int, [_P, _P, _P, _P, _P, C.c_int64, C.c_int, _P, _P]),
     "smt_rope_forward": (C.c_int, [_P, _P, _P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int64, _P, _P, _P]),
     "smt_rope_backward": (C.c_int, [_P, _P, _P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int64, _P, _P, _P]),
+    "smt_qk_norm_rope_forward": (C.c_int, [_P, _P, _P, _P, C.c_float, C.c_float, _P, _P, C.c_int, C.c_int, C.c_int,
+                                           C.c_int, C.c_int64, _P, _P, _P, _P, _P]),
+    "smt_qk_norm_rope_backward": (C.c_int, [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P, C.c_int, C.c_int, C.c_int,
+                                            C.c_int, C.c_int64, _P, _P, _P]),
     "smt_swiglu_forward": (C.c_int, [_P, _P, C.c_int64, _P, _P]),
     "smt_swiglu_backward": (C.c_int, [_P, _P, _P, C.c_int64, _P, _P, _P]),
     "smt_cross_entropy_rows": (C.c_int, [_P, C.c_int64, C.c_int64, C.c_int, _P, C.c_int64, _P, _P, _P]),

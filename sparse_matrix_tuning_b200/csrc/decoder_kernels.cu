@@ -186,6 +186,116 @@ __global__ void __launch_bounds__(kFlatThreads) rope_kernel(const uint4* __restr
   }
 }
 
+// ---- per-head RMSNorm of q and k followed by RoPE (Qwen3 attention) ---------------------------------------------
+// rope_kernel's layout: 8 work items per 128-element head row, item j holding vectors j and 8 + j.  The row sums run
+// over the 8 items with xor shuffles in a fixed order, so every item of a row gets the same bits and the result
+// depends on the row alone (a checkpointed recomputation reproduces the first forward).
+//   forward   rstd = rsqrt(mean(x^2) + eps),  y = bf16(w * bf16(x * rstd)),  out = rope_kernel<false>(y)
+//   backward  dy = rope_kernel<true>(g)  (bf16, as autograd produces it),  gw = dy * w,  xhat = x * rstd,
+//             dx = bf16(rstd * (gw - xhat * mean(gw * xhat)))       (rmsnorm_bwd_kernel's formula; w is frozen)
+// Forward reads `a` = (q, k) and writes rstd; backward reads `a` = (dq_out, dk_out), `x` = (q, k) and rstd.
+__device__ __forceinline__ float sum8_rows(float v, unsigned mask) {
+  v += __shfl_xor_sync(mask, v, 4);
+  v += __shfl_xor_sync(mask, v, 2);
+  v += __shfl_xor_sync(mask, v, 1);
+  return v;
+}
+
+template <bool BWD>
+__global__ void __launch_bounds__(kFlatThreads) qk_norm_rope_kernel(
+    const uint4* __restrict__ a_q, const uint4* __restrict__ a_k, const uint4* __restrict__ x_q,
+    const uint4* __restrict__ x_k, const uint4* __restrict__ wq, const uint4* __restrict__ wk, float eps_q, float eps_k,
+    const uint4* __restrict__ cos_, const uint4* __restrict__ sin_, int S, int Hq, int Hk, int64_t rows_q,
+    int64_t rows_k, int64_t cs_bstride_vec, float* __restrict__ rstd_q, float* __restrict__ rstd_k,
+    uint4* __restrict__ out_q, uint4* __restrict__ out_k) {
+  constexpr int VPR = kHeadDim / 8;
+  constexpr float kInvD = 1.0f / kHeadDim;
+  const int64_t items = (rows_q + rows_k) * 8;
+  // the 8 items of a row are 8 aligned lanes of one warp (block size and grid stride are multiples of 32), and they
+  // enter and leave the loop together
+  const unsigned mask = 0xffu << (threadIdx.x & 24);
+  for (int64_t it = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; it < items; it += (int64_t)gridDim.x * blockDim.x) {
+    int64_t row = it >> 3;
+    const int j = (int)(it & 7);
+    const uint4 *src, *xs, *w;
+    uint4* dst;
+    float* rstd_p;
+    float eps;
+    int64_t tok;
+    if (row < rows_q) {
+      src = a_q + row * VPR;
+      xs = BWD ? x_q + row * VPR : nullptr;
+      dst = out_q + row * VPR;
+      rstd_p = rstd_q + row;
+      w = wq;
+      eps = eps_q;
+      tok = row / Hq;
+    } else {
+      row -= rows_q;
+      src = a_k + row * VPR;
+      xs = BWD ? x_k + row * VPR : nullptr;
+      dst = out_k + row * VPR;
+      rstd_p = rstd_k + row;
+      w = wk;
+      eps = eps_k;
+      tok = row / Hk;
+    }
+    const int64_t b = tok / S, s = tok - b * S;
+    const uint4* cr = cos_ + b * cs_bstride_vec + s * VPR;
+    const uint4* sr = sin_ + b * cs_bstride_vec + s * VPR;
+    float a1[8], a2[8], c1[8], c2[8], s1[8], s2[8], w1[8], w2[8], o1[8], o2[8];
+    unpack_bf16x8(ld_stream_u4(src + j), a1);
+    unpack_bf16x8(ld_stream_u4(src + 8 + j), a2);
+    unpack_bf16x8(cr[j], c1);
+    unpack_bf16x8(cr[8 + j], c2);
+    unpack_bf16x8(sr[j], s1);
+    unpack_bf16x8(sr[8 + j], s2);
+    unpack_bf16x8(w[j], w1);
+    unpack_bf16x8(w[8 + j], w2);
+    if (!BWD) {
+      float ss = 0.f;
+#pragma unroll
+      for (int e = 0; e < 8; ++e) ss += __fmul_rn(a1[e], a1[e]);
+#pragma unroll
+      for (int e = 0; e < 8; ++e) ss += __fmul_rn(a2[e], a2[e]);
+      const float rstd = rsqrtf(__fadd_rn(__fmul_rn(sum8_rows(ss, mask), kInvD), eps));
+      if (j == 0) *rstd_p = rstd;
+#pragma unroll
+      for (int e = 0; e < 8; ++e) {
+        const float y1 = bf16r(w1[e] * bf16r(__fmul_rn(a1[e], rstd)));
+        const float y2 = bf16r(w2[e] * bf16r(__fmul_rn(a2[e], rstd)));
+        o1[e] = bf16r(y1 * c1[e]) + bf16r(-y2 * s1[e]);
+        o2[e] = bf16r(y2 * c2[e]) + bf16r(y1 * s2[e]);
+      }
+    } else {
+      const float rstd = *rstd_p;
+      float x1[8], x2[8];
+      unpack_bf16x8(ld_stream_u4(xs + j), x1);
+      unpack_bf16x8(ld_stream_u4(xs + 8 + j), x2);
+      float dot = 0.f;
+#pragma unroll
+      for (int e = 0; e < 8; ++e) {
+        const float d1 = bf16r(bf16r(a1[e] * c1[e]) + bf16r(a2[e] * s2[e]));
+        const float d2 = bf16r(bf16r(a2[e] * c2[e]) - bf16r(a1[e] * s1[e]));
+        a1[e] = d1 * w1[e];                     // gw, in place of the incoming gradient
+        a2[e] = d2 * w2[e];
+        x1[e] *= rstd;                          // xhat
+        x2[e] *= rstd;
+        dot += a1[e] * x1[e];
+        dot += a2[e] * x2[e];
+      }
+      const float mean_gx = sum8_rows(dot, mask) * kInvD;
+#pragma unroll
+      for (int e = 0; e < 8; ++e) {
+        o1[e] = rstd * (a1[e] - x1[e] * mean_gx);
+        o2[e] = rstd * (a2[e] - x2[e] * mean_gx);
+      }
+    }
+    dst[j] = pack_bf16x8(o1);
+    dst[8 + j] = pack_bf16x8(o2);
+  }
+}
+
 // ---- SwiGLU ----------------------------------------------------------------------------------------------------
 // silu and its derivative are written as in PyTorch's CUDA kernels (exp and division at full precision), so the
 // forward matches torch's `silu(g) * u` bit for bit.
@@ -309,6 +419,50 @@ extern "C" SMT_API int smt_rope_backward(const void* dq_out, const void* dk_out,
                                          int B, int S, int Hq, int Hk, int64_t cs_bstride, void* dq, void* dk,
                                          void* stream) {
   return rope_launch(true, dq_out, dk_out, cos_, sin_, B, S, Hq, Hk, cs_bstride, dq, dk, stream, "smt_rope_backward");
+}
+
+static int qk_norm_rope_launch(bool bwd, const void* a_q, const void* a_k, const void* x_q, const void* x_k,
+                               const void* wq, const void* wk, float eps_q, float eps_k, const void* cos_,
+                               const void* sin_, int B, int S, int Hq, int Hk, int64_t cs_bstride, float* rstd_q,
+                               float* rstd_k, void* out_q, void* out_k, void* stream, const char* who) {
+  SMT_CHECK_ARG(B >= 0 && S >= 0 && Hq >= 0 && Hk >= 0 && cs_bstride >= 0 && cs_bstride % 8 == 0,
+                "%s: bad shape (B %d, S %d, Hq %d, Hk %d, cos/sin batch stride %lld)", who, B, S, Hq, Hk,
+                (long long)cs_bstride);
+  const int64_t rows_q = (int64_t)B * S * Hq, rows_k = (int64_t)B * S * Hk;
+  if (rows_q + rows_k == 0) return SMT_OK;
+  SMT_CHECK_ARG(cos_ && sin_ && (!rows_q || (a_q && wq && rstd_q && out_q && (!bwd || x_q))) &&
+                    (!rows_k || (a_k && wk && rstd_k && out_k && (!bwd || x_k))),
+                "%s: null pointer", who);
+  SMT_CHECK_ARG(aligned16(cos_) && aligned16(sin_) && aligned16(a_q) && aligned16(a_k) && aligned16(x_q) &&
+                    aligned16(x_k) && aligned16(wq) && aligned16(wk) && aligned16(out_q) && aligned16(out_k) &&
+                    (uintptr_t)rstd_q % 4 == 0 && (uintptr_t)rstd_k % 4 == 0,
+                "%s: tensors must be 16-byte aligned (rstd: 4-byte)", who);
+  const int grid = smt::flat_grid((rows_q + rows_k) * 8);
+  auto kern = bwd ? smt::qk_norm_rope_kernel<true> : smt::qk_norm_rope_kernel<false>;
+  kern<<<grid, smt::kFlatThreads, 0, (cudaStream_t)stream>>>(
+      (const uint4*)a_q, (const uint4*)a_k, (const uint4*)x_q, (const uint4*)x_k, (const uint4*)wq, (const uint4*)wk,
+      eps_q, eps_k, (const uint4*)cos_, (const uint4*)sin_, S, Hq > 0 ? Hq : 1, Hk > 0 ? Hk : 1, rows_q, rows_k,
+      cs_bstride / 8, rstd_q, rstd_k, (uint4*)out_q, (uint4*)out_k);
+  SMT_CHECK_LAUNCH();
+  return SMT_OK;
+}
+
+extern "C" SMT_API int smt_qk_norm_rope_forward(const void* q, const void* k, const void* wq, const void* wk,
+                                                float eps_q, float eps_k, const void* cos_, const void* sin_, int B,
+                                                int S, int Hq, int Hk, int64_t cs_bstride, void* q_out, void* k_out,
+                                                float* rstd_q, float* rstd_k, void* stream) {
+  return qk_norm_rope_launch(false, q, k, nullptr, nullptr, wq, wk, eps_q, eps_k, cos_, sin_, B, S, Hq, Hk,
+                             cs_bstride, rstd_q, rstd_k, q_out, k_out, stream, "smt_qk_norm_rope_forward");
+}
+
+extern "C" SMT_API int smt_qk_norm_rope_backward(const void* q, const void* k, const void* wq, const void* wk,
+                                                 const float* rstd_q, const float* rstd_k, const void* cos_,
+                                                 const void* sin_, const void* dq_out, const void* dk_out, int B,
+                                                 int S, int Hq, int Hk, int64_t cs_bstride, void* dq, void* dk,
+                                                 void* stream) {
+  return qk_norm_rope_launch(true, dq_out, dk_out, q, k, wq, wk, 0.f, 0.f, cos_, sin_, B, S, Hq, Hk, cs_bstride,
+                             const_cast<float*>(rstd_q), const_cast<float*>(rstd_k), dq, dk, stream,
+                             "smt_qk_norm_rope_backward");
 }
 
 extern "C" SMT_API int smt_swiglu_forward(const void* g, const void* u, int64_t n, void* h, void* stream) {

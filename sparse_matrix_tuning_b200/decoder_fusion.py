@@ -1,13 +1,16 @@
-"""Native kernels for the elementwise work of transformers' LLaMA decoder layer.
+"""Native kernels for the elementwise work of transformers' LLaMA, Mistral and Qwen3 decoder layers.
 
 Around its GEMMs and attention, an HF `LlamaDecoderLayer` spends most of a training step in short PyTorch ops: the
 fp32 round trip of `LlamaRMSNorm` (six passes where one read and one write do), `rotate_half` + cat + three muls and an
 add per RoPE tensor, `silu(gate) * up`, and the residual adds; with activation checkpointing all of it runs twice.
 `install_layer(layer)` replaces them with the kernels of `csrc/decoder_kernels.cu` through instance-level `forward`
-overrides on the layer, its attention, MLP and two norms (`install_norm` for a model's final norm):
+overrides on the layer, its attention, MLP and two norms (`install_norm` for a model's final norm).  Mistral and Qwen3
+layers have the same bodies except for the attention (`_FAMILIES`), so one set of overrides serves all three:
 
   * LlamaRMSNorm       -> one kernel forward (saves fp32 rstd), one backward (dx only: the weight must be frozen);
-  * LlamaAttention     -> the HF body with `apply_rotary_pos_emb` replaced by one launch for q and k;
+  * LlamaAttention     -> the HF body with `apply_rotary_pos_emb` replaced by one launch for q and k; Mistral's and
+                          Qwen3's bodies also pass `sliding_window` to the attention interface, and Qwen3's per-head
+                          `q_norm` / `k_norm` run inside the same launch as RoPE (`QKNormRoPEFn`);
   * LlamaMLP           -> `down_proj(swiglu(gate_proj(x), up_proj(x)))`, projections still called as modules, so SMT
                           modules, the fused q/k/v group and the warm-up hooks see exactly the calls they saw before;
   * LlamaDecoderLayer  -> the residual add after attention runs inside the post-attention norm kernel, and that norm's
@@ -18,9 +21,10 @@ cache; anything else runs the class's own `forward`.  The overrides are bound wi
 `copy.deepcopy` of a model rebinds them to the copy.  Installed and removed by `smt.fuse_qkv_projections` /
 `smt.unfuse_qkv_projections`.
 
-`install_causal_lm(model)` (`smt.fuse_causal_lm_loss`) overrides `LlamaForCausalLM.forward` so that a training call with
-labels runs the frozen lm_head and the causal-LM cross-entropy chunk by chunk (`LinearCrossEntropyFn`, the kernel of
-`csrc/loss_kernels.cu`) and never materialises the fp32 logits; such a call returns `logits=None`.
+`install_causal_lm(model)` (`smt.fuse_causal_lm_loss`) overrides `<Llama|Mistral|Qwen3>ForCausalLM.forward` so that a
+training call with labels runs the frozen lm_head and the causal-LM cross-entropy chunk by chunk
+(`LinearCrossEntropyFn`, the kernel of `csrc/loss_kernels.cu`) and never materialises the fp32 logits; such a call
+returns `logits=None`.
 """
 from __future__ import annotations
 
@@ -101,6 +105,22 @@ class RoPEFn(torch.autograd.Function):
         return dq, dk, None, None
 
 
+class QKNormRoPEFn(torch.autograd.Function):
+    """(q, k) [B, S, H, 128] -> per-head RMSNorm (frozen weights wq / wk) then RoPE, same layout (Qwen3 attention)."""
+
+    @staticmethod
+    def forward(ctx, q, k, wq, wk, eps_q, eps_k, cos, sin):
+        q_out, k_out, rstd_q, rstd_k = ops.qk_norm_rope_forward(q, k, wq, wk, eps_q, eps_k, cos, sin)
+        ctx.save_for_backward(q, k, rstd_q, rstd_k, wq, wk, cos, sin)
+        return q_out, k_out
+
+    @staticmethod
+    def backward(ctx, dq, dk):
+        q, k, rstd_q, rstd_k, wq, wk, cos, sin = ctx.saved_tensors
+        dq, dk = ops.qk_norm_rope_backward(q, k, wq, wk, rstd_q, rstd_k, cos, sin, dq.contiguous(), dk.contiguous())
+        return dq, dk, None, None, None, None, None, None
+
+
 class SwiGLUFn(torch.autograd.Function):
     """h = silu(g) * u."""
 
@@ -123,6 +143,7 @@ class SwiGLUFn(torch.autograd.Function):
 # 14.5-14.7 ms (the input-gradient GEMM then has 64 tiles for 74 CTA pairs).  2 048 is the smallest transient at no
 # measured cost.
 _CE_CHUNK_ROWS = 2048
+_LM_HEAD_TILE_N = 256       # N tile of the fused forward GEMM (smt_fused_linear_forward takes N % 256 == 0)
 
 
 class LinearCrossEntropyFn(torch.autograd.Function):
@@ -130,17 +151,28 @@ class LinearCrossEntropyFn(torch.autograd.Function):
 
     The input gradient is computed in forward, chunk by chunk: logits = h_c W^T (bf16), the loss kernel overwrites
     them with d loss / d logits, dh_c = dlogits W.  Only one chunk of bf16 logits exists at a time and no fp32 logits at
-    all; the saved state is dh [T, K].  Backward returns dh * grad_output (exact for grad_output == 1)."""
+    all; the saved state is dh [T, K].  Backward returns dh * grad_output (exact for grad_output == 1).
+
+    The fused forward GEMM takes whole N tiles of 256; for V % 256 != 0 (Qwen3: 151 936 = 593 * 256 + 128) it writes
+    the first V - V % 256 columns of each chunk and one library GEMM fills the last V % 256 (under 0.1 % of the work
+    at Qwen3's vocabulary)."""
 
     @staticmethod
     def forward(ctx, h, weight, labels, denom, ignore_index):
         T = h.shape[0]
+        V = weight.shape[0]
+        V0 = V - V % _LM_HEAD_TILE_N
         scale = denom.float().reciprocal().reshape(1)      # the fp32 1/denom autograd of HF's loss propagates
         loss_rows = torch.empty(T, dtype=torch.float32, device=h.device)
         dh = torch.empty_like(h)
         for s in range(0, T, _CE_CHUNK_ROWS):
             e = min(T, s + _CE_CHUNK_ROWS)
-            logits = ops.fused_linear_forward(h[s:e], [weight])[0]
+            if V0 == V:
+                logits = ops.fused_linear_forward(h[s:e], [weight])[0]
+            else:
+                logits = torch.empty(e - s, V, dtype=h.dtype, device=h.device)
+                ops.fused_linear_forward(h[s:e], [weight[:V0]], out=logits[:, :V0])
+                torch.mm(h[s:e], weight[V0:].t(), out=logits[:, V0:])
             loss_rows[s:e] = ops.cross_entropy_rows(logits, labels[s:e], scale, ignore_index)
             ops.fused_linear_dgrad([logits], [weight], out=dh[s:e])
             del logits
@@ -224,11 +256,19 @@ def _mlp_forward(self, x):
     return self.down_proj(h)
 
 
+def _qk_norms_ok(attn) -> bool:
+    # Qwen3's per-head norms: frozen bf16 weights of width 128 that the kernel can read directly
+    return all(not n.weight.requires_grad and _native(n.weight) and n.weight.shape == (128,)
+               and n.weight.is_contiguous() and n.weight.data_ptr() % 16 == 0 for n in (attn.q_norm, attn.k_norm))
+
+
 def _attention_forward(self, hidden_states, position_embeddings=None, attention_mask=None, past_key_values=None,
                        **kwargs):
-    if past_key_values is not None or position_embeddings is None or getattr(_hf_only, "depth", 0):
+    F = _family_of(self, "Attention")
+    if past_key_values is not None or position_embeddings is None or getattr(_hf_only, "depth", 0) \
+            or (F.qk_norm and (self.q_norm.weight.requires_grad or self.k_norm.weight.requires_grad)):
         return type(self).forward(self, hidden_states, position_embeddings, attention_mask, past_key_values, **kwargs)
-    L = _llama()
+    L = F.modeling()
     input_shape = hidden_states.shape[:-1]
     hidden_shape = (*input_shape, -1, self.head_dim)
 
@@ -237,12 +277,19 @@ def _attention_forward(self, hidden_states, position_embeddings=None, attention_
     value_states = self.v_proj(hidden_states).view(hidden_shape).transpose(1, 2)
 
     cos, sin = position_embeddings
-    if _rope_ok(query_states, key_states, cos, sin):
+    if _rope_ok(query_states, key_states, cos, sin) and (not F.qk_norm or _qk_norms_ok(self)):
         # outputs in the projections' [B, S, H, D] layout, handed on as [B, H, S, D] views: the strides HF's
         # elementwise RoPE produces, so the attention kernel is fed exactly as before
-        query_states, key_states = RoPEFn.apply(query_states, key_states, cos, sin)
+        if F.qk_norm:
+            query_states, key_states = QKNormRoPEFn.apply(
+                query_states, key_states, self.q_norm.weight, self.k_norm.weight, float(self.q_norm.variance_epsilon),
+                float(self.k_norm.variance_epsilon), cos, sin)
+        else:
+            query_states, key_states = RoPEFn.apply(query_states, key_states, cos, sin)
         query_states, key_states = query_states.transpose(1, 2), key_states.transpose(1, 2)
     else:
+        if F.qk_norm:
+            query_states, key_states = self.q_norm(query_states), self.k_norm(key_states)
         query_states, key_states = L.apply_rotary_pos_emb(query_states.transpose(1, 2), key_states.transpose(1, 2),
                                                           cos, sin)
 
@@ -256,6 +303,7 @@ def _attention_forward(self, hidden_states, position_embeddings=None, attention_
         attention_mask,
         dropout=0.0 if not self.training else self.attention_dropout,
         scaling=self.scaling,
+        **F.attention_kwargs(self),
         **kwargs,
     )
     attn_output = attn_output.reshape(*input_shape, -1).contiguous()
@@ -291,8 +339,9 @@ def _lm_head_ok(model, h) -> bool:
     if type(head) is not nn.Linear or head.bias is not None:
         return False
     w = head.weight
+    V0 = w.shape[0] - w.shape[0] % _LM_HEAD_TILE_N           # columns the fused forward GEMM computes
     return _native(h, w) and h.requires_grad and not w.requires_grad and w.shape[0] == model.config.vocab_size \
-        and h.shape[-1] == w.shape[1] and w.shape[0] % 8 == 0 and ops.fused_linear_supported([w]) \
+        and h.shape[-1] == w.shape[1] and w.shape[0] % 8 == 0 and V0 > 0 and ops.fused_linear_supported([w[:V0]]) \
         and ops.fused_linear_supported([w], dgrad=True)
 
 
@@ -316,31 +365,50 @@ def _causal_lm_forward(self, input_ids=None, attention_mask=None, position_ids=N
     else:
         logits = self.lm_head(h)
         loss = self.loss_function(logits=logits, labels=labels, vocab_size=self.config.vocab_size, **kwargs)
-    out = _llama().CausalLMOutputWithPast(loss=loss, logits=logits, past_key_values=outputs.past_key_values,
-                                          hidden_states=outputs.hidden_states, attentions=outputs.attentions)
+    from transformers.modeling_outputs import CausalLMOutputWithPast
+    out = CausalLMOutputWithPast(loss=loss, logits=logits, past_key_values=outputs.past_key_values,
+                                 hidden_states=outputs.hidden_states, attentions=outputs.attentions)
     return out if return_dict else out.to_tuple()
 
 
-# ---- version guard and installation ----------------------------------------------------------------------------------
+# ---- model families, version guard and installation ------------------------------------------------------------------
 
+# Forward signatures the overrides copy, by role; LLaMA, Mistral and Qwen3 share them in the transformers version this
+# module was written against.
 _EXPECTED_PARAMS = {
-    "LlamaRMSNorm": ["self", "hidden_states"],
-    "LlamaMLP": ["self", "x"],
-    "LlamaAttention": ["self", "hidden_states", "position_embeddings", "attention_mask", "past_key_values", "kwargs"],
-    "LlamaDecoderLayer": ["self", "hidden_states", "attention_mask", "position_ids", "past_key_values", "use_cache",
-                          "position_embeddings", "kwargs"],
-    "LlamaForCausalLM": ["self", "input_ids", "attention_mask", "position_ids", "past_key_values", "inputs_embeds",
-                         "labels", "use_cache", "logits_to_keep", "kwargs"],
+    "RMSNorm": ["self", "hidden_states"],
+    "MLP": ["self", "x"],
+    "Attention": ["self", "hidden_states", "position_embeddings", "attention_mask", "past_key_values", "kwargs"],
+    "DecoderLayer": ["self", "hidden_states", "attention_mask", "position_ids", "past_key_values", "use_cache",
+                     "position_embeddings", "kwargs"],
+    "ForCausalLM": ["self", "input_ids", "attention_mask", "position_ids", "past_key_values", "inputs_embeds",
+                    "labels", "use_cache", "logits_to_keep", "kwargs"],
 }
-_llama_mod = None
 
 
-def _llama():
-    global _llama_mod
-    if _llama_mod is None:
-        from transformers.models.llama import modeling_llama
-        _llama_mod = modeling_llama
-    return _llama_mod
+class _Family:
+    """One transformers model family whose decoder the overrides reproduce: its modeling module, class-name prefix
+    (`<prefix>DecoderLayer`, ...), the keyword arguments its attention body adds to the attention interface call, and
+    whether q / k pass through a per-head RMSNorm (`q_norm` / `k_norm`) before RoPE."""
+
+    def __init__(self, name, prefix, attention_kwargs, qk_norm):
+        self.name, self.prefix, self.attention_kwargs, self.qk_norm = name, prefix, attention_kwargs, qk_norm
+        self._mod = None
+
+    def modeling(self):
+        if self._mod is None:
+            import importlib
+            self._mod = importlib.import_module(f"transformers.models.{self.name}.modeling_{self.name}")
+        return self._mod
+
+
+_FAMILIES = (
+    _Family("llama", "Llama", lambda attn: {}, qk_norm=False),
+    _Family("mistral", "Mistral", lambda attn: {"sliding_window": getattr(attn.config, "sliding_window", None)},
+            qk_norm=False),
+    _Family("qwen3", "Qwen3", lambda attn: {"sliding_window": attn.sliding_window}, qk_norm=True),
+)
+_family_cache = {}
 
 
 def _causal_lm_loss_fn():
@@ -348,25 +416,40 @@ def _causal_lm_loss_fn():
     return ForCausalLMLoss
 
 
-def _class_matches(module, name: str) -> bool:
-    """`module` is exactly transformers' class `name`, whose forward has the signature these overrides copy."""
+def _class_matches(module, family: _Family, role: str) -> bool:
+    """`module` is exactly `family`'s transformers class for `role`, whose forward has the signature these overrides
+    copy."""
     try:
-        cls = getattr(_llama(), name)
+        cls = getattr(family.modeling(), family.prefix + role)
     except (ImportError, AttributeError):
         return False
-    return type(module) is cls and list(inspect.signature(cls.forward).parameters) == _EXPECTED_PARAMS[name]
+    return type(module) is cls and list(inspect.signature(cls.forward).parameters) == _EXPECTED_PARAMS[role]
+
+
+def _family_of(module, role: str):
+    """The family whose class for `role` `module` is exactly, or None."""
+    key = (type(module), role)
+    if key not in _family_cache:
+        _family_cache[key] = next((f for f in _FAMILIES if _class_matches(module, f, role)), None)
+    return _family_cache[key]
 
 
 def layer_supported(layer) -> bool:
-    """A LLaMA decoder layer of the transformers version this module was written against, with head_dim 128 and
-    a SiLU MLP."""
-    if not _class_matches(layer, "LlamaDecoderLayer"):
+    """A LLaMA, Mistral or Qwen3 decoder layer of the transformers version this module was written against, with
+    head_dim 128 and a SiLU MLP (Qwen3: q_norm / k_norm of width 128)."""
+    F = _family_of(layer, "DecoderLayer")
+    if F is None:
         return False
     attn, mlp = getattr(layer, "self_attn", None), getattr(layer, "mlp", None)
     norms = (getattr(layer, "input_layernorm", None), getattr(layer, "post_attention_layernorm", None))
-    return _class_matches(attn, "LlamaAttention") and _class_matches(mlp, "LlamaMLP") \
-        and all(_class_matches(n, "LlamaRMSNorm") for n in norms) and getattr(attn, "head_dim", None) == 128 \
-        and type(mlp.act_fn).__name__ in ("SiLUActivation", "SiLU")
+    if not (_class_matches(attn, F, "Attention") and _class_matches(mlp, F, "MLP")
+            and all(_class_matches(n, F, "RMSNorm") for n in norms) and getattr(attn, "head_dim", None) == 128
+            and type(mlp.act_fn).__name__ in ("SiLUActivation", "SiLU")):
+        return False
+    if F.qk_norm:
+        qk = (getattr(attn, "q_norm", None), getattr(attn, "k_norm", None))
+        return all(_class_matches(n, F, "RMSNorm") and tuple(n.weight.shape) == (128,) for n in qk)
+    return True
 
 
 def install_layer(layer) -> bool:
@@ -383,15 +466,16 @@ def install_layer(layer) -> bool:
 
 def install_norm(norm) -> bool:
     """The RMSNorm override alone (a model's final norm)."""
-    if not _class_matches(norm, "LlamaRMSNorm"):
+    if _family_of(norm, "RMSNorm") is None:
         return False
     install_forward(norm, _rmsnorm_forward)
     return True
 
 
 def install_causal_lm(model) -> bool:
-    """The fused lm_head + causal-LM loss override on a `LlamaForCausalLM`; False for any other class."""
-    if not _class_matches(model, "LlamaForCausalLM"):
+    """The fused lm_head + causal-LM loss override on a `LlamaForCausalLM`, `MistralForCausalLM` or `Qwen3ForCausalLM`;
+    False for any other class."""
+    if _family_of(model, "ForCausalLM") is None:
         return False
     install_forward(model, _causal_lm_forward)
     return True

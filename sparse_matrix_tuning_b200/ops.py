@@ -589,14 +589,24 @@ def _seg_arrays(tensors: Sequence[torch.Tensor]):
     return ptrs, lds
 
 
-def fused_linear_forward(x2d: torch.Tensor, weights: Sequence[torch.Tensor]) -> list:
-    """[x2d @ W_j^T for j] in ONE tcgen05 launch (smt.py:366 for every module that reads x).  x2d: [T, K]."""
+def fused_linear_forward(x2d: torch.Tensor, weights: Sequence[torch.Tensor],
+                         out: Optional[torch.Tensor] = None) -> list:
+    """[x2d @ W_j^T for j] in ONE tcgen05 launch (smt.py:366 for every module that reads x).  x2d: [T, K].
+    `out`: optional [T, N] destination of a single weight's product, with unit column stride (e.g. the leading columns
+    of a wider buffer)."""
     require_cuda(x2d, *weights)
     _req(x2d.dim() == 2 and x2d.stride(1) == 1 and x2d.dtype == weights[0].dtype and x2d.shape[1] == weights[0].shape[1],
          "x2d.dim() == 2 and x2d.stride(1) == 1 and x2d.dtype == weights[0].dtype and x2d.shape[1] == K")
     _req(x2d.data_ptr() % 16 == 0 and (x2d.stride(0) * 2) % 16 == 0, "16-byte aligned x")
     T, K = x2d.shape
-    ys = [torch.empty(T, w.shape[0], dtype=x2d.dtype, device=x2d.device) for w in weights]
+    if out is None:
+        ys = [torch.empty(T, w.shape[0], dtype=x2d.dtype, device=x2d.device) for w in weights]
+    else:
+        require_cuda(out)
+        _req(len(weights) == 1 and out.shape == (T, weights[0].shape[0]) and out.dtype == x2d.dtype
+             and out.stride(1) == 1 and out.data_ptr() % 16 == 0 and (out.stride(0) * 2) % 16 == 0,
+             "out [T, N] of one weight, x's dtype, unit column stride, 16-byte aligned rows")
+        ys = [out]
     n = len(weights)
     wp, wl = _seg_arrays(weights)
     yp, yl = _seg_arrays(ys)
@@ -682,7 +692,8 @@ def rmsnorm_backward(x: torch.Tensor, weight: torch.Tensor, rstd: torch.Tensor, 
     return dx
 
 
-def _rope(fn_name: str, q: torch.Tensor, k: torch.Tensor, cos: torch.Tensor, sin: torch.Tensor):
+def _rope_shapes(q: torch.Tensor, k: torch.Tensor, cos: torch.Tensor, sin: torch.Tensor):
+    """Checks q [B, S, Hq, 128], k [B, S, Hk, 128] and the cos / sin tables; returns (B, S, Hq, Hk, cos batch stride)."""
     _bf16_operands(q, k)
     require_cuda(cos, sin)
     _req(q.dim() == 4 and k.dim() == 4 and q.shape[:2] == k.shape[:2] and q.shape[3] == 128 and k.shape[3] == 128,
@@ -693,7 +704,11 @@ def _rope(fn_name: str, q: torch.Tensor, k: torch.Tensor, cos: torch.Tensor, sin
          and cos.dtype == torch.bfloat16 and sin.dtype == torch.bfloat16, "bf16 cos / sin of shape [1 or B, S, 128]")
     _req(cos.stride() == sin.stride() and cos.stride()[1:] == (128, 1) and cos.data_ptr() % 16 == 0
          and sin.data_ptr() % 16 == 0 and cos.stride(0) % 8 == 0, "cos / sin with rows of 128 contiguous elements")
-    bstride = 0 if cos.shape[0] == 1 else cos.stride(0)
+    return B, S, Hq, Hk, 0 if cos.shape[0] == 1 else cos.stride(0)
+
+
+def _rope(fn_name: str, q: torch.Tensor, k: torch.Tensor, cos: torch.Tensor, sin: torch.Tensor):
+    B, S, Hq, Hk, bstride = _rope_shapes(q, k, cos, sin)
     qo, ko = torch.empty_like(q), torch.empty_like(k)
     check(getattr(load(), fn_name)(ptr(q), ptr(k), ptr(cos), ptr(sin), B, S, Hq, Hk, bstride, ptr(qo), ptr(ko), _st(q)),
           fn_name)
@@ -710,6 +725,49 @@ def rope_forward(q: torch.Tensor, k: torch.Tensor, cos: torch.Tensor, sin: torch
 def rope_backward(dq_out: torch.Tensor, dk_out: torch.Tensor, cos: torch.Tensor, sin: torch.Tensor):
     """Gradients of q and k through `rope_forward`, in ONE launch."""
     return _rope("smt_rope_backward", dq_out, dk_out, cos, sin)
+
+
+def _qk_norm_weights(wq: torch.Tensor, wk: torch.Tensor) -> None:
+    _bf16_operands(wq, wk)
+    _req(wq.shape == (128,) and wk.shape == (128,), "q / k norm weights of shape [128]")
+
+
+def qk_norm_rope_forward(q: torch.Tensor, k: torch.Tensor, wq: torch.Tensor, wk: torch.Tensor, eps_q: float,
+                         eps_k: float, cos: torch.Tensor, sin: torch.Tensor):
+    """HF Qwen3 `q_norm` / `k_norm` (RMSNorm over each 128-wide head) then `apply_rotary_pos_emb`, on q [B, S, Hq, 128]
+    and k [B, S, Hk, 128] (contiguous) in ONE launch.  Returns (q_out, k_out, rstd_q [B*S*Hq], rstd_k [B*S*Hk])."""
+    B, S, Hq, Hk, bstride = _rope_shapes(q, k, cos, sin)
+    _qk_norm_weights(wq, wk)
+    qo, ko = torch.empty_like(q), torch.empty_like(k)
+    rq = torch.empty(B * S * Hq, dtype=torch.float32, device=q.device)
+    rk = torch.empty(B * S * Hk, dtype=torch.float32, device=q.device)
+    check(load().smt_qk_norm_rope_forward(ptr(q), ptr(k), ptr(wq), ptr(wk), float(eps_q), float(eps_k), ptr(cos),
+                                          ptr(sin), B, S, Hq, Hk, bstride, ptr(qo), ptr(ko), ptr(rq), ptr(rk), _st(q)),
+          "smt_qk_norm_rope_forward")
+    if q.numel() + k.numel() > 0:
+        _count()
+    return qo, ko, rq, rk
+
+
+def qk_norm_rope_backward(q: torch.Tensor, k: torch.Tensor, wq: torch.Tensor, wk: torch.Tensor, rstd_q: torch.Tensor,
+                          rstd_k: torch.Tensor, cos: torch.Tensor, sin: torch.Tensor, dq_out: torch.Tensor,
+                          dk_out: torch.Tensor):
+    """Gradients of q and k through `qk_norm_rope_forward` (frozen weights), in ONE launch; reads the forward's
+    inputs and rstd."""
+    B, S, Hq, Hk, bstride = _rope_shapes(q, k, cos, sin)
+    _qk_norm_weights(wq, wk)
+    _bf16_operands(dq_out, dk_out)
+    _req(dq_out.shape == q.shape and dk_out.shape == k.shape, "dq_out / dk_out of q's / k's shape")
+    for r, n in ((rstd_q, B * S * Hq), (rstd_k, B * S * Hk)):
+        _req(r.dtype == torch.float32 and r.is_contiguous() and r.numel() == n, "fp32 rstd with one entry per head row")
+    dq, dk = torch.empty_like(q), torch.empty_like(k)
+    check(load().smt_qk_norm_rope_backward(ptr(q), ptr(k), ptr(wq), ptr(wk), ptr(rstd_q), ptr(rstd_k), ptr(cos),
+                                           ptr(sin), ptr(dq_out), ptr(dk_out), B, S, Hq, Hk, bstride, ptr(dq), ptr(dk),
+                                           _st(q)),
+          "smt_qk_norm_rope_backward")
+    if q.numel() + k.numel() > 0:
+        _count()
+    return dq, dk
 
 
 def swiglu_forward(g: torch.Tensor, u: torch.Tensor) -> torch.Tensor:

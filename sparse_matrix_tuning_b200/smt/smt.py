@@ -464,8 +464,9 @@ def _shared_group_forward(self, x):
 
 def fuse_qkv_projections(model) -> int:
     """Fuses the dense-side work of every decoder layer it can: q_proj / k_proj / v_proj of each attention module become
-    one fused dense GEMM per direction (see above), and in a LLaMA decoder layer whose projections were fused the
-    elementwise ops around them - the two RMSNorms with the residual add, RoPE and SwiGLU - run on the native kernels of
+    one fused dense GEMM per direction (see above), and in a LLaMA, Mistral or Qwen3 decoder layer whose projections
+    were fused the elementwise ops around them - the two RMSNorms with the residual add, RoPE (with Qwen3's per-head
+    q/k norms) and SwiGLU - run on the native kernels of
     `decoder_fusion` (the model's final norm too).  Returns the number of layers whose projections were fused.  Call
     after `convert_linear_layer_to_matrix_sparsity` / `convert_linear_layer_to_channel_sparsity`; undone by
     `unfuse_qkv_projections` (and automatically by `convert_matrix_sparsity_to_linear_layer` /
@@ -497,8 +498,8 @@ def fuse_qkv_projections(model) -> int:
                 decoder_fusion.install_norm(getattr(m, "norm", None))
     if n_elementwise < len(layers):
         warnings.warn(f"fuse_qkv_projections: elementwise ops of {len(layers) - n_elementwise} of {len(layers)} decoder "
-                      "layers left to transformers (not a LLaMA decoder layer of the supported transformers version, "
-                      "head_dim 128, SiLU)")
+                      "layers left to transformers (not a LLaMA, Mistral or Qwen3 decoder layer of the supported "
+                      "transformers version, head_dim 128, SiLU)")
     return fused
 
 
@@ -517,9 +518,10 @@ def unfuse_qkv_projections(model) -> int:
 
 
 def fuse_causal_lm_loss(model) -> bool:
-    """Runs a `LlamaForCausalLM`'s lm_head and causal-LM cross-entropy as one chunked native op that never builds the
-    fp32 logits (`decoder_fusion.LinearCrossEntropyFn`).  It applies to training calls with `labels` (grad mode on,
-    `logits_to_keep=0`, no KV cache, CUDA bf16, a frozen bias-free lm_head with `out_features == vocab_size`); those
+    """Runs the lm_head and causal-LM cross-entropy of a `LlamaForCausalLM`, `MistralForCausalLM` or `Qwen3ForCausalLM`
+    as one chunked native op that never builds the fp32 logits (`decoder_fusion.LinearCrossEntropyFn`).  It applies to
+    training calls with `labels` (grad mode on, `logits_to_keep=0`, no KV cache, CUDA bf16, a frozen bias-free lm_head
+    with `out_features == vocab_size`, a vocabulary that is a multiple of 64 and at least 256); those
     return the loss with `logits=None`.  `shift_labels`, `ignore_index` and `num_items_in_batch` are honoured as
     transformers' `ForCausalLMLoss` honours them.  Every other call runs the class's own forward, so evaluation under
     `no_grad` still gets logits.  Returns False (and changes nothing) for any other model class.  The override is a
