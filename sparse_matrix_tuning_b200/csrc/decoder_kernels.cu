@@ -353,8 +353,9 @@ extern "C" SMT_API int smt_rmsnorm_forward(const void* a, const void* res, const
                 "smt_rmsnorm_forward: H = %d must be a positive multiple of 8 and <= %d", H, smt::kRowMaxVec * 8192);
   if (T == 0) return SMT_OK;
   SMT_CHECK_ARG(a && w && y && rstd && (!res || h_out), "smt_rmsnorm_forward: null pointer");
-  SMT_CHECK_ARG(aligned16(a) && aligned16(w) && aligned16(y) && (!res || (aligned16(res) && aligned16(h_out))),
-                "smt_rmsnorm_forward: tensors must be 16-byte aligned");
+  SMT_CHECK_ARG(aligned16(a) && aligned16(w) && aligned16(y) && (!res || (aligned16(res) && aligned16(h_out))) &&
+                    (uintptr_t)rstd % 4 == 0,
+                "smt_rmsnorm_forward: tensors must be 16-byte aligned (rstd: 4-byte)");
   const int nvec = H / 8;
   const int threads = smt::row_threads(nvec);
   const float inv_n = 1.0f / (float)H;
@@ -374,8 +375,9 @@ extern "C" SMT_API int smt_rmsnorm_backward(const void* x, const void* w, const 
                 "smt_rmsnorm_backward: H = %d must be a positive multiple of 8 and <= %d", H, smt::kRowMaxVec * 8192);
   if (T == 0) return SMT_OK;
   SMT_CHECK_ARG(x && w && rstd && dy && dx, "smt_rmsnorm_backward: null pointer");
-  SMT_CHECK_ARG(aligned16(x) && aligned16(w) && aligned16(dy) && aligned16(dx) && (!dres || aligned16(dres)),
-                "smt_rmsnorm_backward: tensors must be 16-byte aligned");
+  SMT_CHECK_ARG(aligned16(x) && aligned16(w) && aligned16(dy) && aligned16(dx) && (!dres || aligned16(dres)) &&
+                    (uintptr_t)rstd % 4 == 0,
+                "smt_rmsnorm_backward: tensors must be 16-byte aligned (rstd: 4-byte)");
   const int nvec = H / 8;
   const int threads = smt::row_threads(nvec);
   const float inv_n = 1.0f / (float)H;

@@ -138,7 +138,7 @@ def _tiny_cfg(**kw):
     return LlamaConfig(**base)
 
 
-def _train(M, fuse, sel_attn, sel_mlp, steps=3, lr=1e-3):
+def _train(M, fuse, sel_attn, sel_mlp, steps=3, lr=1e-3, padded=False):
     from transformers import LlamaForCausalLM
     from sparse_matrix_tuning_b200.optim import SMTAdam
     torch.manual_seed(0)
@@ -158,8 +158,9 @@ def _train(M, fuse, sel_attn, sel_mlp, steps=3, lr=1e-3):
         losses = []
         for _ in range(steps):
             ids = torch.randint(0, 512, (2, 128), generator=gen).cuda()
+            mask, pos, labels = _padded_batch(ids) if padded else (None, None, ids)
             opt.zero_grad()
-            loss = model(input_ids=ids, labels=ids, use_cache=False).loss
+            loss = model(input_ids=ids, attention_mask=mask, position_ids=pos, labels=labels, use_cache=False).loss
             loss.backward()
             opt.step()
             losses.append(loss.item())
@@ -170,15 +171,27 @@ def _train(M, fuse, sel_attn, sel_mlp, steps=3, lr=1e-3):
         M.unfuse_qkv_projections(model)
 
 
-@pytest.mark.parametrize("with_mlp", [False, True])
-def test_tiny_llama_smt_training_fused_matches_unfused(M, with_mlp):
+def _padded_batch(ids):
+    """attention_mask, position_ids and labels for `ids` [2, S]: the first sequence left-padded by S // 4 tokens (HF's
+    position ids cumsum(mask) - 1, padding at 1), the second three packed documents whose positions restart at 0."""
+    B, S = ids.shape
+    mask = torch.ones_like(ids)
+    mask[0, :S // 4] = 0
+    pos = (mask.cumsum(-1) - 1).masked_fill(mask == 0, 1)
+    pos[1] = torch.cat([torch.arange(n, device=ids.device) for n in (S // 3, S // 3, S - 2 * (S // 3))])
+    return mask, pos, ids.masked_fill(mask == 0, -100)
+
+
+@pytest.mark.parametrize("with_mlp,padded", [(False, False), (True, False), (True, True)],
+                         ids=["False", "True", "True-padded"])
+def test_tiny_llama_smt_training_fused_matches_unfused(M, with_mlp, padded):
     sel_attn = {("q_proj", 0): [(0, 1), (1, 0)], ("k_proj", 0): [(0, 0)], ("v_proj", 1): [(0, 1)],
                 ("q_proj", 1): [(1, 1)]}
     sel_mlp = {("gate_proj", 0): [(1, 0), (3, 1)], ("up_proj", 1): [(2, 0)], ("down_proj", 0): [(0, 2)]} \
         if with_mlp else {}
     steps, lr = 3, 1e-3
-    l0, p0 = _train(M, False, sel_attn, sel_mlp, steps, lr)
-    l1, p1 = _train(M, True, sel_attn, sel_mlp, steps, lr)
+    l0, p0 = _train(M, False, sel_attn, sel_mlp, steps, lr, padded)
+    l1, p1 = _train(M, True, sel_attn, sel_mlp, steps, lr, padded)
     assert max(abs(a - b) for a, b in zip(l0, l1)) <= 1e-2, (l0, l1)
     assert (p1 - p0).abs().max().item() <= 2 * steps * lr
 

@@ -115,7 +115,7 @@ def _model(family, **kw):
     return getattr(transformers, f"{family}ForCausalLM")(_cfg(family, **kw)).cuda().bfloat16()
 
 
-def _train(M, family, fuse, sel_attn, sel_mlp, steps=3, lr=1e-3, **kw):
+def _train(M, family, fuse, sel_attn, sel_mlp, steps=3, lr=1e-3, padded=False, **kw):
     from sparse_matrix_tuning_b200.optim import SMTAdam
     model = _model(family, **kw)
     M.freeze_unselected_matrix_layer(model, sel_mlp, sel_attn)
@@ -133,8 +133,9 @@ def _train(M, family, fuse, sel_attn, sel_mlp, steps=3, lr=1e-3, **kw):
         losses = []
         for _ in range(steps):
             ids = torch.randint(0, 512, (2, 128), generator=gen).cuda()
+            mask, pos, labels = _padded_batch(ids) if padded else (None, None, ids)
             opt.zero_grad()
-            out = model(input_ids=ids, labels=ids, use_cache=False)
+            out = model(input_ids=ids, attention_mask=mask, position_ids=pos, labels=labels, use_cache=False)
             assert (out.logits is None) == fuse
             out.loss.backward()
             opt.step()
@@ -147,17 +148,32 @@ def _train(M, family, fuse, sel_attn, sel_mlp, steps=3, lr=1e-3, **kw):
         M.unfuse_causal_lm_loss(model)
 
 
-@pytest.mark.parametrize("family,with_mlp,tied", [("Qwen3", False, False), ("Qwen3", True, False),
-                                                   ("Qwen3", True, True), ("Mistral", False, False),
-                                                   ("Mistral", True, False)])
-def test_tiny_smt_training_fused_matches_unfused(M, family, with_mlp, tied):
+def _padded_batch(ids):
+    """attention_mask, position_ids and labels for `ids` [2, S]: the first sequence left-padded by S // 4 tokens (HF's
+    position ids cumsum(mask) - 1, padding at 1), the second three packed documents whose positions restart at 0."""
+    B, S = ids.shape
+    mask = torch.ones_like(ids)
+    mask[0, :S // 4] = 0
+    pos = (mask.cumsum(-1) - 1).masked_fill(mask == 0, 1)
+    pos[1] = torch.cat([torch.arange(n, device=ids.device) for n in (S // 3, S // 3, S - 2 * (S // 3))])
+    return mask, pos, ids.masked_fill(mask == 0, -100)
+
+
+_TRAIN_CASES = [("Qwen3", False, False, False), ("Qwen3", True, False, False), ("Qwen3", True, True, False),
+                ("Mistral", False, False, False), ("Mistral", True, False, False), ("Qwen3", True, False, True),
+                ("Mistral", True, False, True)]
+
+
+@pytest.mark.parametrize("family,with_mlp,tied,padded", _TRAIN_CASES,
+                         ids=["-".join(map(str, c[:3])) + ("-padded" if c[3] else "") for c in _TRAIN_CASES])
+def test_tiny_smt_training_fused_matches_unfused(M, family, with_mlp, tied, padded):
     sel_attn = {("q_proj", 0): [(0, 1), (1, 0)], ("k_proj", 0): [(0, 0)], ("v_proj", 1): [(0, 1)],
                 ("q_proj", 1): [(1, 1)]}
     sel_mlp = {("gate_proj", 0): [(1, 0), (3, 1)], ("up_proj", 1): [(2, 0)], ("down_proj", 0): [(0, 2)]} \
         if with_mlp else {}
     steps, lr = 3, 1e-3
-    l0, p0 = _train(M, family, False, sel_attn, sel_mlp, steps, lr, tie_word_embeddings=tied)
-    l1, p1 = _train(M, family, True, sel_attn, sel_mlp, steps, lr, tie_word_embeddings=tied)
+    l0, p0 = _train(M, family, False, sel_attn, sel_mlp, steps, lr, padded, tie_word_embeddings=tied)
+    l1, p1 = _train(M, family, True, sel_attn, sel_mlp, steps, lr, padded, tie_word_embeddings=tied)
     assert max(abs(a - b) for a, b in zip(l0, l1)) <= 1e-2, (l0, l1)
     assert (p1 - p0).abs().max().item() <= 2 * steps * lr
 
@@ -288,10 +304,11 @@ def mm_calls(monkeypatch):
     return calls
 
 
-@pytest.mark.parametrize("V", [1216, 1024])
-def test_fused_loss_at_a_vocabulary_off_the_256_grid(M, mm_calls, V):
+@pytest.mark.parametrize("family,V", [("Qwen3", 1216), ("Qwen3", 1024), ("Llama", 32064)],
+                         ids=["1216", "1024", "Llama-32064"])
+def test_fused_loss_at_a_vocabulary_off_the_256_grid(M, mm_calls, family, V):
     from sparse_matrix_tuning_b200 import decoder_fusion as D
-    model = _model("Qwen3", vocab_size=V, num_hidden_layers=1)
+    model = _model(family, vocab_size=V, num_hidden_layers=1)
     for p in model.parameters():
         p.requires_grad_(False)
     model.enable_input_require_grads()
