@@ -358,7 +358,10 @@ int check_adam_args(const char* who, float* master, float* exp_avg, float* exp_a
                     int grad_dtype, int64_t n_elems, float lr, float beta1, float beta2, float eps, float weight_decay,
                     float bias_correction1, float bias_correction2, float grad_scale, const float* sqnorm, int n_sqnorm,
                     float max_norm, void* compact_out, int* compact_dtype, AdamArgs* a) {
-  SMT_CHECK_ARG(master && exp_avg && exp_avg_sq && grad, "%s: null pointer", who);
+  SMT_CHECK_ARG(master != nullptr, "%s: null pointer (master)", who);
+  SMT_CHECK_ARG(exp_avg != nullptr, "%s: null pointer (exp_avg)", who);
+  SMT_CHECK_ARG(exp_avg_sq != nullptr, "%s: null pointer (exp_avg_sq)", who);
+  SMT_CHECK_ARG(grad != nullptr, "%s: null pointer (grad)", who);
   SMT_CHECK_ARG(grad_dtype >= SMT_F32 && grad_dtype <= SMT_F16, "%s: bad grad dtype %d", who, grad_dtype);
   SMT_CHECK_ARG(n_elems % 8 == 0, "%s: n_elems must be a multiple of 8", who);
   SMT_CHECK_ARG(aligned16(master) && aligned16(exp_avg) && aligned16(exp_avg_sq) && aligned16(grad) &&
@@ -384,9 +387,12 @@ extern "C" SMT_API size_t smt_grad_sqnorm_workspace_bytes(void) { return kSqPart
 
 extern "C" SMT_API int smt_grad_sqnorm(const void* grad, int grad_dtype, int64_t n, float* out_sqnorm,
                                void* workspace, size_t workspace_bytes, void* stream) {
-  SMT_CHECK_ARG(grad && out_sqnorm, "smt_grad_sqnorm: null pointer");
   SMT_CHECK_ARG(grad_dtype >= SMT_F32 && grad_dtype <= SMT_F16, "smt_grad_sqnorm: bad dtype %d", grad_dtype);
   SMT_CHECK_ARG(n >= 0, "smt_grad_sqnorm: n < 0");
+  // n = 0 needs no gradient pointer (an empty tensor's data_ptr() is 0), but still writes 0 to out_sqnorm: the clip
+  // of smt_compact_adam reads it
+  SMT_CHECK_ARG(grad != nullptr || n == 0, "smt_grad_sqnorm: null pointer (grad)");
+  SMT_CHECK_ARG(out_sqnorm != nullptr, "smt_grad_sqnorm: null pointer (out_sqnorm)");
   SMT_CHECK_ARG(aligned16(grad), "smt_grad_sqnorm: grad must be 16-byte aligned");
   if (workspace == nullptr || workspace_bytes < smt_grad_sqnorm_workspace_bytes()) {
     set_error("smt_grad_sqnorm: workspace too small");

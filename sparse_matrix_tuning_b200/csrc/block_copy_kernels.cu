@@ -39,7 +39,8 @@ int launch_copy(bool gather, const smt_block_ref* table, int n_blocks, int block
                 void* compact, void* stream, const char* who) {
   SMT_CHECK_ARG(n_blocks >= 0, "%s: n_blocks < 0", who);
   if (n_blocks == 0) return SMT_OK;
-  SMT_CHECK_ARG(table && compact, "%s: null pointer", who);
+  SMT_CHECK_ARG(table != nullptr, "%s: null pointer (table)", who);
+  SMT_CHECK_ARG(compact != nullptr, "%s: null pointer (compact)", who);
   SMT_CHECK_ARG(block_ok(block), "%s: block size %d not in {64,128,256}", who, block);
   SMT_CHECK_ARG(elem_bytes == 2 || elem_bytes == 4, "%s: elem_bytes must be 2 or 4", who);
   SMT_CHECK_ARG(aligned16(compact), "%s: compact must be 16-byte aligned", who);

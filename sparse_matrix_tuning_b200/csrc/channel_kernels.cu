@@ -82,7 +82,9 @@ int column_copy(bool gather, void* W, int64_t ldw, int out_features, int in_feat
                 int elem_bytes, void* compact, void* stream, const char* who) {
   SMT_CHECK_ARG(n >= 0 && out_features >= 0, "%s: negative size", who);
   if (n == 0 || out_features == 0) return SMT_OK;
-  SMT_CHECK_ARG(W && idx && compact, "%s: null pointer", who);
+  SMT_CHECK_ARG(W != nullptr, "%s: null pointer (W)", who);
+  SMT_CHECK_ARG(idx != nullptr, "%s: null pointer (idx)", who);
+  SMT_CHECK_ARG(compact != nullptr, "%s: null pointer (compact)", who);
   SMT_CHECK_ARG(elem_bytes == 2 || elem_bytes == 4, "%s: elem_bytes must be 2 or 4", who);
   SMT_CHECK_ARG(ldw >= in_features && in_features > 0, "%s: bad leading dimension", who);
   SMT_CHECK_ARG((n + kTile - 1) / kTile <= 65535, "%s: too many channels", who);
@@ -97,7 +99,9 @@ extern "C" SMT_API int smt_channel_gather(const void* x, int64_t T, int64_t ldx,
                                           int elem_bytes, void* out, void* stream) {
   SMT_CHECK_ARG(T >= 0 && n >= 0, "smt_channel_gather: negative size");
   if (T == 0 || n == 0) return SMT_OK;
-  SMT_CHECK_ARG(x && idx && out, "smt_channel_gather: null pointer");
+  SMT_CHECK_ARG(x != nullptr, "smt_channel_gather: null pointer (x)");
+  SMT_CHECK_ARG(idx != nullptr, "smt_channel_gather: null pointer (idx)");
+  SMT_CHECK_ARG(out != nullptr, "smt_channel_gather: null pointer (out)");
   SMT_CHECK_ARG(elem_bytes == 2 || elem_bytes == 4, "smt_channel_gather: elem_bytes must be 2 or 4");
   SMT_CHECK_ARG(ldx > 0, "smt_channel_gather: bad leading dimension");
   const int64_t total = T * (int64_t)n;

@@ -376,11 +376,12 @@ using namespace smt;
 
 extern "C" SMT_API int smt_score_accumulate(float* acc, const void* grad, int grad_dtype, int64_t n,
                                     void* stream) {
-  SMT_CHECK_ARG(acc && grad, "smt_score_accumulate: null pointer");
   SMT_CHECK_ARG(n >= 0, "smt_score_accumulate: n < 0");
   SMT_CHECK_ARG(grad_dtype >= SMT_F32 && grad_dtype <= SMT_F16, "smt_score_accumulate: bad dtype %d",
                 grad_dtype);
-  if (n == 0) return SMT_OK;
+  if (n == 0) return SMT_OK;                 // no data pointer needed (an empty tensor's data_ptr() is 0)
+  SMT_CHECK_ARG(acc != nullptr, "smt_score_accumulate: null pointer (acc)");
+  SMT_CHECK_ARG(grad != nullptr, "smt_score_accumulate: null pointer (grad)");
   cudaStream_t st = (cudaStream_t)stream;
   int64_t n_vec = (aligned16(acc) && aligned16(grad)) ? n / 8 : 0;
   if (n_vec > 0) {
@@ -401,8 +402,9 @@ extern "C" SMT_API int smt_score_accumulate(float* acc, const void* grad, int gr
 }
 
 namespace {
-int check_blocked(const char* who, const void* p, int rows, int cols, int64_t ld, int block, int elem_bytes) {
-  SMT_CHECK_ARG(p != nullptr, "%s: null pointer", who);
+int check_blocked(const char* who, const char* name, const void* p, int rows, int cols, int64_t ld, int block,
+                  int elem_bytes) {
+  SMT_CHECK_ARG(p != nullptr, "%s: null pointer (%s)", who, name);
   SMT_CHECK_ARG(block_ok(block), "%s: block size %d not in {64,128,256}", who, block);
   SMT_CHECK_ARG(rows > 0 && cols > 0 && rows % block == 0 && cols % block == 0,
                 "%s: matrix %dx%d is not a multiple of block %d", who, rows, cols, block);
@@ -415,7 +417,7 @@ int check_blocked(const char* who, const void* p, int rows, int cols, int64_t ld
 
 extern "C" SMT_API int smt_block_score_reduce(const float* acc, int rows, int cols, int64_t ld, int block,
                                       int strategy, float* scores, void* stream) {
-  if (int rc = check_blocked("smt_block_score_reduce", acc, rows, cols, ld, block, 4)) return rc;
+  if (int rc = check_blocked("smt_block_score_reduce", "acc", acc, rows, cols, ld, block, 4)) return rc;
   SMT_CHECK_ARG(scores != nullptr, "smt_block_score_reduce: null scores");
   SMT_CHECK_ARG(strategy >= SMT_MEAN_ABS && strategy <= SMT_L2, "smt_block_score_reduce: unknown strategy %d", strategy);
   cudaStream_t st = (cudaStream_t)stream;
@@ -438,7 +440,8 @@ extern "C" SMT_API int smt_block_score_reduce(const float* acc, int rows, int co
 extern "C" SMT_API int smt_block_sum_accumulate(float* block_sums, const void* grad, int grad_dtype, int rows,
                                         int cols, int64_t ld, int block, void* stream) {
   SMT_CHECK_ARG(grad_dtype >= SMT_F32 && grad_dtype <= SMT_F16, "smt_block_sum_accumulate: bad dtype %d", grad_dtype);
-  if (int rc = check_blocked("smt_block_sum_accumulate", grad, rows, cols, ld, block, dtype_bytes(grad_dtype))) return rc;
+  if (int rc = check_blocked("smt_block_sum_accumulate", "grad", grad, rows, cols, ld, block, dtype_bytes(grad_dtype)))
+    return rc;
   SMT_CHECK_ARG(block_sums != nullptr, "smt_block_sum_accumulate: null block_sums");
   cudaStream_t st = (cudaStream_t)stream;
   dim3 grid(cols / block, rows / block);
@@ -458,7 +461,8 @@ extern "C" SMT_API int smt_block_sum_accumulate(float* block_sums, const void* g
 
 extern "C" SMT_API int smt_block_sum_finalize(const float* block_sums, float* scores, int64_t n, int block,
                                       void* stream) {
-  SMT_CHECK_ARG(block_sums && scores, "smt_block_sum_finalize: null pointer");
+  SMT_CHECK_ARG(block_sums != nullptr, "smt_block_sum_finalize: null pointer (block_sums)");
+  SMT_CHECK_ARG(scores != nullptr, "smt_block_sum_finalize: null pointer (scores)");
   SMT_CHECK_ARG(block_ok(block), "smt_block_sum_finalize: bad block %d", block);
   if (n <= 0) return SMT_OK;
   int grid = (int)((n + 255) / 256);
@@ -536,7 +540,8 @@ extern "C" SMT_API int smt_block_outer_accumulate(float* block_sums, const float
 
 extern "C" SMT_API int smt_act_score_accumulate(float* acc, const void* x, int x_dtype, int batch, int seq,
                                         int channels, void* stream) {
-  SMT_CHECK_ARG(acc && x, "smt_act_score_accumulate: null pointer");
+  SMT_CHECK_ARG(acc != nullptr, "smt_act_score_accumulate: null pointer (acc)");
+  SMT_CHECK_ARG(x != nullptr, "smt_act_score_accumulate: null pointer (x)");
   SMT_CHECK_ARG(x_dtype >= SMT_F32 && x_dtype <= SMT_F16, "smt_act_score_accumulate: bad dtype %d", x_dtype);
   SMT_CHECK_ARG(batch > 0 && seq > 0 && channels > 0, "smt_act_score_accumulate: empty input");
   SMT_CHECK_ARG(channels % 8 == 0 && aligned16(acc) && aligned16(x), "smt_act_score_accumulate: channels must be a multiple of 8 and pointers 16-byte aligned");
@@ -552,7 +557,8 @@ extern "C" SMT_API int smt_act_score_accumulate(float* acc, const void* x, int x
 
 extern "C" SMT_API int smt_channel_score_reduce(const float* acc, int seq, int channels, int strategy,
                                         float* out, void* stream) {
-  SMT_CHECK_ARG(acc && out, "smt_channel_score_reduce: null pointer");
+  SMT_CHECK_ARG(acc != nullptr, "smt_channel_score_reduce: null pointer (acc)");
+  SMT_CHECK_ARG(out != nullptr, "smt_channel_score_reduce: null pointer (out)");
   SMT_CHECK_ARG(seq > 0 && channels > 0 && channels % 4 == 0, "smt_channel_score_reduce: channels must be a positive multiple of 4");
   SMT_CHECK_ARG(aligned16(acc) && aligned16(out), "smt_channel_score_reduce: pointers must be 16-byte aligned");
   SMT_CHECK_ARG(strategy >= SMT_MEAN_ABS && strategy <= SMT_L2, "smt_channel_score_reduce: unknown strategy %d", strategy);

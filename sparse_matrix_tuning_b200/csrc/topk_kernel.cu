@@ -141,7 +141,11 @@ extern "C" SMT_API int smt_topk_blocks(const float* scores, const uint32_t* tieb
                                void* workspace, size_t workspace_bytes, void* stream) {
   SMT_CHECK_ARG(num_segments >= 0, "smt_topk_blocks: num_segments < 0");
   if (num_segments == 0 || n_scores == 0) return SMT_OK;
-  SMT_CHECK_ARG(scores && seg_offsets && seg_k && out_offsets && out_idx, "smt_topk_blocks: null pointer");
+  SMT_CHECK_ARG(scores != nullptr, "smt_topk_blocks: null pointer (scores)");
+  SMT_CHECK_ARG(seg_offsets != nullptr, "smt_topk_blocks: null pointer (seg_offsets)");
+  SMT_CHECK_ARG(seg_k != nullptr, "smt_topk_blocks: null pointer (seg_k)");
+  SMT_CHECK_ARG(out_offsets != nullptr, "smt_topk_blocks: null pointer (out_offsets)");
+  SMT_CHECK_ARG(out_idx != nullptr, "smt_topk_blocks: null pointer (out_idx)");
   SMT_CHECK_ARG((tiebreak_rank == nullptr) == (inv_rank == nullptr), "smt_topk_blocks: tiebreak_rank and inv_rank must be given together");
   SMT_CHECK_ARG(n_scores < (1ll << 31), "smt_topk_blocks: too many scores");
   if (workspace_bytes < smt_topk_workspace_bytes(n_scores) || workspace == nullptr) {

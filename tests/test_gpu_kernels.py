@@ -62,7 +62,7 @@ def test_score_accumulate_matches_capture_loop(ops, dtype):
     assert torch.equal(odd.cpu(), g.float())
 
 
-@pytest.mark.parametrize("block", [64, 256])
+@pytest.mark.parametrize("block", [64, 256, 128])
 def test_block_sum_mode_reproduces_mean_abs(ops, block):
     torch.manual_seed(2)
     sums = torch.zeros(512 // block, 768 // block, device="cuda")
@@ -149,7 +149,7 @@ def test_topk_segments_and_degenerate_sizes(ops):
 # ---- gather / scatter: byte-exact -------------------------------------------------------------------------
 
 @pytest.mark.parametrize("block", [64, 128, 256])
-@pytest.mark.parametrize("dtype", [torch.bfloat16, torch.float32])
+@pytest.mark.parametrize("dtype", [torch.bfloat16, torch.float32, torch.float16])
 def test_gather_scatter_vs_oracle(ops, block, dtype):
     torch.manual_seed(block)
     w = torch.randn(512, 768).to(dtype)
@@ -168,7 +168,7 @@ def test_gather_scatter_vs_oracle(ops, block, dtype):
 
 # ---- optimizer ----------------------------------------------------------------------------------------------
 
-@pytest.mark.parametrize("grad_dtype", [torch.bfloat16, torch.float32])
+@pytest.mark.parametrize("grad_dtype", [torch.bfloat16, torch.float32, torch.float16])
 def test_compact_adam_bit_exact_vs_numpy_restatement(ops, grad_dtype):
     """fp32 master / exp_avg / exp_avg_sq after each step are BIT-IDENTICAL to oracle.adamw_fused_step (every op
     individually rounded), including the in-kernel clip coefficient; bf16 outputs are the RNE rounding of the master."""
