@@ -22,12 +22,9 @@ import torch
 from .smt import smt as _smt
 
 
-_SPARSE_TYPES = (_smt.LinearLayer_MatrixSparsity, _smt.LinearLayer_ChannelSparsity)
-
-
 def sparse_modules(model) -> "OrderedDict[str, torch.nn.Module]":
     """Every converted module (block- or channel-sparse), by qualified name."""
-    return OrderedDict((n, m) for n, m in model.named_modules() if isinstance(m, _SPARSE_TYPES))
+    return OrderedDict((n, m) for n, m in model.named_modules() if isinstance(m, _smt._SparseLinear))
 
 
 def _plain_index(entry):

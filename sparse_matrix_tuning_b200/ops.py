@@ -6,6 +6,7 @@ Every function launches on the CURRENT CUDA stream of the tensors' device.
 from __future__ import annotations
 
 import ctypes as C
+import functools
 from typing import Optional, Sequence, Tuple
 
 import torch
@@ -121,6 +122,33 @@ def make_block_rc(index_list: Sequence[Tuple[int, int]], device) -> torch.Tensor
     if len(index_list) == 0:
         return torch.empty((0, 2), dtype=torch.int32, device=device)
     return torch.tensor([[int(r), int(c)] for r, c in index_list], dtype=torch.int32, device=device)
+
+
+_index_cache: dict = {}   # id(index_list) -> (snapshot, {(build, device, args): table})
+_INDEX_CACHE_MAX = 4096
+
+
+def index_table(index_list, build=None, device=None, *args):
+    """(snapshot, table) of a Python index list: the snapshot is an immutable copy of the list ((row, col) tuples of
+    ints or channel ints), the table `build(snapshot, device, *args)` (None without `build`).  Layers and autograd
+    functions receive only the plain list, exactly like the reference, so both are cached per list object and
+    validated by value on every call: the common case (same list, same contents) costs one tuple comparison, an edit
+    of the list in place yields a new snapshot and new tables.  At most _INDEX_CACHE_MAX lists are cached."""
+    hit = _index_cache.get(id(index_list))
+    if hit is None or len(hit[0]) != len(index_list) or tuple(index_list) != hit[0]:
+        snap = tuple(tuple(int(v) for v in e) if isinstance(e, (tuple, list)) else int(e) for e in index_list)
+        if hit is None or hit[0] != snap:
+            if len(_index_cache) >= _INDEX_CACHE_MAX:
+                _index_cache.clear()
+            hit = _index_cache[id(index_list)] = (snap, {})
+    snap, tables = hit
+    if build is None:
+        return snap, None
+    key = (build, device, args)
+    table = tables.get(key)
+    if table is None:
+        table = tables[key] = build(snap, device, *args)
+    return snap, table
 
 
 # ---- warm-up scoring -------------------------------------------------------------------------------
@@ -345,7 +373,6 @@ def column_scatter(W: torch.Tensor, idx: torch.Tensor, compact: torch.Tensor) ->
 # ---- block-gradient GEMM --------------------------------------------------------------------------------
 
 _ws_cache: dict = {}
-_channel_items: dict = {}
 
 
 def channel_grad_block(n: int, out_f: int) -> int:
@@ -353,15 +380,9 @@ def channel_grad_block(n: int, out_f: int) -> int:
     return 128 if (out_f % 128 == 0 and n > 64) else 64
 
 
+@functools.lru_cache(maxsize=64)
 def _channel_tiles(rows: int, cols: int) -> tuple:
-    key = ("tiles", rows, cols)
-    hit = _channel_items.get(key)
-    if hit is None:
-        hit = tuple((r, c) for r in range(rows) for c in range(cols))
-        if len(_channel_items) > 64:
-            _channel_items.clear()
-        _channel_items[key] = hit
-    return hit
+    return tuple((r, c) for r in range(rows) for c in range(cols))
 
 
 def channel_grad_gemm(partial: torch.Tensor, n: int, dy2d: torch.Tensor, out: Optional[torch.Tensor] = None,
@@ -373,55 +394,19 @@ def channel_grad_gemm(partial: torch.Tensor, n: int, dy2d: torch.Tensor, out: Op
     the tiles assemble the row-major [n, out_features] gradient directly.  fp32 accumulation over all tokens, ONE
     rounding.  `partial`: [T, n8] (n8 >= n, row pitch a multiple of 16 bytes, columns >= n zero); returns [n, out].
     `out` (optional): contiguous [ceil(n/b)*b, out_features] destination (b = channel_grad_block(n, out_features)); its
-    rows past n receive zeros.  `accumulate` adds into it instead of overwriting it."""
-    require_cuda(partial, dy2d, out)
-    _req(partial.dim() == 2 and dy2d.dim() == 2 and partial.shape[0] == dy2d.shape[0] and partial.dtype == dy2d.dtype,
-         "partial.dim() == 2 and dy2d.dim() == 2 and partial.shape[0] == dy2d.shape[0] and partial.dtype == dy2d.dtype")
-    _req(partial.stride(1) == 1 and dy2d.stride(1) == 1 and partial.dtype in (torch.bfloat16, torch.float16),
-         "partial.stride(1) == 1 and dy2d.stride(1) == 1 and partial.dtype in (torch.bfloat16, torch.float16)")
-    T, out_f = dy2d.shape
-    _req(0 < n <= partial.shape[1] and (partial.stride(0) * 2) % 16 == 0 and (dy2d.stride(0) * 2) % 16 == 0,
-         "0 < n <= partial.shape[1] and 16-byte row pitches")
-    _req(out_f % 64 == 0, "out_features % 64 == 0")
-    block = channel_grad_block(n, out_f)
-    rows, cols = (n + block - 1) // block, out_f // block
-    dev = dy2d.device
+    rows past n receive zeros.  `accumulate` adds into it instead of overwriting it.
+    It is one `BlockGradBatch.add_channel` problem, launched (and timed as "block_grad_gemm") by the batch's flush."""
+    out_f = dy2d.shape[-1]
     if out is None:
-        out = torch.empty(rows * block, out_f, dtype=dy2d.dtype, device=dev)
+        block = channel_grad_block(n, out_f)
+        out = torch.empty(max(n + block - 1, 0) // block * block, out_f, dtype=dy2d.dtype, device=dy2d.device)
         accumulate = False
-    _req(out.is_contiguous() and out.shape == (rows * block, out_f) and out.dtype == dy2d.dtype,
-         "out: contiguous [ceil(n/b)*b, out_features] of dy's dtype")
-    if T == 0:
-        if not accumulate:
-            out.zero_()
-        return out[:n]
-    import numpy as np
-    key = (rows, cols, block, out_f, bool(accumulate))
-    arr = _channel_items.get(key)
-    if arr is None:
-        flags = 0 if accumulate else _lib.ITEM_OVERWRITE
-        arr = np.array([(0, 1, r, c, r * block * out_f + c * block, flags, -1)
-                        for r in range(rows) for c in range(cols)], dtype=_item_dtype())
-        if len(_channel_items) > 64:
-            _channel_items.clear()
-        _channel_items[key] = arr
-    lib = load()
-    n_items = len(arr)
-    stage = torch.empty(2 * 128 + arr.nbytes, dtype=torch.uint8, pin_memory=True)
-    in_id = dtype_id(dy2d.dtype)
-    check(lib.smt_encode_operand_map(stage.data_ptr(), partial.data_ptr(), partial.shape[1], T, partial.stride(0),
-                                     in_id, block), "smt_encode_operand_map")
-    check(lib.smt_encode_operand_map(stage.data_ptr() + 128, dy2d.data_ptr(), out_f, T, dy2d.stride(0), in_id, block),
-          "smt_encode_operand_map")
-    stage.numpy()[256:] = arr.view("u1").reshape(-1)
-    dev_buf = stage.to(dev, non_blocking=True)
-    ws_bytes = lib.smt_block_grad_gemm_grouped_workspace_bytes(n_items, block, T)
-    ws = _workspace(ws_bytes, dev)
-    with _timed("channel_grad_gemm", dev, (n, out_f, T)):
-        check(lib.smt_block_grad_gemm_grouped(dev_buf.data_ptr(), dev_buf.data_ptr() + 256, n_items, T, block, in_id,
-                                              out.data_ptr(), dtype_id(out.dtype), 1 if accumulate else 0, out_f, 0,
-                                              ptr(ws), ws_bytes, stream_ptr(dev)), "smt_block_grad_gemm_grouped")
-    _count(lib.smt_last_launch_count())
+    batch = BlockGradBatch()
+    batch.add_channel(partial, dy2d, n, out, accumulate=accumulate)         # checks every argument
+    if dy2d.shape[0] > 0:
+        batch.flush()                           # the per-item flags overwrite unless `accumulate`
+    elif not accumulate:
+        out.zero_()
     return out[:n]
 
 
@@ -439,20 +424,18 @@ def _workspace(nbytes: int, device, tag: str = "gemm") -> Optional[torch.Tensor]
     return buf
 
 
-_runs_cache: dict = {}
 LAST_SINGLE: dict = {}    # which kernel the last single-problem block_grad_gemm used (tests / reports)
 
 
 def _runs_for(index_list, block: int, device):
-    """Strip-sharing runs of an index list (cached per list object, validated by value): blocks grouped by block row,
-    columns ascending, cut into runs of at most `run width` blocks (b = 64 / 128).
+    """Strip-sharing runs of an index list (cached by `index_table`): blocks grouped by block row, columns ascending,
+    cut into runs of at most `run width` blocks (b = 64 / 128).
     Returns (device tensor of smt_gemm_run, number of runs, fraction of the blocks that sit in a run of >= 2)."""
+    return index_table(index_list, _make_runs, device, block)[1]
+
+
+def _make_runs(snap, device, block: int):
     import numpy as np
-    snap = _snapshot_index_list(index_list)
-    key = (id(index_list), block, device)
-    hit = _runs_cache.get(key)
-    if hit is not None and hit[0] is snap:
-        return hit[1]
     width = load().smt_block_grad_gemm_run_width(block)
     by_row: dict = {}
     for i, (r, c) in enumerate(snap):
@@ -470,11 +453,7 @@ def _runs_for(index_list, block: int, device):
     arr = np.array(rows, dtype=np.int32).reshape(-1, 10)
     assert arr.shape[1] * 4 == C.sizeof(_lib.GemmRun)
     dev = torch.from_numpy(arr).to(device) if len(rows) else torch.empty((0, 10), dtype=torch.int32, device=device)
-    res = (dev, len(rows), shared / max(len(snap), 1))
-    if len(_runs_cache) > 4096:
-        _runs_cache.clear()
-    _runs_cache[key] = (snap, res)
-    return res
+    return dev, len(rows), shared / max(len(snap), 1)
 
 
 def block_grad_gemm(x2d: torch.Tensor, dy2d: torch.Tensor, block_rc: torch.Tensor, block: int,
@@ -895,29 +874,15 @@ def _item_dtype():
 
 
 class _Problem:
-    __slots__ = ("x", "dy", "idx", "idx_id", "out", "block", "accumulate", "sq", "sq_slot0", "sink", "ld_out")
+    __slots__ = ("x", "dy", "idx", "out", "block", "accumulate", "sq", "sq_slot0", "sink", "ld_out")
 
-    def __init__(self, x, dy, idx, idx_id, out, block, accumulate, sq, sq_slot0, sink, ld_out=0):
-        self.x, self.dy, self.idx, self.idx_id, self.out, self.block = x, dy, idx, idx_id, out, block
+    def __init__(self, x, dy, idx, out, block, accumulate, sq, sq_slot0, sink, ld_out=0):
+        self.x, self.dy, self.idx, self.out, self.block = x, dy, idx, out, block
         self.accumulate, self.sq, self.sq_slot0, self.sink = accumulate, sq, sq_slot0, sink
         self.ld_out = ld_out          # 0: compact b x b tiles; > 0: tiles of a row-major matrix with this row pitch
 
 
-_idx_snap: dict = {}      # id(index_list) -> tuple snapshot (validated by value on every use)
-
-
-def _snapshot_index_list(index_list):
-    """Immutable ((row, col), ...) copy of a Python index list; the common case (same list object, same contents as
-    last step) costs one tuple comparison instead of n int() conversions."""
-    key = id(index_list)
-    hit = _idx_snap.get(key)
-    if hit is not None and len(hit) == len(index_list) and tuple(index_list) == hit:
-        return hit
-    snap = tuple((int(r), int(c)) for r, c in index_list)
-    if len(_idx_snap) > 8192:
-        _idx_snap.clear()
-    _idx_snap[key] = snap
-    return snap
+_plans: dict = {}         # work-item arrays of BlockGradBatch._items_for, shared by every batch
 
 
 class BlockGradBatch:
@@ -935,7 +900,6 @@ class BlockGradBatch:
         self.problems = []
         self.last_flushed = []
         self._out_ptrs = set()
-        self._plans: dict = {}
 
     def __len__(self):
         return len(self.problems)
@@ -958,8 +922,8 @@ class BlockGradBatch:
             # the same output twice in one launch would race (two tiles read-modify-write the same block)
             self.flush()
         self._out_ptrs.add(out.data_ptr())
-        self.problems.append(_Problem(x2d, dy2d, _snapshot_index_list(index_list), id(index_list), out, int(block),
-                                      bool(accumulate), sq, int(sq_slot0), sink))
+        self.problems.append(_Problem(x2d, dy2d, index_table(index_list)[0], out, int(block), bool(accumulate), sq,
+                                      int(sq_slot0), sink))
 
     def add_channel(self, partial: torch.Tensor, dy2d: torch.Tensor, n: int, out: torch.Tensor, accumulate: bool = True,
                     sq: Optional[torch.Tensor] = None, sq_slot0: int = -1, sink=None) -> None:
@@ -983,8 +947,8 @@ class BlockGradBatch:
             self.flush()
         self._out_ptrs.add(out.data_ptr())
         # the packed channels are the `dy` operand, grad_output the `x` operand (see channel_grad_gemm)
-        self.problems.append(_Problem(dy2d, partial, _channel_tiles(rows, out_f // block), None, out, block,
-                                      bool(accumulate), sq, int(sq_slot0), sink, ld_out=out_f))
+        self.problems.append(_Problem(dy2d, partial, _channel_tiles(rows, out_f // block), out, block, bool(accumulate),
+                                      sq, int(sq_slot0), sink, ld_out=out_f))
 
     def flush(self, accumulate: bool = True) -> int:
         """Launches everything collected so far; returns the number of grouped launches.  `last_flushed` keeps the
@@ -1025,7 +989,7 @@ class BlockGradBatch:
         key = (T, block, ld_out, tuple((pr.idx, (pr.out.data_ptr() - base_ptr) // esize, pr.accumulate,
                                 pr.sq_slot0 if pr.sq is not None else -1, mx, mdy)
                                for pr, (mx, mdy) in zip(prs, maps_of)))
-        hit = self._plans.get(key)
+        hit = _plans.get(key)
         if hit is not None:
             return hit
         items, carry = [], []
@@ -1049,9 +1013,9 @@ class BlockGradBatch:
         arr = np.array(items, dtype=_item_dtype())
         n_pairs = sum(1 for k in range(0, len(items) - 1, 2)
                       if items[k][0] == items[k + 1][0] and items[k][2] == items[k + 1][2])
-        if len(self._plans) > 64:
-            self._plans.clear()
-        self._plans[key] = (arr, n_pairs)
+        if len(_plans) > 64:
+            _plans.clear()
+        _plans[key] = (arr, n_pairs)
         return arr, n_pairs
 
     def _launch_group(self, T, in_dt, out_dt, block, dev, prs, accumulate, ld_out=0) -> None:

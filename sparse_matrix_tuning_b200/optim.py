@@ -35,7 +35,6 @@ itself at the next backward and starts from an overwrite; parameters without a s
 """
 from __future__ import annotations
 
-import weakref
 from typing import List, Optional
 
 import torch
@@ -441,8 +440,3 @@ class SMTAdam(torch.optim.Optimizer):
         else:
             torch.autograd.graph.increment_version(p)
 
-
-def register_owner(param: torch.nn.Parameter, module) -> None:
-    """Ties a `selected_weight` Parameter to its LinearLayer_MatrixSparsity (weakly) so the optimizer can
-    find the dense weight to write back into."""
-    param._smt_owner = weakref.ref(module)

@@ -26,16 +26,18 @@ What changed underneath:
 The channel-sparsity twins (`LinearLayer_ChannelSparsity`, `linearChannel`, `convert_linear_layer_to_channel_sparsity`,
 `freeze_unselected_channel_layer`; smt.py:25-80, 185-296, 748-831) keep the reference's names and signatures but use
 COLUMN semantics: the reference selects input channels, differentiates weight columns and copies weight rows, which
-fails for every non-square weight (SURVEY.md section 2 row 16).  Its gradient formula is kept exactly.
+fails for every non-square weight (SURVEY.md section 2 row 16).  Its gradient formula is kept exactly.  The two layer
+kinds share their base class (`_SparseLinear`), their gradient delivery (`_deliver`) and their device index tables
+(`ops.index_table`); only the gather / scatter and the gradient problem differ.
 """
 from __future__ import annotations
 
 import contextlib
+import functools
 import re
 import threading
 import warnings
 import weakref
-from typing import Dict, Tuple
 
 import torch
 from torch import nn
@@ -87,26 +89,6 @@ def _attn_kind(name: str):
         if kind in name:
             return kind
     return None
-
-
-# ---- device-side index tables ---------------------------------------------------------------------------
-
-_rc_cache: Dict[Tuple[int, torch.device], Tuple[tuple, torch.Tensor]] = {}
-
-
-def _block_rc_for(index_list, device) -> torch.Tensor:
-    """int32 [n, 2] device copy of a Python index list, cached per list object and validated by value
-    (linearZ receives only the plain list, exactly like the reference)."""
-    snap = tuple((int(r), int(c)) for r, c in index_list)
-    key = (id(index_list), device)
-    hit = _rc_cache.get(key)
-    if hit is not None and hit[0] == snap:
-        return hit[1]
-    t = ops.make_block_rc(snap, device)
-    if len(_rc_cache) > 4096:
-        _rc_cache.clear()
-    _rc_cache[key] = (snap, t)
-    return t
 
 
 # ---- deferred, grouped block-gradient launches (native mode only) ------------------------------------------------
@@ -174,25 +156,27 @@ def flush_block_grads() -> int:
         return _flush_locked()
 
 
-def _enqueue(xkey, device, add) -> None:
-    """Queue one module's gradient problem (`add()` puts it into `_pending`); `xkey` identifies the module's input, so
-    that a chunked flush happens at a layer boundary."""
+def _deliver(sw_param, sink, xkey, device, grouped: bool, add, launch) -> None:
+    """Native mode: one module's weight gradient into the GradSink of its parameter.  The sink says whether this
+    delivery accumulates or overwrites (the first one after a lazy zero_grad).  Grouped: `add(accumulate=, sq=,
+    sq_slot0=, sink=)` (a `_pending.add` / `_pending.add_channel` with the operands bound) queues the problem for the
+    grouped launch(es) of this backward pass; `xkey` identifies the module's input, so that a chunked flush happens at
+    a layer boundary.  Otherwise `launch(accumulate=)` runs it now; a per-module launch emits no sums of squares."""
+    accumulate = sink.begin_delivery(sw_param)
+    if not grouped:
+        launch(accumulate=accumulate)
+        sink.sq_ok = False
+        return
     with _pending_lock:
         chunk = _grouped["chunk_blocks"]
         if chunk > 0 and _pending_state["last_x"] not in (None, xkey) and _pending.n_blocks() >= chunk:
             _flush_locked()                                     # layer boundary with a GPU-filling chunk pending
         _pending_state["last_x"] = xkey
-        add()
+        add(accumulate=accumulate, sq=sink.sq, sq_slot0=sink.sq_slot0, sink=sink)
         _pending_state["stream"] = torch.cuda.current_stream(device)
         if not _pending_state["callback_queued"]:
             _pending_state["callback_queued"] = True
             torch.autograd.Variable._execution_engine.queue_callback(flush_block_grads)
-
-
-def _enqueue_block_grad(x2, dy2, index_list, sink, block, accumulate) -> None:
-    _enqueue((x2.data_ptr(), x2.shape[0]), x2.device,
-             lambda: _pending.add(x2, dy2, index_list, sink.view, block, accumulate=accumulate, sq=sink.sq,
-                                  sq_slot0=sink.sq_slot0, sink=sink))
 
 
 class linearZ(torch.autograd.Function):
@@ -237,35 +221,84 @@ def _block_weight_grad(sw_param, index_list, x2, dy2, b, out_dtype):
     n = len(index_list)
     if x2.dtype != dy2.dtype:
         x2 = x2.to(dy2.dtype)
+
+    def launch(**kw):
+        rc = ops.index_table(index_list, ops.make_block_rc, dy2.device)[1]
+        return ops.block_grad_gemm(x2, dy2, rc, b, index_list=index_list, **kw)
+
     sink = getattr(sw_param, "_smt_sink", None)
-    if sink is not None:
-        # the sink says whether this delivery accumulates or overwrites (first one after a lazy zero_grad)
-        accumulate = sink.begin_delivery(sw_param)
-        if _grouped["enabled"] and dy2.dtype != torch.float32 and n > 0:
-            _enqueue_block_grad(x2, dy2, index_list, sink, b, accumulate)   # grouped launch(es) per backward
-        else:
-            rc = _block_rc_for(index_list, dy2.device)
-            ops.block_grad_gemm(x2, dy2, rc, b, out=sink.view, accumulate=accumulate, index_list=index_list)
-            sink.sq_ok = False
-        return None
-    rc = _block_rc_for(index_list, dy2.device)
-    return ops.block_grad_gemm(x2, dy2, rc, b, out_dtype=out_dtype, index_list=index_list).view(n * b, b)   # smt.py:382-404
+    if sink is None:
+        return launch(out_dtype=out_dtype).view(n * b, b)                                  # smt.py:382-404
+    _deliver(sw_param, sink, (x2.data_ptr(), x2.shape[0]), x2.device,
+             _grouped["enabled"] and dy2.dtype != torch.float32 and n > 0,
+             functools.partial(_pending.add, x2, dy2, index_list, sink.view, b), functools.partial(launch, out=sink.view))
+    return None
 
 
-class LinearLayer_MatrixSparsity(nn.Module):
+class _SparseLinear(nn.Module):
+    """What the block- and the channel-sparse layer share: a frozen dense `weight`, the only trainable parameter
+    `selected_weight` (a compact copy of the selected part of `weight`, gathered by the subclass), the compact -> dense
+    write-back before every forward (`_scatter`), and the protocol of SMTAdam's arena (optim._Arena): `_smt_owner`,
+    `_arena_ok`, `_arena_layout`, `_writeback`, `_writeback_args`, `mark_synced` and `sync_weight`."""
+
+    def __init__(self, weight, bias, index_list):
+        super().__init__()
+        if not weight.is_cuda:
+            raise SMTLibraryError(f"{type(self).__name__} needs its weight on a CUDA device: the SMT kernels have no "
+                                  "CPU fallback")
+        self.weight = weight
+        self.weight.requires_grad = False                 # smt.py:308 / 191
+        self.bias = bias                                  # kept but unused, exactly like smt.py:309,343 / 192,214
+        self.index_list = index_list
+
+    def _set_selected(self, compact: torch.Tensor, fn) -> None:
+        """The constructor's last step, once the subclass has validated `index_list` and gathered `compact`."""
+        self.selected_weight = nn.Parameter(compact, requires_grad=True)
+        self.selected_weight._smt_owner = weakref.ref(self)   # lets SMTAdam find the dense weight to write back
+        self.fn = fn
+        # Set ONLY by `mark_synced()` (= SMTAdam after its fused write-back): (storage pointer, version) of
+        # selected_weight at that moment.  None = "nobody vouches for the dense weight": scatter on every forward.
+        self._synced = None
+
+    def _apply(self, fn, *args, **kwargs):
+        out = super()._apply(fn, *args, **kwargs)
+        self._synced = None
+        return out
+
+    def mark_synced(self) -> None:
+        """Called by the fused optimizer (SMTAdam) right after it has written the updated blocks / channels into
+        `weight` itself.  The mark is tied to the parameter's storage pointer and version counter: re-pointing `.data`
+        (DeepSpeed / ZeRO flat buffers) or any version-counted write to the Parameter invalidates it.  Writes
+        through `selected_weight.data` are invisible to the version counter, so whoever does that while SMTAdam
+        owns the parameter must call `sync_weight(force=True)`; without SMTAdam nothing is ever skipped."""
+        self._synced = (self.selected_weight.data_ptr(), self.selected_weight._version)
+
+    def sync_weight(self, force: bool = False) -> None:
+        """compact -> dense write-back (smt.py:332-341 / 208-211): ONE launch per call.  Unconditional like the
+        reference's loop - whatever optimizer updated `selected_weight` (also through `.data` or an aliased flat
+        buffer) is seen - except right after an SMTAdam step that wrote the dense weight itself (see `mark_synced`)."""
+        if not force and self._synced is not None and \
+                self._synced == (self.selected_weight.data_ptr(), self.selected_weight._version):
+            return
+        self._synced = None
+        if len(self.index_list):
+            sw = self.selected_weight.data
+            if sw.dtype != self.weight.dtype:
+                sw = sw.to(self.weight.dtype)
+            self._scatter(sw.contiguous())
+
+    def forward(self, x):
+        self.sync_weight()
+        return self.fn(x, self.selected_weight, self.index_list, self.weight)   # smt.py:343 / 213
+
+
+class LinearLayer_MatrixSparsity(_SparseLinear):
     """Linear layer whose only trainable parameter is a compact copy of its selected b x b blocks.
     Reference: smt.py:302-344 (same constructor signature and attribute names)."""
 
     def __init__(self, weight, bias=None, index_list=[]):
-        super().__init__()
-        if not weight.is_cuda:
-            raise SMTLibraryError("LinearLayer_MatrixSparsity needs its weight on a CUDA device: the SMT kernels "
-                                  "have no CPU fallback")
+        super().__init__(weight, bias, index_list)
         b = Block_dimension
-        self.weight = weight
-        self.weight.requires_grad = False                 # smt.py:308
-        self.bias = bias                                  # kept but unused, exactly like smt.py:309,343
-        self.index_list = index_list
         self.block = b
         for (r, c) in index_list:
             if not (0 <= r < weight.shape[0] // b and 0 <= c < weight.shape[1] // b):
@@ -276,12 +309,7 @@ class LinearLayer_MatrixSparsity(nn.Module):
         self._table_key = None
         if n:
             ops.block_gather(self._block_table(), n, b, compact)       # smt.py:317-325
-        self.selected_weight = nn.Parameter(compact, requires_grad=True)
-        self.selected_weight._smt_owner = weakref.ref(self)   # lets SMTAdam find the dense weight to write back
-        self.fn = linearZ.apply
-        # Set ONLY by `mark_synced()` (= SMTAdam after its fused write-back): (storage pointer, version) of
-        # selected_weight at that moment.  None = "nobody vouches for the dense weight": scatter on every forward.
-        self._synced = None
+        self._set_selected(compact, linearZ.apply)
 
     # -- device table of (W pointer, ld, row, col) per block, rebuilt if the weight storage moves --
     def _block_table(self) -> torch.Tensor:
@@ -292,10 +320,12 @@ class LinearLayer_MatrixSparsity(nn.Module):
             self._table_key = key
         return self._table
 
+    def _scatter(self, compact: torch.Tensor) -> None:
+        ops.block_scatter(self._block_table(), len(self.index_list), self.block, compact)   # smt.py:332-341
+
     def _apply(self, fn, *args, **kwargs):
         out = super()._apply(fn, *args, **kwargs)
         self._table = None
-        self._synced = None
         return out
 
     # -- what SMTAdam's arena (optim._Arena) asks of the layer that owns a parameter --
@@ -315,32 +345,6 @@ class LinearLayer_MatrixSparsity(nn.Module):
     @staticmethod
     def _writeback_args(key, entries, device) -> dict:
         return dict(table=ops.make_block_table(entries, device), n_blocks=len(entries), block=key[1], w_dtype=key[2])
-
-    def mark_synced(self) -> None:
-        """Called by the fused optimizer (SMTAdam) right after it has written the updated blocks into `weight`
-        itself.  The mark is tied to the parameter's storage pointer and version counter: re-pointing `.data`
-        (DeepSpeed / ZeRO flat buffers) or any version-counted write to the Parameter invalidates it.  Writes
-        through `selected_weight.data` are invisible to the version counter, so whoever does that while SMTAdam
-        owns the parameter must call `sync_weight(force=True)`; without SMTAdam nothing is ever skipped."""
-        self._synced = (self.selected_weight.data_ptr(), self.selected_weight._version)
-
-    def sync_weight(self, force: bool = False) -> None:
-        """compact -> dense write-back (smt.py:332-341): ONE launch per call.  Unconditional like the reference's
-        loop, except right after an SMTAdam step that wrote the dense blocks itself (see `mark_synced`)."""
-        if not force and self._synced is not None and \
-                self._synced == (self.selected_weight.data_ptr(), self.selected_weight._version):
-            return
-        self._synced = None
-        n = len(self.index_list)
-        if n:
-            sw = self.selected_weight.data
-            if sw.dtype != self.weight.dtype:
-                sw = sw.to(self.weight.dtype)
-            ops.block_scatter(self._block_table(), n, self.block, sw.contiguous())
-
-    def forward(self, x):
-        self.sync_weight()
-        return self.fn(x, self.selected_weight, self.index_list, self.weight)   # smt.py:343
 
 
 # ---- fused q/k/v projections (SURVEY section 8f row 2: the dense side of linearZ) --------------------------------
@@ -371,7 +375,7 @@ class fusedLinearZ(torch.autograd.Function):
         ctx.x_shape = input.shape
         ctx.xkey = (x2.data_ptr(), x2.shape[0])
         partials = []
-        sparse = [m for m in group.members if isinstance(m, _SPARSE_LAYERS)]
+        sparse = [m for m in group.members if isinstance(m, _SparseLinear)]
         for k, m in enumerate(sparse):
             if isinstance(m, LinearLayer_ChannelSparsity):
                 partials.append(ops.channel_gather(x2, _channel_idx_for(m.index_list, x2.device, 8))
@@ -394,7 +398,7 @@ class fusedLinearZ(torch.autograd.Function):
         grads, k, j = [], 0, 0
         x2 = None
         for m, dy2 in zip(members, dys):
-            if not isinstance(m, _SPARSE_LAYERS):
+            if not isinstance(m, _SparseLinear):
                 continue
             g = None
             if isinstance(m, LinearLayer_ChannelSparsity):
@@ -440,7 +444,7 @@ class _SharedInputGroup:
                 self._cache = None
             return y
         if role == 0 and self._supported(x):
-            sparse = [m for m in self.members if isinstance(m, _SPARSE_LAYERS)]
+            sparse = [m for m in self.members if isinstance(m, _SparseLinear)]
             for m in sparse:
                 m.sync_weight()                         # smt.py:332-341 / 208-211, unless SMTAdam vouches
             outs = list(fusedLinearZ.apply(x, self, *[m.selected_weight for m in sparse]))
@@ -574,12 +578,12 @@ def convert_linear_layer_to_matrix_sparsity(model,
     return model
 
 
-def convert_matrix_sparsity_to_linear_layer(model, part_module_name=['.layers']):
-    """Reference: smt.py:416-457: write the trained blocks back and restore plain nn.Linear modules that
-    share the (now merged) weight Parameter."""
+def _to_linear_layers(model, cls, part_module_name):
+    """Every `cls` module under `part_module_name` writes its trained part back and becomes a plain nn.Linear that
+    shares the (now merged) weight Parameter."""
     unfuse_qkv_projections(model)
     names = [name for name, module in model.named_modules()
-             if isinstance(module, LinearLayer_MatrixSparsity) and any(part in name for part in part_module_name)]
+             if isinstance(module, cls) and any(part in name for part in part_module_name)]
     for name in names:
         module = _getattr_path(model, name)
         module.sync_weight(force=True)
@@ -589,6 +593,12 @@ def convert_matrix_sparsity_to_linear_layer(model, part_module_name=['.layers'])
         linear.weight = module.weight                      # smt.py:451 — same Parameter, no clone
         _setattr_path(model, name, linear)
     return model
+
+
+def convert_matrix_sparsity_to_linear_layer(model, part_module_name=['.layers']):
+    """Reference: smt.py:416-457: write the trained blocks back and restore plain nn.Linear modules that
+    share the (now merged) weight Parameter."""
+    return _to_linear_layers(model, LinearLayer_MatrixSparsity, part_module_name)
 
 
 def freeze_unselected_matrix_layer(model,
@@ -673,22 +683,10 @@ def get_optimizer_qk_augment_grouped_parameters(
 # and trains the wrong entries for square ones.  Here channel i owns COLUMN index_list[i] of W; `selected_weight` is
 # [n, out_features] (row i = W[:, index_list[i]]), so the gradient formula is the reference's, bit for bit in fp32.
 
-_idx_cache: Dict[Tuple[int, torch.device], Tuple[tuple, torch.Tensor]] = {}
-
-
 def _channel_idx_for(index_list, device, pad_to: int = 1) -> torch.Tensor:
-    """int32 device copy of a channel index list (cached per list object, validated by value); `pad_to` > 1 appends -1
-    entries ("zero column") up to a multiple of it."""
-    snap = tuple(int(i) for i in index_list)
-    key = (id(index_list), device, pad_to)
-    hit = _idx_cache.get(key)
-    if hit is not None and hit[0] == snap:
-        return hit[1]
-    t = ops.make_channel_idx(snap, device, pad_to)
-    if len(_idx_cache) > 4096:
-        _idx_cache.clear()
-    _idx_cache[key] = (snap, t)
-    return t
+    """int32 device copy of a channel index list (cached by ops.index_table); `pad_to` > 1 appends -1 entries ("zero
+    column") up to a multiple of it."""
+    return ops.index_table(index_list, ops.make_channel_idx, device, pad_to)[1]
 
 
 class linearChannel(torch.autograd.Function):
@@ -700,9 +698,7 @@ class linearChannel(torch.autograd.Function):
 
     @staticmethod
     def forward(ctx, input, selected_weight, channel_index_list, weight):
-        x2 = input.reshape(-1, input.shape[-1])
-        if x2.stride(-1) != 1:
-            x2 = x2.contiguous()
+        x2 = _as_operand(input.reshape(-1, input.shape[-1]))
         # packed copy of the selected input channels, ONE launch (smt.py:240-247 does n strided slice copies); padded
         # with zero columns so that the tcgen05 gradient kernel can read it through TMA (16-byte row pitch) - fp32 inputs
         # take the fp32 block kernel, which wants whole 64-column blocks
@@ -719,9 +715,7 @@ class linearChannel(torch.autograd.Function):
         partial, weight = ctx.saved_tensors
         grad_input = grad_weight = None
         if ctx.needs_input_grad[1]:
-            dy2 = grad_output.reshape(-1, grad_output.shape[-1])
-            if dy2.stride(-1) != 1 or (dy2.stride(0) * dy2.element_size()) % 16 != 0:
-                dy2 = dy2.contiguous()
+            dy2 = _as_operand(grad_output.reshape(-1, grad_output.shape[-1]))
             grad_weight = _channel_weight_grad(ctx.sw_ref, partial, ctx.n_channels, dy2, ctx.xkey)
         if ctx.needs_input_grad[0]:
             grad_input = torch.matmul(grad_output, weight)                                      # smt.py:286
@@ -731,20 +725,15 @@ class linearChannel(torch.autograd.Function):
 def _channel_weight_grad(sw_param, partial, n, dy2, xkey):
     """The channel gradient of one module (smt.py:283-284).  Native mode (the parameter owns a GradSink): delivered
     into the padded arena region of the parameter - grouped with the other modules of the backward pass when grouping
-    is enabled - and None is returned; otherwise the [n, out_features] gradient is returned.  `xkey` identifies the
-    module's input (chunked flushes happen at layer boundaries)."""
+    is enabled - and None is returned; otherwise the [n, out_features] gradient is returned.  `dy2` is a TMA operand
+    (`_as_operand`); `xkey` identifies the module's input (chunked flushes happen at layer boundaries)."""
     if partial.dtype != dy2.dtype:
         partial = partial.to(dy2.dtype)
     sink = getattr(sw_param, "_smt_sink", None)
     if sink is not None:
-        dy2 = _as_operand(dy2)
-        accumulate = sink.begin_delivery(sw_param)
-        if _grouped["enabled"]:
-            _enqueue(xkey, dy2.device, lambda: _pending.add_channel(partial, dy2, n, sink.store, accumulate=accumulate,
-                                                                    sq=sink.sq, sq_slot0=sink.sq_slot0, sink=sink))
-        else:
-            ops.channel_grad_gemm(partial, n, dy2, out=sink.store, accumulate=accumulate)
-            sink.sq_ok = False
+        _deliver(sw_param, sink, xkey, dy2.device, _grouped["enabled"],
+                 functools.partial(_pending.add_channel, partial, dy2, n, sink.store),
+                 functools.partial(ops.channel_grad_gemm, partial, n, dy2, out=sink.store))
         return None
     out_f = dy2.shape[1]
     # smt.py:283-284: sum over the batch of partial^T @ dy == ONE contraction over all tokens, on the same tcgen05
@@ -775,19 +764,12 @@ def _channel_grad_by_blocks(partial, n, dy2):
     return full[:n, :out_f].contiguous()
 
 
-class LinearLayer_ChannelSparsity(nn.Module):
+class LinearLayer_ChannelSparsity(_SparseLinear):
     """Linear layer whose only trainable parameter is a compact copy of its selected input channels (weight columns).
     Reference: smt.py:185-217 (same constructor signature and attribute names; column semantics, see above)."""
 
     def __init__(self, weight, bias=None, index_list=[]):
-        super().__init__()
-        if not weight.is_cuda:
-            raise SMTLibraryError("LinearLayer_ChannelSparsity needs its weight on a CUDA device: the SMT kernels "
-                                  "have no CPU fallback")
-        self.weight = weight
-        self.weight.requires_grad = False                 # smt.py:191
-        self.bias = bias                                  # kept but unused, like smt.py:192,214
-        self.index_list = index_list
+        super().__init__(weight, bias, index_list)
         seen = set()
         for i in index_list:
             if not 0 <= int(i) < weight.shape[1]:
@@ -799,16 +781,10 @@ class LinearLayer_ChannelSparsity(nn.Module):
         compact = torch.empty(n, weight.shape[0], dtype=weight.dtype, device=weight.device)
         if n:
             ops.column_gather(weight.data, _channel_idx_for(index_list, weight.device), compact)
-        self.selected_weight = nn.Parameter(compact, requires_grad=True)
-        self.selected_weight._smt_owner = weakref.ref(self)   # lets SMTAdam find the dense weight to write back
-        self.fn = linearChannel.apply
-        # Set ONLY by `mark_synced()` (SMTAdam after its fused column write-back); see LinearLayer_MatrixSparsity.
-        self._synced = None
+        self._set_selected(compact, linearChannel.apply)
 
-    def _apply(self, fn, *args, **kwargs):
-        out = super()._apply(fn, *args, **kwargs)
-        self._synced = None
-        return out
+    def _scatter(self, compact: torch.Tensor) -> None:
+        ops.column_scatter(self.weight.data, _channel_idx_for(self.index_list, self.weight.device), compact)
 
     # -- what SMTAdam's arena (optim._Arena) asks of the layer that owns a parameter (see LinearLayer_MatrixSparsity) --
     def _arena_ok(self) -> bool:
@@ -839,33 +815,6 @@ class LinearLayer_ChannelSparsity(nn.Module):
     def _writeback_args(key, entries, device) -> dict:
         return dict(columns=ops.make_column_table(entries, device), n_columns=len(entries), w_dtype=key[1])
 
-    def mark_synced(self) -> None:
-        """Called by SMTAdam right after it has written the updated channels into the columns of `weight` itself; the
-        same rule as LinearLayer_MatrixSparsity.mark_synced (storage pointer + version counter of selected_weight)."""
-        self._synced = (self.selected_weight.data_ptr(), self.selected_weight._version)
-
-    def sync_weight(self, force: bool = False) -> None:
-        """compact -> dense write-back (smt.py:208-211): one launch on every forward, like the reference's loop —
-        whatever optimizer updated `selected_weight` (also through `.data` or an aliased flat buffer) is seen.  The only
-        exception is right after an SMTAdam step that wrote the columns itself (see `mark_synced`)."""
-        if not force and self._synced is not None and \
-                self._synced == (self.selected_weight.data_ptr(), self.selected_weight._version):
-            return
-        self._synced = None
-        if len(self.index_list):
-            sw = self.selected_weight.data
-            if sw.dtype != self.weight.dtype:
-                sw = sw.to(self.weight.dtype)
-            ops.column_scatter(self.weight.data, _channel_idx_for(self.index_list, self.weight.device),
-                               sw.contiguous())
-
-    def forward(self, x):
-        self.sync_weight()
-        return self.fn(x, self.selected_weight, self.index_list, self.weight)   # smt.py:213
-
-
-_SPARSE_LAYERS = (LinearLayer_MatrixSparsity, LinearLayer_ChannelSparsity)
-
 
 def convert_linear_layer_to_channel_sparsity(model,
                                              selected_channel,
@@ -893,18 +842,7 @@ def convert_linear_layer_to_channel_sparsity(model,
 def convert_channel_sparsity_to_linear_layer(model, part_module_name=['.layers']):
     """Write the trained channels back and restore plain nn.Linear modules (the channel twin of smt.py:416-457; the
     reference has no such function for channels)."""
-    unfuse_qkv_projections(model)
-    names = [name for name, module in model.named_modules()
-             if isinstance(module, LinearLayer_ChannelSparsity) and any(part in name for part in part_module_name)]
-    for name in names:
-        module = _getattr_path(model, name)
-        module.sync_weight(force=True)
-        out_f, in_f = module.weight.shape
-        linear = nn.Linear(in_f, out_f, bias=False, device="meta")
-        linear = linear.to_empty(device=module.weight.device).to(module.weight.dtype)
-        linear.weight = module.weight
-        _setattr_path(model, name, linear)
-    return model
+    return _to_linear_layers(model, LinearLayer_ChannelSparsity, part_module_name)
 
 
 def freeze_unselected_channel_layer(model,

@@ -224,6 +224,41 @@ def test_product_path_fails_loudly_without_cuda():
         H.select_submatrix_based_on_grads({}, {}, 1, calculate_strategy="bogus")
 
 
+def test_index_table_cache_follows_the_list_by_value():
+    """ops.index_table: one cache of index-list snapshots and the device tables derived from them, keyed on the list
+    object and checked by value on every call."""
+    from sparse_matrix_tuning_b200 import ops
+    idx = [(0, 1), (2, 3)]
+    snap, rc = ops.index_table(idx, ops.make_block_rc, "cpu")
+    assert snap == ((0, 1), (2, 3)) and rc.tolist() == [[0, 1], [2, 3]]
+    assert ops.index_table(idx, ops.make_block_rc, "cpu")[1] is rc               # same list, same contents
+    assert ops.index_table(idx)[0] is snap
+    idx[1] = (4, 5)                                                             # edited in place
+    snap2, rc2 = ops.index_table(idx, ops.make_block_rc, "cpu")
+    assert snap2 == ((0, 1), (4, 5)) and rc2 is not rc and rc2.tolist() == [[0, 1], [4, 5]]
+    idx.append((6, 7))
+    assert ops.index_table(idx, ops.make_block_rc, "cpu")[1].tolist() == [[0, 1], [4, 5], [6, 7]]
+    twin = [list(e) for e in idx]                                               # equal, distinct, lists not tuples
+    snap3, rc3 = ops.index_table(twin, ops.make_block_rc, "cpu")
+    assert snap3 == ((0, 1), (4, 5), (6, 7)) and rc3.tolist() == [[0, 1], [4, 5], [6, 7]]
+    assert ops.index_table(twin, ops.make_block_rc, "cpu")[1] is rc3
+    # a different kind (builder or its arguments) or device is a separate entry of the same list
+    ch = [5, 3, 9]
+    plain = ops.index_table(ch, ops.make_channel_idx, "cpu", 1)[1]
+    padded = ops.index_table(ch, ops.make_channel_idx, "cpu", 8)[1]
+    meta = ops.index_table(ch, ops.make_channel_idx, "meta", 8)[1]
+    assert plain.tolist() == [5, 3, 9] and padded.tolist() == [5, 3, 9] + [-1] * 5
+    assert meta.device.type == "meta" and meta.shape == (8,)
+    assert ops.index_table(ch, ops.make_channel_idx, "cpu", 1)[1] is plain
+    assert ops.index_table(ch, ops.make_channel_idx, "cpu", 8)[1] is padded
+    assert ops.index_table(ch, ops.make_channel_idx, "meta", 8)[1] is meta
+    # bounded
+    lists = [[i] for i in range(ops._INDEX_CACHE_MAX + 10)]
+    for i, lst in enumerate(lists):
+        assert ops.index_table(lst, ops.make_channel_idx, "cpu", 1)[1].tolist() == [i]
+    assert len(ops._index_cache) <= ops._INDEX_CACHE_MAX
+
+
 def test_no_oracle_import_in_product_package():
     pkg = os.path.join(ROOT, "sparse_matrix_tuning_b200")
     for dirpath, _d, files in os.walk(pkg):
